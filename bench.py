@@ -13,6 +13,8 @@ A "step" is one pass of the hot path over one batch of synthetic input:
   * --workload hisfrag: BASELINE.json configs[3]'s model (patch16 / 512 px) on `--items` synthetic fragments, all
           pairs a <= b, rows sharded over the ranks by the reference sampler's boundaries, through
           grid.score_fragments (NCCL all-gather inside); fixed total work -> "strong" scaling.
+`--dump-outputs DIR` writes what the timed path returned in its last timed step to DIR/<name>.npy (see dump_outputs);
+the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 `value` is timed on the device with the piece images already resident in HBM; `e2e` goes through the public API with
 HOST buffers (pinned), H2D and D2H inside the timed region. `roofline` is measured live: one extra step with a CUDA
 event before every launch (engine option PROFILE) gives every kernel family's summed duration; the family with the
@@ -30,6 +32,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the tree it runs from as it found it (it may be read-only)
 
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
@@ -43,6 +46,7 @@ F_DEC_PAIR = 8 * (28 * 384 * 384 * 65 + 4 * 65 * 65 * 384 + 4 * 65 * 64 * 384) +
 F_ENC_ITEM = 8 * (24 * 384 * 384 * 64 + 4 * 64 * 64 * 384) + 2 * 64 * 192 * 384
 F_KV_ITEM = 8 * 4 * 384 * 384 * 64
 F_PREP_ITEM = 2 * 64 * 192 * 384
+DUMP_LIMIT = 64_000_000   # bytes that --dump-outputs writes at most, .npy headers included
 
 
 def load_peaks():
@@ -52,6 +56,25 @@ def load_peaks():
         return dict(hbm_gbs=d['hbm_gbs'], tf_burst=d['bf16_tflops'], tf_sustained=d.get('bf16_tflops_sustained', d['bf16_tflops']),
                     source='measured (MEASURED_PEAKS.json)')
     return dict(hbm_gbs=6650.0, tf_burst=1590.0, tf_sustained=1400.0, source='fallback (B200_PROFILING.md)')
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each tensor of `arrays` (name -> tensor) as out_dir/<name>.npy, float64 kept as float64 and
+    everything else as float32. Smallest first, each array gets an equal share of what DUMP_LIMIT has left; one that
+    does not fit its share is written as a fixed sample of its flattened elements instead (1-D, indices drawn with
+    replacement by a generator seeded with 0 and sorted), so every run with the same arguments samples the same
+    elements. Outputs that fit DUMP_LIMIT together are written whole."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: (v.detach().double() if v.dtype == torch.float64 else v.detach().float()).cpu() for k, v in arrays.items()}
+    header = 4096   # bytes reserved per file for the .npy header
+    left = DUMP_LIMIT
+    for i, (name, v) in enumerate(sorted(arrays.items(), key=lambda kv: kv[1].numel() * kv[1].element_size())):
+        share = left // (len(arrays) - i) - header
+        if v.numel() * v.element_size() > share:
+            idx = torch.randint(v.numel(), (share // v.element_size(),), generator=torch.Generator().manual_seed(0))
+            v = v.reshape(-1)[idx.sort().values]
+        np.save(os.path.join(out_dir, f'{name}.npy'), v.numpy())
+        left -= v.numel() * v.element_size() + header
 
 
 # ----------------------------------------------------------------------------------------------- workloads
@@ -333,7 +356,7 @@ def run_ours(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        step(dev_images)
+        scores = step(dev_images)
     e1.record()
     torch.cuda.synchronize()
     clock_info = clocks.stop()
@@ -341,6 +364,9 @@ def run_ours(args):
     launches = model.launch_count() - launches0
     ms_step = max_over_ranks(e0.elapsed_time(e1) / args.steps, world)
     value = n_pairs_job / (ms_step / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {f'logits_puzzle{pz}': s for pz, s in enumerate(scores)})
+    del scores
 
     # ---- end to end through the public API with host buffers
     for _ in range(2):
@@ -559,6 +585,8 @@ def run_hisfrag(args):
     launches = model.launch_count() - launches0
     ms = max_over_ranks(e0.elapsed_time(e1) / args.steps, world)
     assert sim.shape == (n, n)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {'similarity': sim})
     # each rank's own share without the collective (what limits the curve: the sampler's boundaries balance PAIRS, the
     # per-rank encoder work follows the ROWS)
     l0, l1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -633,10 +661,15 @@ def run_train(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        loss, logits, groups, _ = train.train_step(model, samples, labels, generator=gen)
+        loss, logits, groups, pair_labels = train.train_step(model, samples, labels, generator=gen)
     e1.record()
     torch.cuda.synchronize()
     ms = max_over_ranks(e0.elapsed_time(e1) / args.steps, world)
+    if args.dump_outputs and rank == 0:
+        # rank 0's own pairs and logits; the gradients are averaged over the ranks (flattened, named_parameters order)
+        dump_outputs(args.dump_outputs, {
+            'loss': loss.reshape(1), 'logits': logits, 'groups': groups.double(), 'labels': pair_labels,
+            'grads': torch.cat([p.grad.reshape(-1) for p in model.parameters()])})
     gnorm = float(torch.sqrt(sum(p.grad.double().pow(2).sum() for p in model.parameters())))
     train.train_step(model, samples, labels, generator=gen, profile=True)
     prof = model.train_profile
@@ -674,9 +707,16 @@ def main():
     ap.add_argument('--lean', action='store_true',
                     help='--workload hisfrag at full size: warm up on 96 fragments, one timed pass, no local / profile passes '
                          '(ms_local = the rank\'s own timed pass incl. the all-gather, kernel shares from a 96-fragment pass)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the timed path returned in its last timed step as DIR/<name>.npy (float32 / '
+                         'float64, %d bytes at most: larger outputs as a fixed seeded sample)' % DUMP_LIMIT)
     args = ap.parse_args()
-    if args.warmup < 3 and args.impl == 'ours':
-        args.warmup = max(args.warmup, 0)
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.warmup < 0:
+        ap.error('--warmup must not be negative')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs: the reference arm sizes its sample by the host\'s speed, so its outputs differ from run to run')
     if args.impl == 'reference':
         run_reference(args)
     else:

@@ -1,7 +1,9 @@
 """CPU: the solver distance tables (SURVEY 8f row 3). The oracle restatement against the fixture written by the
 reference's own InterPieceDistance class (tests/golden/make_golden_tables.py), the host-side pieces of
-vited_b200.solver_tables, and -- where /root/reference is present (the build container) -- the prebuilt object dropped
-into the reference's solver against the solver run with its own callbacks."""
+vited_b200.solver_tables, the object install() builds against the constructor state stored in that fixture, and --
+where VITED_REFERENCE names a checkout of the reference project -- the prebuilt object against the reference's own
+constructor and dropped into the reference's solver against the solver run with its own callbacks."""
+import enum
 import os
 import sys
 
@@ -13,7 +15,7 @@ from tests.conftest import GOLDEN
 sys.path.insert(0, GOLDEN)
 import make_golden_tables as mg  # noqa: E402
 
-REF = '/root/reference'
+REF = os.environ.get('VITED_REFERENCE', '')
 KEYS = ['asym_dist', 'asym_compat', 'mutual_compat', 'min_dist', 'second_dist', 'candidates', 'best_buddy',
         'start_order', 'start_compat']
 
@@ -77,7 +79,68 @@ def _tables_from_oracle(d, order, rules='numpy2'):
     return tables
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason='needs the reference checkout (build container only)')
+class _Side(enum.Enum):
+    """What install() uses of the reference's PuzzlePieceSide (paikin_tal_solver/puzzle_piece.py)."""
+    top = 0
+    right = 1
+    bottom = 2
+    left = 3
+
+    @staticmethod
+    def get_all_sides():
+        return [_Side.top, _Side.right, _Side.bottom, _Side.left]
+
+    @property
+    def complementary_side(self):
+        return _Side((self.value + 2) % 4)
+
+
+class _PieceInfo:
+    """What install() uses of the reference's PieceDistanceInformation: the state its constructor starts from."""
+
+    def __init__(self, id_numb, numb_pieces, puzzle_type):
+        self._id, self._numb_pieces, self._puzzle_type = id_numb, numb_pieces, puzzle_type
+        self._best_buddy_candidates = [[] for _ in range(4)]
+        self._best_buddies = [[] for _ in range(4)]
+
+
+class _InterPieceDistance:
+    pass
+
+
+@pytest.mark.parametrize('case', mg.CASES, ids=lambda c: f'seed{c[0]}_{c[1]}x{c[2]}')
+def test_installed_object_matches_reference_fixture(case):
+    """install() leaves an InterPieceDistance in the state the reference's own constructor left it in, as the fixture
+    stores that state (tests/golden/make_golden_tables.py, run under NumPy >= 2 scalar rules like the tables here)."""
+    from vited_b200 import solver_tables
+    z, _ = _cases()
+    seed = case[0]
+    d, order = mg.case_inputs(*case)
+    n = len(order)
+    pieces = [mg._Piece(o) for o in order]
+    ipd = solver_tables.install(_tables_from_oracle(d, order), pieces, 'type1', _InterPieceDistance, _PieceInfo, _Side)
+    assert isinstance(ipd, _InterPieceDistance)
+    assert [p.id_number for p in pieces] == list(range(n))
+    assert ipd._numb_pieces == n and ipd._puzzle_type == 'type1' and ipd._distance_function is None
+    assert [(a, b) for a, b, _ in ipd._start_piece_ordering] == [tuple(r) for r in z[f'start_order_{seed}'].tolist()]
+    assert np.array_equal(np.array([float(c) for _, _, c in ipd._start_piece_ordering]), z[f'start_compat_{seed}'])
+    assert len(ipd._piece_distance_info) == n
+    for i, info in enumerate(ipd._piece_distance_info):
+        assert info._id == i and info._numb_pieces == n
+        for name, key in (('_asymmetric_distances', 'asym_dist'), ('_asymmetric_compatibilities', 'asym_compat'),
+                          ('_mutual_compatibilities', 'mutual_compat')):
+            x, y = getattr(info, name), z[f'{key}_{seed}'][i]
+            assert x.shape == (4, n, 1) and x.dtype == y.dtype and np.array_equal(x[:, :, 0], y), name
+        assert [int(v) for v in info._min_distance] == z[f'min_dist_{seed}'][i].tolist()
+        assert [int(v) for v in info._second_best_distance] == z[f'second_dist_{seed}'][i].tolist()
+        for s in range(4):
+            cs = _Side((s + 2) % 4)
+            assert info._best_buddy_candidates[s] == [(int(j), cs) for j in np.nonzero(z[f'candidates_{seed}'][i, s])[0]]
+            b = int(z[f'best_buddy_{seed}'][i, s])
+            assert info._best_buddies[s] == ([(b, cs)] if b >= 0 else [])
+
+
+@pytest.mark.skipif(not os.path.isdir(REF), reason='needs a checkout of the reference project (VITED_REFERENCE)')
 @pytest.mark.parametrize('case', [mg.CASES[1], mg.CASES[4], mg.CASES[6]], ids=lambda c: f'seed{c[0]}')
 def test_installed_object_equals_reference_constructor(case):
     """install() leaves the reference's InterPieceDistance in exactly the state its own constructor does."""
@@ -116,7 +179,7 @@ def test_installed_object_equals_reference_constructor(case):
         assert a._id == b._id and a._numb_pieces == b._numb_pieces
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason='needs the reference checkout (build container only)')
+@pytest.mark.skipif(not os.path.isdir(REF), reason='needs a checkout of the reference project (VITED_REFERENCE)')
 def test_reference_solver_runs_unmodified_on_prebuilt_tables(tmp_path, monkeypatch):
     """paikin_tal_driver (solver_driver.py:17-30) with the InterPieceDistance name in solver.py:212 bound to
     solver_tables.factory places every piece exactly where the run with the Python callbacks places it."""
