@@ -243,6 +243,15 @@ VITED_API int vited_op_gemm_resid_ln(const void* A, const void* W, const float* 
 VITED_API int vited_op_mlp_resid_ln(const void* h_in, const void* W1, const float* b1, const void* W2, const float* b2,
                           float* x, const float* ln_w, const float* ln_b, void* h_out, int M, int D, int hidden,
                           float eps, void* stream);
+/* the cross-attention projection + residual + norm2 in front of the fused MLP sub-block (D must be 384, hidden a
+ * multiple of 64): x_mid = x + o[M,384] h16 * Wp[384,384]^T h16 + bp; h = LayerNorm(x_mid) * ln2_w + ln2_b (h16);
+ * x[M,384] f32 = x_mid + GELU(h * W1^T + b1) * W2^T + b2; h_out[M,384] h16 = LayerNorm(x) * ln_w + ln_b
+ * (a decoder CrossBlock's cross_attn.proj and Mlp, vision_transformer.py:271-272, + the next norm1). x_mid and h are
+ * never written: on return x holds the block's output rows. */
+VITED_API int vited_op_cproj_mlp_resid_ln(const void* o, const void* Wp, const float* bp, float* x, const float* ln2_w,
+                                const float* ln2_b, const void* W1, const float* b1, const void* W2, const float* b2,
+                                const float* ln_w, const float* ln_b, void* h_out, int M, int D, int hidden, float eps,
+                                void* stream);
 /* x += delta (h16, may be NULL); h = LayerNorm(x) * w + b as h16 (w NULL => skipped). Split token layout. */
 VITED_API int vited_op_resid_ln(float* x, const void* delta, const float* ln_w, const float* ln_b, void* h, int n_seq,
                       int n_patch, int has_cls, int D, float eps, void* stream);

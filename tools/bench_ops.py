@@ -101,6 +101,35 @@ def main():
                             tflops_frac=fl / ms / 1e9 / tf, gbs=by / ms / 1e6, gbs_frac=by / ms / 1e6 / hbm))
         os.environ.pop('VITED_EPI_WARPS', None)
         del hin, xx, hh
+        # the decoder's cross projection + residual + norm2 + MLP sub-block in one launch, against the gemm_ln + mlp_ln
+        # pair it replaces, at the engine's chunk shape (524,288 rows)
+        Mc = 524288
+        o = torch.randn(Mc, 384, device='cuda').to(L.act_dtype())
+        Wp = (torch.randn(384, 384, device='cuda') / math.sqrt(384)).to(L.act_dtype())
+        bp = torch.randn(384, device='cuda')
+        xx = torch.randn(Mc, 384, device='cuda')
+        hh = torch.empty(Mc, 384, dtype=L.act_dtype(), device='cuda')
+
+        def pair():
+            L.check(L.lib.vited_op_gemm_resid_ln(o.data_ptr(), Wp.data_ptr(), bp.data_ptr(), xx.data_ptr(), lw.data_ptr(),
+                                                 lb.data_ptr(), hh.data_ptr(), Mc, 384, 384, 1e-6, st), 'gemm_ln')
+            L.check(L.lib.vited_op_mlp_resid_ln(hh.data_ptr(), W1.data_ptr(), b1.data_ptr(), W2.data_ptr(), b2.data_ptr(),
+                                                xx.data_ptr(), lw.data_ptr(), lb.data_ptr(), hh.data_ptr(), Mc, 384, 1536, 1e-6,
+                                                st), 'mlp_ln')
+
+        def fused():
+            L.check(L.lib.vited_op_cproj_mlp_resid_ln(o.data_ptr(), Wp.data_ptr(), bp.data_ptr(), xx.data_ptr(), lw.data_ptr(),
+                                                      lb.data_ptr(), W1.data_ptr(), b1.data_ptr(), W2.data_ptr(), b2.data_ptr(),
+                                                      lw.data_ptr(), lb.data_ptr(), hh.data_ptr(), Mc, 384, 1536, 1e-6, st),
+                    'mlp_ln_cproj')
+
+        fl = 2.0 * Mc * 384 * 384 + 4.0 * Mc * 384 * 1536
+        for name, fn, per_row in (('gemm_ln_cproj+mlp_ln', pair, 2 * 4608), ('mlp_ln_cproj', fused, 4608)):
+            ms = timeit(fn, flush=flush)
+            by = Mc * per_row + 2 * 384 * 384 + 4 * 384 * 1536
+            out.append(dict(op=name, M=Mc, D=384, hidden=1536, ms=ms, tflops=fl / ms / 1e9, tflops_frac=fl / ms / 1e9 / tf,
+                            gbs=by / ms / 1e6, gbs_frac=by / ms / 1e6 / hbm))
+        del o, xx, hh
     if want('ln'):
         x = torch.randn(M, D, device='cuda')
         delta = torch.randn(M, D, device='cuda').to(L.act_dtype())

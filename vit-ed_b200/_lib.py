@@ -88,6 +88,8 @@ SIGNATURES = {
     "vited_op_gemm": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
     "vited_op_gemm_resid_ln": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _f, _vp]),
     "vited_op_mlp_resid_ln": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _f, _vp]),
+    "vited_op_cproj_mlp_resid_ln": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _f,
+                                         _vp]),
     "vited_op_resid_ln": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _f, _vp]),
     "vited_op_attention": (_i, [_vp, _i, _vp, _i, _vp, _i, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _f, _i, _vp]),
     "vited_op_im2col": (_i, [_vp, _vp, _i, _i, _i, _i, _vp]),

@@ -266,22 +266,25 @@ static int L_gemm_ln(vited_engine* e, const act_t* A, const Linear& l, float* x,
   }
   return gemm_resid_ln(A, l.w, l.b, x, ln.w, ln.b, h, M, l.out, l.in, 1e-6f, s);
 }
-// fused x += fc2(GELU(fc1(h))) ; h = LN(x)  (mlp_ln.cu)
-static bool use_fused_mlp(vited_engine* e, size_t rows, const Linear& fc1, const Linear& fc2) {
-  return e->fuse_mlp && use_fused_ln(e, rows, fc2) && fc1.in == e->D && fc2.in == fc1.out &&
-         mlp_resid_ln_supported((int)rows, e->D, fc1.out);
+// fused x += cproj(o); x += fc2(GELU(fc1(norm2(x)))) ; h = LN(x)  (mlp_ln.cu)
+static bool use_fused_mlp(vited_engine* e, size_t rows, const Linear& cproj, const Linear& fc1, const Linear& fc2) {
+  return e->fuse_mlp && use_fused_ln(e, rows, fc2) && use_fused_ln(e, rows, cproj) && cproj.out == e->D &&
+         fc1.in == e->D && fc2.in == fc1.out && cproj_mlp_resid_ln_supported((int)rows, e->D, cproj.in, fc1.out);
 }
-static int L_mlp_ln(vited_engine* e, const act_t* h_in, const Linear& fc1, const Linear& fc2, float* x, const LNorm& ln,
-                    act_t* h_out, int M, cudaStream_t s) {
+static int L_cproj_mlp_ln(vited_engine* e, const act_t* o, const Linear& cproj, const LNorm& norm2, const Linear& fc1,
+                          const Linear& fc2, float* x, const LNorm& ln, act_t* h_out, int M, cudaStream_t s) {
   if (e->profile) {
+    // the name starts with mlp_ln: bench.py's mlp_ln family. Bytes: o (2) + x (4) in, x (4) + h (2) out per element
     char nm[64];
-    snprintf(nm, sizeof(nm), "mlp_ln_d%d_h%d", fc1.in, fc1.out);
-    prof_mark(e, nm, 4.0 * M * (double)fc1.out * fc1.in,
-              4.0 * (double)fc1.out * fc1.in + (double)M * fc1.in * (2.0 + 4.0 + 4.0 + 2.0), s);
+    snprintf(nm, sizeof(nm), "mlp_ln_cproj_d%d_h%d", fc1.in, fc1.out);
+    prof_mark(e, nm, 2.0 * M * (double)cproj.out * cproj.in + 4.0 * M * (double)fc1.out * fc1.in,
+              2.0 * (double)cproj.out * cproj.in + 4.0 * (double)fc1.out * fc1.in +
+                  (double)M * fc1.in * (2.0 + 4.0 + 4.0 + 2.0), s);
   } else {
     e->launches++;
   }
-  return mlp_resid_ln(h_in, fc1.w, fc1.b, fc2.w, fc2.b, x, ln.w, ln.b, h_out, M, fc1.in, fc1.out, 1e-6f, s);
+  return cproj_mlp_resid_ln(o, cproj.w, cproj.b, x, norm2.w, norm2.b, fc1.w, fc1.b, fc2.w, fc2.b, ln.w, ln.b, h_out, M,
+                            fc1.in, fc1.out, 1e-6f, s);
 }
 static int L_resid_ln(vited_engine* e, float* x, const act_t* delta, const float* gsrc, const int* gidx, int n_src,
                       const LNorm* ln, act_t* h, int n_seq, int has_cls, int write_x, cudaStream_t s, int g_off = 0) {
@@ -521,24 +524,27 @@ static int decode_chunk(vited_engine* e, int P, const int* ci, const int* xj, co
       }
       TRY(L_gemm(e, h, b.q, q, (int)rows, ACT_NONE, s));
       TRY(L_attn_cross(e, q, kvl, o, P, n_kv_seq, ci, s));
-      if (fuse) {
-        TRY(L_gemm_ln(e, o, b.cproj, x, b.norm2, h, (int)rows, s));
-      } else {
-        TRY(L_gemm(e, o, b.cproj, delta, (int)rows, ACT_NONE, s));
-        TRY(L_resid_ln(e, x, delta, nullptr, nullptr, 0, &b.norm2, h, P, 1, 1, s));
-      }
       h_is_norm1 = false;
-      if (fuse && l + 1 < L && use_fused_mlp(e, rows, b.fc1, b.fc2)) {
-        // the whole MLP sub-block, its residual add and the next layer's norm1 in one kernel: `hid` is never written
-        TRY(L_mlp_ln(e, h, b.fc1, b.fc2, x, e->dec[l + 1].norm1, h, (int)rows, s));
-        h_is_norm1 = true;
-      } else if (fuse && l + 1 < L) {
-        TRY(L_gemm(e, h, b.fc1, hid, (int)rows, ACT_GELU, s));
-        TRY(L_gemm_ln(e, hid, b.fc2, x, e->dec[l + 1].norm1, h, (int)rows, s));
+      if (fuse && l + 1 < L && use_fused_mlp(e, rows, b.cproj, b.fc1, b.fc2)) {
+        // the cross projection, its residual add and norm2, the whole MLP sub-block, its residual add and the next
+        // layer's norm1 in one kernel: neither the intermediate residual rows nor norm2's output nor `hid` is written
+        TRY(L_cproj_mlp_ln(e, o, b.cproj, b.norm2, b.fc1, b.fc2, x, e->dec[l + 1].norm1, h, (int)rows, s));
         h_is_norm1 = true;
       } else {
-        TRY(L_gemm(e, h, b.fc1, hid, (int)rows, ACT_GELU, s));
-        TRY(L_gemm(e, hid, b.fc2, delta, (int)rows, ACT_NONE, s));
+        if (fuse) {
+          TRY(L_gemm_ln(e, o, b.cproj, x, b.norm2, h, (int)rows, s));
+        } else {
+          TRY(L_gemm(e, o, b.cproj, delta, (int)rows, ACT_NONE, s));
+          TRY(L_resid_ln(e, x, delta, nullptr, nullptr, 0, &b.norm2, h, P, 1, 1, s));
+        }
+        if (fuse && l + 1 < L) {
+          TRY(L_gemm(e, h, b.fc1, hid, (int)rows, ACT_GELU, s));
+          TRY(L_gemm_ln(e, hid, b.fc2, x, e->dec[l + 1].norm1, h, (int)rows, s));
+          h_is_norm1 = true;
+        } else {
+          TRY(L_gemm(e, h, b.fc1, hid, (int)rows, ACT_GELU, s));
+          TRY(L_gemm(e, hid, b.fc2, delta, (int)rows, ACT_NONE, s));
+        }
       }
     } else {
       float* x_c = x + cls_off * D;
@@ -882,6 +888,14 @@ int vited_op_mlp_resid_ln(const void* h_in, const void* W1, const float* b1, con
                           void* stream) {
   return mlp_resid_ln((const act_t*)h_in, (const act_t*)W1, b1, (const act_t*)W2, b2, x, ln_w, ln_b, (act_t*)h_out, M, D,
                       hidden, eps, (cudaStream_t)stream);
+}
+
+int vited_op_cproj_mlp_resid_ln(const void* o, const void* Wp, const float* bp, float* x, const float* ln2_w,
+                                const float* ln2_b, const void* W1, const float* b1, const void* W2, const float* b2,
+                                const float* ln_w, const float* ln_b, void* h_out, int M, int D, int hidden, float eps,
+                                void* stream) {
+  return cproj_mlp_resid_ln((const act_t*)o, (const act_t*)Wp, bp, x, ln2_w, ln2_b, (const act_t*)W1, b1,
+                            (const act_t*)W2, b2, ln_w, ln_b, (act_t*)h_out, M, D, hidden, eps, (cudaStream_t)stream);
 }
 
 int vited_op_resid_ln(float* x, const void* delta, const float* ln_w, const float* ln_b, void* h, int n_seq,

@@ -37,6 +37,15 @@ bool mlp_resid_ln_supported(int M, int D, int hidden);
 int mlp_resid_ln(const act_t* h_in, const act_t* W1, const float* b1, const act_t* W2, const float* b2, float* x,
                  const float* ln_w, const float* ln_b, act_t* h_out, int M, int D, int hidden, float eps,
                  cudaStream_t stream);
+// the cross-attention projection + residual + norm2 in front of the same kernel (a decoder CrossBlock's
+// `x = x + cross_attn.proj(o); x = x + mlp(norm2(x))` followed by the next layer's norm1):
+//   x_mid = x + o[M,384] Wp[384,384]^T + bp;  x = x_mid + fc2(GELU(fc1(LayerNorm(x_mid) * ln2_w + ln2_b)));
+//   h_out = LayerNorm(x) * ln_w + ln_b.  x_mid and norm2(x_mid) never leave the SM; x holds the final rows only.
+bool cproj_mlp_resid_ln_supported(int M, int D, int K, int hidden);
+int cproj_mlp_resid_ln(const act_t* o, const act_t* Wp, const float* bp, float* x, const float* ln2_w,
+                       const float* ln2_b, const act_t* W1, const float* b1, const act_t* W2, const float* b2,
+                       const float* ln_w, const float* ln_b, act_t* h_out, int M, int D, int hidden, float eps,
+                       cudaStream_t stream);
 
 // ---- row-wise kernels (rowops.cu) ----
 // x[r,:] = (gather ? src[map(r),:] : x[r,:]) + delta[r,:]; optionally h[r,:] = LayerNorm(x[r,:]) * w + b (fp16).
