@@ -68,9 +68,15 @@ enum {
                                    (embed_dim 384, large row counts); 0 = separate resid_ln kernel                  */
   VITED_OPT_KV_BUDGET_MB = 7,   /* vited_score_grid processes context rows in blocks whose K/V cache (all decoder
                                    layers) fits this many MB (default 8000; Hisfrag: 18.9 MB per fragment)          */
-  VITED_OPT_FUSE_MLP = 8        /* 1 (default) = the MLP sub-block (fc1, GELU, fc2), its residual add and the next
+  VITED_OPT_FUSE_MLP = 8,       /* 1 (default) = the MLP sub-block (fc1, GELU, fc2), its residual add and the next
                                    layer's LayerNorm run in one kernel, hidden activations never written (needs
                                    FUSE_LN; embed_dim 384, large row counts); 0 = fc1 GEMM + fused fc2 GEMM          */
+  VITED_OPT_XSRC_BUDGET_MB = 9  /* vited_score_grid(_u8) holds the decoder input states of at most this many MB of grid
+                                   columns at once (default 32000; (N_e + 1) * embed_dim * 4 bytes per column item,
+                                   Hisfrag: 1.57 MB). When all columns of a call fit, they are built once up front;
+                                   otherwise they are rebuilt per window of columns for every K/V row block (at least
+                                   one column per window). Same scores either way, up to fp32 rounding noise of the
+                                   different chunk shapes.                                                         */
 };
 
 /* Library-wide last error message (thread-local). */
@@ -112,6 +118,16 @@ VITED_API int vited_forward_pairs(vited_engine* e, const float* pairs, int B, fl
  * Entries that are not part of the mode's pair set (the diagonal, or j < i) are left untouched. */
 VITED_API int vited_score_grid(vited_engine* e, const float* images, int N, int mode, int row_begin, int row_end, float* out,
                      void* stream);
+/* vited_score_grid on the decoded bytes: images [N, S, S, in_chans] u8 (HWC, the crops a dataset yields; 1 byte per
+ * value against 4 for the f32 form, e.g. 0.79 MB against 3.15 MB per 512 x 512 RGB fragment); ToTensor +
+ * Normalize(.5, .5) (hisfrag.py:89-93, data/transforms.py:12-26) is applied while the patch matrix is formed, with the
+ * arithmetic of vited_normalize_u8, so the result is bit-identical to vited_score_grid on the normalised f32 images.
+ * Built for in_chans 3 and patch sizes 4, 8, 16, 32. Everything else as vited_score_grid.
+ * Device memory of one call beyond the images: the decoder input states of the columns, (N_e + 1) * embed_dim * 4
+ * bytes per column item, at most VITED_OPT_XSRC_BUDGET_MB; the K/V cache of one row block, at most
+ * VITED_OPT_KV_BUDGET_MB; and a workspace of about one decoder chunk (VITED_OPT_CHUNK_ROWS token rows). */
+VITED_API int vited_score_grid_u8(vited_engine* e, const uint8_t* images, int N, int mode, int row_begin, int row_end,
+                                  float* out, void* stream);
 
 /* number of kernels launched by this engine since creation (bench.py's gpu_launches) */
 VITED_API int64_t vited_launch_count(vited_engine* e);
@@ -261,6 +277,9 @@ VITED_API int vited_op_attention(const void* q, int q_ld, const void* k, int k_l
                        int k_has_cls, int n_kv_seq, const int32_t* kv_index, float scale, int impl, void* stream);
 /* images [B,C,S,S] f32 -> [B*(S/p)^2, C*p*p] h16 */
 VITED_API int vited_op_im2col(const float* images, void* out, int B, int C, int S, int p, void* stream);
+/* images [B,S,S,C] u8 -> the same [B*(S/p)^2, C*p*p] h16, bit-identical to vited_normalize_u8 + vited_op_im2col
+ * (C = 3, p in {4, 8, 16, 32}; `images` aligned to the largest power of two <= 16 that divides p*C) */
+VITED_API int vited_op_im2col_u8(const uint8_t* images, void* out, int B, int C, int S, int p, void* stream);
 
 #ifdef __cplusplus
 }

@@ -43,6 +43,7 @@ OPT_PRUNE_TAIL = 5
 OPT_FUSE_LN = 6
 OPT_KV_BUDGET_MB = 7
 OPT_FUSE_MLP = 8
+OPT_XSRC_BUDGET_MB = 9
 
 _vp = ctypes.c_void_p
 _i = ctypes.c_int
@@ -63,6 +64,7 @@ SIGNATURES = {
     "vited_decode": (_i, [_vp, _vp, _vp, _i, _vp, _vp]),
     "vited_forward_pairs": (_i, [_vp, _vp, _i, _vp, _vp]),
     "vited_score_grid": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp]),
+    "vited_score_grid_u8": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp]),
     "vited_profile_json": (ctypes.c_char_p, [_vp, _vp]),
     "vited_launch_count": (_i64, [_vp]),
     "vited_act_dtype": (_i, []),
@@ -93,6 +95,7 @@ SIGNATURES = {
     "vited_op_resid_ln": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _f, _vp]),
     "vited_op_attention": (_i, [_vp, _i, _vp, _i, _vp, _i, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _f, _i, _vp]),
     "vited_op_im2col": (_i, [_vp, _vp, _i, _i, _i, _i, _vp]),
+    "vited_op_im2col_u8": (_i, [_vp, _vp, _i, _i, _i, _i, _vp]),
 }
 
 

@@ -33,12 +33,12 @@ const char* get_error() { return g_err; }
 struct DevBuf {
   void* p = nullptr;
   size_t cap = 0;
-  int ensure(size_t bytes) {
+  int ensure(size_t bytes, bool headroom = true) {
     if (bytes <= cap) return 0;
     if (p) cudaFree(p);
     p = nullptr;
     cap = 0;
-    size_t want = bytes + (bytes >> 3);  // 12.5% headroom against re-allocation churn
+    size_t want = headroom ? bytes + (bytes >> 3) : bytes;  // 12.5% headroom against re-allocation churn
     cudaError_t e = cudaMalloc(&p, want);
     if (e != cudaSuccess) {
       set_error("cudaMalloc(%zu bytes) failed: %s", want, cudaGetErrorString(e));
@@ -96,6 +96,7 @@ struct vited_engine {
   int fuse_ln = 1;      // residual + LayerNorm in the epilogue of the N = 384 GEMMs (gemm_ln.cu)
   int fuse_mlp = 1;     // fc1 + GELU + fc2 + residual + LayerNorm in one kernel (mlp_ln.cu); needs fuse_ln
   int kv_budget_mb = 8000;  // K/V cache budget of one block of context rows in vited_score_grid
+  int64_t xsrc_budget_mb = 32000;  // decoder input states of one window of grid columns in vited_score_grid
   int64_t launches = 0;
   // optional per-kernel timing (bench.py's roofline): one event before every launch, intervals summed per class
   int profile = 0;
@@ -386,21 +387,28 @@ static int items_per_batch(vited_engine* e) {
   return (int)(n < 1 ? 1 : n);
 }
 
-// patch tokens of B images -> e->tok (fp16 [B*Ne, D]); img_stride = elements between consecutive images
-static int patch_tokens(vited_engine* e, const float* images, size_t img_stride, int B, cudaStream_t s) {
+// patch tokens of B images -> e->tok (fp16 [B*Ne, D]); img_stride = elements between consecutive images.
+// `u8`: the images are [B, S, S, in_chans] bytes (ToTensor + Normalize(.5, .5) applied on the way, im2col_u8_patches),
+// otherwise [B, in_chans, S, S] fp32.
+static int patch_tokens(vited_engine* e, const void* images, bool u8, size_t img_stride, int B, cudaStream_t s) {
   const vited_config& c = e->cfg;
   const size_t rows = (size_t)B * e->Ne;
   TRY(e->col.ensure(rows * e->Kpe * 2));
   TRY(e->tok.ensure(rows * e->D * 2));
   const size_t img_elems = (size_t)c.in_chans * c.img_size * c.img_size;
-  if (img_stride == img_elems) {
+  if (u8) {
+    VITED_CHECK(img_stride == img_elems, "patch_tokens: uint8 images must be contiguous");
+    prof_mark(e, "im2col_u8", 0.0, (double)rows * e->Kpe * 3.0, s);
+    TRY(im2col_u8_patches(static_cast<const uint8_t*>(images), e->col.as<act_t>(), B, c.in_chans, c.img_size,
+                          c.patch_size, s));
+  } else if (img_stride == img_elems) {
     prof_mark(e, "im2col", 0.0, (double)rows * e->Kpe * 6.0, s);
-    TRY(im2col_patches(images, e->col.as<act_t>(), B, c.in_chans, c.img_size, c.patch_size, s));
+    TRY(im2col_patches(static_cast<const float*>(images), e->col.as<act_t>(), B, c.in_chans, c.img_size, c.patch_size, s));
   } else {
     for (int b = 0; b < B; ++b) {
       prof_mark(e, "im2col", 0.0, (double)e->Ne * e->Kpe * 6.0, s);
-      TRY(im2col_patches(images + (size_t)b * img_stride, e->col.as<act_t>() + (size_t)b * e->Ne * e->Kpe, 1, c.in_chans,
-                         c.img_size, c.patch_size, s));
+      TRY(im2col_patches(static_cast<const float*>(images) + (size_t)b * img_stride,
+                         e->col.as<act_t>() + (size_t)b * e->Ne * e->Kpe, 1, c.in_chans, c.img_size, c.patch_size, s));
     }
   }
   TRY(L_gemm(e, e->col.as<act_t>(), e->patch, e->tok.as<act_t>(), (int)rows, ACT_NONE, s));
@@ -585,14 +593,14 @@ static int decode_chunk(vited_engine* e, int P, const int* ci, const int* xj, co
   return 0;
 }
 
-// pair list of grid rows [r0, r1) into e->ci / e->xj (generated on the device; nothing to upload or wait for)
-static int build_pair_list(vited_engine* e, int mode, int r0, int r1, int N, size_t* total, cudaStream_t s) {
-  *total = pair_list_count(mode, r0, r1, N);
+// pair list of grid rows [r0, r1) x columns [ca, cb) into e->ci / e->xj (generated on the device; nothing to upload or wait for)
+static int build_pair_list(vited_engine* e, int mode, int r0, int r1, int ca, int cb, size_t* total, cudaStream_t s) {
+  *total = pair_list_count(mode, r0, r1, ca, cb);
   if (*total == 0) return 0;
   TRY(e->ci.ensure(*total * sizeof(int) + 16));
   TRY(e->xj.ensure(*total * sizeof(int) + 16));
   prof_mark(e, "pair_list", 0.0, (double)*total * 8.0, s);
-  return pair_list(mode, r0, r1, N, e->ci.as<int>(), e->xj.as<int>(), s);
+  return pair_list(mode, r0, r1, ca, cb, e->ci.as<int>(), e->xj.as<int>(), s);
 }
 
 }  // namespace vited
@@ -667,6 +675,10 @@ int vited_set_option(vited_engine* e, int option, int64_t value) {
       VITED_CHECK(value >= 1, "kv budget must be positive");
       e->kv_budget_mb = value;
       return 0;
+    case VITED_OPT_XSRC_BUDGET_MB:
+      VITED_CHECK(value >= 1, "column state budget must be positive");
+      e->xsrc_budget_mb = value;
+      return 0;
     case VITED_OPT_PROFILE:
       e->profile = value ? 1 : 0;
       e->recs.clear();
@@ -714,7 +726,7 @@ int vited_encode(vited_engine* e, const float* images, int B, float* out_tokens,
   const int step = items_per_batch(e);
   for (int i0 = 0; i0 < B; i0 += step) {
     const int n = (B - i0 < step) ? (B - i0) : step;
-    TRY(patch_tokens(e, images + (size_t)i0 * img, img, n, s));
+    TRY(patch_tokens(e, images + (size_t)i0 * img, false, img, n, s));
     TRY(encoder_stack(e, n, out_tokens + (size_t)i0 * e->Ne * e->D, s));
   }
   return 0;
@@ -726,13 +738,13 @@ static int decode_impl(vited_engine* e, const float* ctx_tokens, const float* im
   for (int i0 = 0; i0 < B; i0 += step) {
     const int n = (B - i0 < step) ? (B - i0) : step;
     // decoder input state of the n x2 images
-    TRY(patch_tokens(e, images + (size_t)i0 * img_stride, img_stride, n, s));
+    TRY(patch_tokens(e, images + (size_t)i0 * img_stride, false, img_stride, n, s));
     TRY(decoder_item_state(e, n, s));
     TRY(e->xsrc.ensure((size_t)n * e->Nd * e->D * 4));
     VITED_CUDA_OK(cudaMemcpyAsync(e->xsrc.p, e->x.p, (size_t)n * e->Nd * e->D * 4, cudaMemcpyDeviceToDevice, s));
     TRY(build_kv(e, ctx_tokens + (size_t)i0 * e->Ne * e->D, n, s));
     size_t total = 0;
-    TRY(build_pair_list(e, 2, 0, n, n, &total, s));   // pair p: context p, decoder state p
+    TRY(build_pair_list(e, 2, 0, n, 0, n, &total, s));   // pair p: context p, decoder state p
     HeadArgs head = {};
     head.out = out_logits + (size_t)i0 * e->C;
     head.ci = nullptr; head.xj = nullptr; head.row_begin = 0; head.n_items = 0;
@@ -761,39 +773,59 @@ int vited_forward_pairs(vited_engine* e, const float* pairs, int B, float* out_l
     const int n = (B - i0 < step) ? (B - i0) : step;
     const float* base = pairs + (size_t)i0 * 2 * img;
     TRY(e->tmp_tok.ensure((size_t)n * e->Ne * e->D * 4));
-    TRY(patch_tokens(e, base, 2 * img, n, s));            // x1 = pairs[:, 0]
+    TRY(patch_tokens(e, base, false, 2 * img, n, s));            // x1 = pairs[:, 0]
     TRY(encoder_stack(e, n, e->tmp_tok.as<float>(), s));
     TRY(decode_impl(e, e->tmp_tok.as<float>(), base + img, 2 * img, n, out_logits + (size_t)i0 * e->C, s));  // x2 = pairs[:, 1]
   }
   return 0;
 }
 
-int vited_score_grid(vited_engine* e, const float* images, int N, int mode, int row_begin, int row_end, float* out,
-                     void* stream) {
+// decoder input states of items [ca, cb) -> e->xsrc (split layout, cb - ca sequences)
+static int build_xsrc(vited_engine* e, const char* images, bool u8, size_t img_bytes, int ca, int cb, bool headroom,
+                      cudaStream_t s) {
+  const int n_src = cb - ca;
+  const size_t img = (size_t)e->cfg.in_chans * e->cfg.img_size * e->cfg.img_size;
+  const int step = items_per_batch(e);
+  TRY(e->xsrc.ensure((size_t)n_src * e->Nd * e->D * 4, headroom));
+  for (int i0 = 0; i0 < n_src; i0 += step) {
+    const int n = (n_src - i0 < step) ? (n_src - i0) : step;
+    TRY(patch_tokens(e, images + (size_t)(ca + i0) * img_bytes, u8, img, n, s));
+    TRY(decoder_item_state(e, n, s));
+    TRY(scatter_split(e, e->xsrc.as<float>(), n_src, i0, n, s));
+  }
+  return 0;
+}
+
+// vited_score_grid / vited_score_grid_u8: one grid loop for both image formats
+static int score_grid_impl(vited_engine* e, const void* images_in, bool u8, int N, int mode, int row_begin, int row_end,
+                           float* out, cudaStream_t s) {
   TRY(check_ready(e));
   DeviceScope scope(e->device);
   VITED_CHECK(mode == VITED_GRID_ORDERED_OFFDIAG || mode == VITED_GRID_UPPER_TRI_DIAG, "unknown grid mode %d", mode);
   VITED_CHECK(N >= 0 && row_begin >= 0 && row_begin <= row_end && row_end <= N, "bad row range [%d, %d) for N=%d",
               row_begin, row_end, N);
   if (N == 0 || row_begin == row_end) return 0;
-  VITED_CHECK(images && out, "vited_score_grid: null pointer");
-  cudaStream_t s = (cudaStream_t)stream;
+  VITED_CHECK(images_in && out, "vited_score_grid: null pointer");
+  const char* images = static_cast<const char*>(images_in);
   const size_t img = (size_t)e->cfg.in_chans * e->cfg.img_size * e->cfg.img_size;
+  const size_t img_bytes = img * (u8 ? 1 : 4);
   const size_t D = e->D, Ne = e->Ne, Nd = e->Nd;
   const int step = items_per_batch(e);
+  const int pair_mode = mode == VITED_GRID_ORDERED_OFFDIAG ? 0 : 1;
 
   // 1) decoder input state of every item that appears as a COLUMN of this row shard: computed once per item, reused
   //    by every pair. The upper-triangular grid (hisfrag.py:166-167) never pairs a row with a column j < row_begin,
-  //    so a row shard builds (and holds) only the states of items [row_begin, N).
+  //    so a row shard builds (and holds) only the states of items [row_begin, N). When those states exceed the
+  //    budget (default 32 GB: 20,345 Hisfrag items at 1.57 MB), they are built per column window of at most the
+  //    budget, inside the loop over K/V row blocks below; otherwise once, here, for the whole call.
   const int c0 = (mode == VITED_GRID_UPPER_TRI_DIAG) ? row_begin : 0;
   const int n_cols = N - c0;
-  TRY(e->xsrc.ensure((size_t)n_cols * Nd * D * 4));
-  for (int i0 = 0; i0 < n_cols; i0 += step) {
-    const int n = (n_cols - i0 < step) ? (n_cols - i0) : step;
-    TRY(patch_tokens(e, images + (size_t)(c0 + i0) * img, img, n, s));
-    TRY(decoder_item_state(e, n, s));
-    TRY(scatter_split(e, e->xsrc.as<float>(), n_cols, i0, n, s));
-  }
+  const size_t xsrc_bytes_per_item = Nd * D * 4;
+  int64_t cw = (int64_t)((size_t)e->xsrc_budget_mb * 1000000 / xsrc_bytes_per_item);
+  if (cw < 1) cw = 1;
+  const bool one_window = n_cols <= cw;
+  const int win = one_window ? n_cols : (int)cw;
+  if (one_window) TRY(build_xsrc(e, images, u8, img_bytes, c0, N, true, s));
 
   // 2) context rows in blocks whose K/V cache stays within the budget (default 8 GB)
   const size_t kv_bytes_per_item = e->dec.size() * Ne * 2 * D * 2;
@@ -807,29 +839,45 @@ int vited_score_grid(vited_engine* e, const float* images, int N, int mode, int 
     TRY(e->enc_tok.ensure((size_t)nr * Ne * D * 4));
     for (int i0 = 0; i0 < nr; i0 += step) {
       const int n = (nr - i0 < step) ? (nr - i0) : step;
-      TRY(patch_tokens(e, images + (size_t)(r0 + i0) * img, img, n, s));
+      TRY(patch_tokens(e, images + (size_t)(r0 + i0) * img_bytes, u8, img, n, s));
       TRY(encoder_stack(e, n, e->enc_tok.as<float>() + (size_t)i0 * Ne * D, s));
     }
     TRY(build_kv(e, e->enc_tok.as<float>(), nr, s));
-    // pair list of the block, i-major (data/datasets/pieces_dataset.py:27-32 / hisfrag.py:166-167)
-    size_t total = 0;
-    TRY(build_pair_list(e, mode == VITED_GRID_ORDERED_OFFDIAG ? 0 : 1, r0, r1, N, &total, s));
-    if (total == 0) continue;
-    // equal chunks: a short last chunk would run every kernel of the stack at a fraction of a wave
-    const size_t n_chunks = (total + pairs_per_chunk - 1) / pairs_per_chunk;
-    const size_t chunk = (total + n_chunks - 1) / n_chunks;
-    for (size_t p0 = 0; p0 < total; p0 += chunk) {
-      const int P = (int)((total - p0 < chunk) ? (total - p0) : chunk);
-      HeadArgs head = {};
-      head.out = out + (size_t)(r0 - row_begin) * N * e->C;
-      head.ci = e->ci.as<int>() + p0;
-      head.xj = e->xj.as<int>() + p0;
-      head.row_begin = 0;  // ci is already relative to r0
-      head.n_items = N;
-      TRY(decode_chunk(e, P, e->ci.as<int>() + p0, e->xj.as<int>() + p0, e->xsrc.as<float>(), n_cols, c0, nr, head, s));
+    for (int ca = c0; ca < N; ca += win) {
+      const int cb = (ca + win < N) ? (ca + win) : N;
+      if (mode == VITED_GRID_UPPER_TRI_DIAG && cb <= r0) continue;   // no column of the window pairs with these rows
+      if (!one_window) TRY(build_xsrc(e, images, u8, img_bytes, ca, cb, false, s));
+      // pair list of the block x window, i-major (data/datasets/pieces_dataset.py:27-32 / hisfrag.py:166-167)
+      size_t total = 0;
+      TRY(build_pair_list(e, pair_mode, r0, r1, ca, cb, &total, s));
+      if (total == 0) continue;
+      // equal chunks: a short last chunk would run every kernel of the stack at a fraction of a wave
+      const size_t n_chunks = (total + pairs_per_chunk - 1) / pairs_per_chunk;
+      const size_t chunk = (total + n_chunks - 1) / n_chunks;
+      for (size_t p0 = 0; p0 < total; p0 += chunk) {
+        const int P = (int)((total - p0 < chunk) ? (total - p0) : chunk);
+        HeadArgs head = {};
+        head.out = out + (size_t)(r0 - row_begin) * N * e->C;
+        head.ci = e->ci.as<int>() + p0;
+        head.xj = e->xj.as<int>() + p0;
+        head.row_begin = 0;  // ci is already relative to r0
+        head.n_items = N;
+        TRY(decode_chunk(e, P, e->ci.as<int>() + p0, e->xj.as<int>() + p0, e->xsrc.as<float>(), cb - ca, ca, nr, head,
+                         s));
+      }
     }
   }
   return 0;
+}
+
+int vited_score_grid(vited_engine* e, const float* images, int N, int mode, int row_begin, int row_end, float* out,
+                     void* stream) {
+  return score_grid_impl(e, images, false, N, mode, row_begin, row_end, out, (cudaStream_t)stream);
+}
+
+int vited_score_grid_u8(vited_engine* e, const uint8_t* images, int N, int mode, int row_begin, int row_end, float* out,
+                        void* stream) {
+  return score_grid_impl(e, images, true, N, mode, row_begin, row_end, out, (cudaStream_t)stream);
 }
 
 const char* vited_profile_json(vited_engine* e, void* stream) {
@@ -920,6 +968,10 @@ int vited_op_attention(const void* q, int q_ld, const void* k, int k_ld, const v
 
 int vited_op_im2col(const float* images, void* out, int B, int C, int S, int p, void* stream) {
   return im2col_patches(images, (act_t*)out, B, C, S, p, (cudaStream_t)stream);
+}
+
+int vited_op_im2col_u8(const uint8_t* images, void* out, int B, int C, int S, int p, void* stream) {
+  return im2col_u8_patches(images, (act_t*)out, B, C, S, p, (cudaStream_t)stream);
 }
 
 // ---- training-step kernels (train_ops.cu) ----

@@ -68,6 +68,9 @@ int resid_ln(const ResidLnArgs& a, cudaStream_t stream);
 
 // images [B,3,S,S] f32 -> patch matrix [B*G*G, 3*p*p] fp16, column = c*p*p + py*p + px (Conv2d weight.view order)
 int im2col_patches(const float* images, act_t* out, int B, int C, int S, int p, cudaStream_t stream);
+// images [B,S,S,C] u8 (HWC bytes) -> the same patch matrix, bit-identical to normalize_u8 + im2col_patches
+// (ToTensor + Normalize(.5, .5) folded in). Built for C = 3 and p in {4, 8, 16, 32}; anything else is an error.
+int im2col_u8_patches(const uint8_t* images, act_t* out, int B, int C, int S, int p, cudaStream_t stream);
 
 // x0 (f32, split layout, B sequences): patch rows = tok (fp16 [B*Np, D]) + pos[1+t]; cls rows = cls + pos[0]
 int assemble_tokens(const act_t* tok, const float* pos_embed, const float* cls_token, float* x, int B, int n_patch,
@@ -90,13 +93,14 @@ struct HeadArgs {
 };
 int head_logits(const HeadArgs& a, cudaStream_t stream);
 
-// pair list of grid rows [r0, r1) on the device, i-major: ci[p] = i - r0 (context row inside the block), xj[p] = j.
-//   mode 0: ordered off-diagonal pairs, j in [0, N) \ {i}  (data/datasets/pieces_dataset.py:27-32)
-//   mode 1: upper triangle incl. diagonal, j in [i, N)       (hisfrag.py:166-167)
-//   mode 2: identity, ci[p] = xj[p] = p for p in [0, r1 - r0)  (two-phase / one-shot decode of B pairs)
-// pair_list_count returns the number of pairs (the caller sizes ci / xj with it).
-size_t pair_list_count(int mode, int r0, int r1, int N);
-int pair_list(int mode, int r0, int r1, int N, int* ci, int* xj, cudaStream_t stream);
+// pair list of grid rows [r0, r1) x column window [ca, cb) on the device, i-major with j ascending:
+// ci[p] = i - r0 (context row inside the block), xj[p] = j (absolute item index).
+//   mode 0: ordered off-diagonal pairs, j in [ca, cb) \ {i}  (data/datasets/pieces_dataset.py:27-32)
+//   mode 1: upper triangle incl. diagonal, j in [max(i, ca), cb)  (hisfrag.py:166-167)
+//   mode 2: identity, ci[p] = xj[p] = p for p in [0, r1 - r0)  (two-phase / one-shot decode of B pairs; window unused)
+// The whole grid row is the window [0, N). pair_list_count returns the number of pairs (the caller sizes ci / xj with it).
+__host__ __device__ size_t pair_list_count(int mode, int r0, int r1, int ca, int cb);
+int pair_list(int mode, int r0, int r1, int ca, int cb, int* ci, int* xj, cudaStream_t stream);
 
 // plain copy/convert helpers
 int f32_to_act(const float* in, act_t* out, size_t n, cudaStream_t stream);

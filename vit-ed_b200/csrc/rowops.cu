@@ -43,6 +43,92 @@ int im2col_patches(const float* images, act_t* out, int B, int C, int S, int p, 
   return 0;
 }
 
+// The same patch matrix straight from the decoded bytes [B, S, S, C] (HWC uint8), with the normalisation of
+// normalize_u8_kernel (ToTensor + Normalize(.5, .5), hisfrag.py:89-93) folded in. A byte has 256 values, so every
+// block first evaluates that arithmetic once per value into a shared table of 16-bit results (rounded by pack_act,
+// as im2col_kernel rounds): the output is bit-identical to normalize_u8 followed by im2col_patches.
+// One thread = one pixel row of one patch: P*C contiguous bytes (48 at P = 16), loaded as VB-byte vectors and
+// de-interleaved in registers, then P 16-bit values per channel stored contiguously. gx runs fastest across a warp,
+// so a warp reads whole pixel rows and every thread writes whole 32-byte sectors.
+template <int P, int C, int VB>
+__global__ void __launch_bounds__(256) im2col_u8_kernel(const uint8_t* __restrict__ img, act_t* __restrict__ out,
+                                                        int B, int S) {
+  __shared__ uint16_t lut[256];
+  for (int v = threadIdx.x; v < 256; v += blockDim.x) {
+    const float f = __fdiv_rn(__fsub_rn(__fdiv_rn((float)v, 255.0f), 0.5f), 0.5f);
+    lut[v] = (uint16_t)(pack_act(f, f) & 0xffffu);
+  }
+  __syncthreads();
+  constexpr int NB = P * C;             // bytes of one patch pixel row
+  constexpr int K = C * P * P;
+  static_assert(NB % VB == 0 && NB % 4 == 0 && P % 4 == 0, "patch row must split into whole vectors");
+  const int G = S / P;
+  const size_t total = (size_t)B * S * G;   // (b, gy, py, gx), gx fastest
+  for (size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
+    const int gx = (int)(idx % G);
+    const size_t by = idx / G;              // b * S + gy * P + py: the pixel row
+    const int y = (int)(by % S);
+    const size_t b = by / S;
+    const int gy = y / P, py = y % P;
+    uint32_t w[NB / 4];
+    const uint8_t* src = img + (by * S + (size_t)gx * P) * C;
+#pragma unroll
+    for (int k = 0; k < NB / VB; ++k) {
+      if constexpr (VB == 16) {
+        const uint4 v = *reinterpret_cast<const uint4*>(src + k * 16);
+        w[4 * k] = v.x; w[4 * k + 1] = v.y; w[4 * k + 2] = v.z; w[4 * k + 3] = v.w;
+      } else if constexpr (VB == 8) {
+        const uint2 v = *reinterpret_cast<const uint2*>(src + k * 8);
+        w[2 * k] = v.x; w[2 * k + 1] = v.y;
+      } else {
+        w[k] = *reinterpret_cast<const uint32_t*>(src + k * 4);
+      }
+    }
+    const size_t row = (b * G + gy) * G + gx;
+    act_t* dst = out + row * K + py * P;
+#pragma unroll
+    for (int c = 0; c < C; ++c) {
+      uint32_t o[P / 2];
+#pragma unroll
+      for (int px = 0; px < P; px += 2) {
+        const int i0 = px * C + c, i1 = (px + 1) * C + c;     // byte of (px, c) inside the loaded row
+        const uint32_t lo = lut[(w[i0 >> 2] >> (8 * (i0 & 3))) & 0xffu];
+        const uint32_t hi = lut[(w[i1 >> 2] >> (8 * (i1 & 3))) & 0xffu];
+        o[px / 2] = lo | (hi << 16);
+      }
+      act_t* d = dst + c * P * P;
+#pragma unroll
+      for (int k = 0; k < P / 8; ++k)
+        *reinterpret_cast<uint4*>(d + 8 * k) = make_uint4(o[4 * k], o[4 * k + 1], o[4 * k + 2], o[4 * k + 3]);
+      if constexpr (P % 8 != 0) *reinterpret_cast<uint2*>(d + P - 4) = make_uint2(o[P / 2 - 2], o[P / 2 - 1]);
+    }
+  }
+}
+
+int im2col_u8_patches(const uint8_t* images, act_t* out, int B, int C, int S, int p, cudaStream_t stream) {
+  VITED_CHECK(B >= 0 && p > 0 && S % p == 0, "im2col_u8: patch size %d must divide img size %d", p, S);
+  const size_t total = (size_t)B * S * (S / p);
+  if (total == 0) return 0;
+  int blocks = (int)((total + 255) / 256);
+  if (blocks > 148 * 16) blocks = 148 * 16;
+  // a pixel row of one patch starts at a multiple of p*C bytes; the vector width must divide that and the pointer
+  const uintptr_t a = (uintptr_t)images;
+#define VITED_IM2COL_U8(P_, C_, VB_)                                                                    \
+  if (p == P_ && C == C_) {                                                                             \
+    VITED_CHECK(a % VB_ == 0, "im2col_u8: images must be %d-byte aligned for patch %d", VB_, P_);       \
+    im2col_u8_kernel<P_, C_, VB_><<<blocks, 256, 0, stream>>>(images, out, B, S);                       \
+    VITED_CUDA_OK(cudaGetLastError());                                                                  \
+    return 0;                                                                                           \
+  }
+  VITED_IM2COL_U8(16, 3, 16)
+  VITED_IM2COL_U8(8, 3, 8)
+  VITED_IM2COL_U8(32, 3, 16)
+  VITED_IM2COL_U8(4, 3, 4)
+#undef VITED_IM2COL_U8
+  set_error("im2col_u8: no kernel for patch size %d with %d channels (built for 4, 8, 16, 32 with 3)", p, C);
+  return 1;
+}
+
 // ------------------------------------------------------------------------------------------------------------
 // x0 = patch tokens + pos_embed[:, 1:]  (vision_transformer.py:378-380);  cls row = cls_token + pos_embed[:, 0]
 // (timm _pos_embed, called at :392).  Split layout: B*Np patch rows, then B cls rows.
@@ -280,41 +366,47 @@ int head_logits(const HeadArgs& a, cudaStream_t stream) {
 // ------------------------------------------------------------------------------------------------------------
 // pair lists of a block of grid rows, generated where they are consumed (no host vectors, no upload, no sync)
 // ------------------------------------------------------------------------------------------------------------
-size_t pair_list_count(int mode, int r0, int r1, int N) {
+__host__ __device__ size_t pair_list_count(int mode, int r0, int r1, int ca, int cb) {
   const size_t nr = (size_t)(r1 - r0);
-  if (mode == 0) return nr * (size_t)(N - 1);
-  if (mode == 1) return nr * (size_t)N - ((size_t)r1 * (r1 - 1) - (size_t)r0 * (r0 - 1)) / 2;
+  if (mode == 0) {     // nr * (cb - ca) minus the diagonal entries inside the window
+    const int lo = r0 > ca ? r0 : ca, hi = r1 < cb ? r1 : cb;
+    return nr * (size_t)(cb - ca) - (size_t)(hi > lo ? hi - lo : 0);
+  }
+  if (mode == 1) {     // rows i < ca see the whole window, rows i in [ca, cb) see [i, cb)
+    const int below = (r1 < ca ? r1 : ca) - r0;
+    const int lo = r0 > ca ? r0 : ca, hi = r1 < cb ? r1 : cb;
+    size_t n = below > 0 ? (size_t)below * (size_t)(cb - ca) : 0;
+    if (hi > lo) n += (size_t)(hi - lo) * (size_t)cb - ((size_t)lo + hi - 1) * (size_t)(hi - lo) / 2;
+    return n;
+  }
   return nr;
 }
 
-__global__ void __launch_bounds__(256) pair_list_kernel(int mode, int r0, int r1, int N, int* __restrict__ ci,
+__global__ void __launch_bounds__(256) pair_list_kernel(int mode, int r0, int r1, int ca, int cb, int* __restrict__ ci,
                                                         int* __restrict__ xj) {
   for (int i = r0 + (int)blockIdx.x; i < r1; i += (int)gridDim.x) {
     if (mode == 2) {
       if (threadIdx.x == 0) { ci[i - r0] = i - r0; xj[i - r0] = i - r0; }
       continue;
     }
-    size_t off;
-    int j0, len;
-    if (mode == 0) {
-      off = (size_t)(i - r0) * (N - 1); j0 = 0; len = N - 1;
-    } else {
-      off = (size_t)(i - r0) * N - ((size_t)i * (i - 1) - (size_t)r0 * (r0 - 1)) / 2; j0 = i; len = N - i;
-    }
+    const size_t off = pair_list_count(mode, r0, i, ca, cb);
+    const int len = (int)pair_list_count(mode, i, i + 1, ca, cb);
+    const int j0 = (mode == 0 || i < ca) ? ca : i;
+    const bool skip_diag = (mode == 0) && i >= ca;
     for (int t = threadIdx.x; t < len; t += blockDim.x) {
-      const int j = (mode == 0) ? t + (t >= i ? 1 : 0) : j0 + t;
+      const int j = j0 + t + ((skip_diag && j0 + t >= i) ? 1 : 0);
       ci[off + t] = i - r0;
       xj[off + t] = j;
     }
   }
 }
 
-int pair_list(int mode, int r0, int r1, int N, int* ci, int* xj, cudaStream_t stream) {
-  VITED_CHECK(mode >= 0 && mode <= 2 && r0 >= 0 && r0 <= r1, "pair_list: bad arguments");
+int pair_list(int mode, int r0, int r1, int ca, int cb, int* ci, int* xj, cudaStream_t stream) {
+  VITED_CHECK(mode >= 0 && mode <= 2 && r0 >= 0 && r0 <= r1 && ca >= 0 && ca <= cb, "pair_list: bad arguments");
   if (r1 == r0) return 0;
   int blocks = r1 - r0;
   if (blocks > 148 * 8) blocks = 148 * 8;
-  pair_list_kernel<<<blocks, 256, 0, stream>>>(mode, r0, r1, N, ci, xj);
+  pair_list_kernel<<<blocks, 256, 0, stream>>>(mode, r0, r1, ca, cb, ci, xj);
   VITED_CUDA_OK(cudaGetLastError());
   return 0;
 }

@@ -51,9 +51,38 @@ def indicates_row_ranges(indexes, num_replicas):
     return sizes
 
 
+def hisfrag_row_ranges(n, num_replicas):
+    """``indicates_row_ranges(upper_tri_pairs(n)[:, 0], num_replicas)`` in O(num_replicas) Python integer operations,
+    without the n(n+1)/2-entry pair list (200 M pairs, gigabytes of host arrays, at 20,000 fragments). Row a of the
+    upper-triangular grid holds pair indices [off(a), off(a + 1)) with off(a) = a*n - a(a-1)/2; the row of a pair index
+    is the inverse of that quadratic (math.isqrt, then a +-1 fix-up for the rounding of the root)."""
+    n_pairs = n * (n + 1) // 2
+    n_per = -(-n_pairs // num_replicas)
+
+    def off(a):
+        return a * n - a * (a - 1) // 2
+
+    def row(k):
+        b = 2 * n + 1
+        a = (b - math.isqrt(b * b - 8 * k)) // 2
+        while a > 0 and off(a) > k:
+            a -= 1
+        while off(a + 1) <= k:
+            a += 1
+        return a
+
+    starts = range(0, n_pairs, n_per)      # the reference's chunk starts (ValueError for an empty grid, as there)
+    sizes = [0]
+    for c in range(1, len(starts)):
+        first, prev_last = row(starts[c]), row(starts[c] - 1)
+        sizes.append(first - 1 if first == prev_last else first)
+    sizes.append(row(n_pairs - 1) + 1)
+    return sizes
+
+
 def hisfrag_row_range(n, world, rank):
     """Rows of the upper-triangular grid owned by ``rank`` (hisfrag.py:166-170)."""
-    sizes = indicates_row_ranges(upper_tri_pairs(n)[:, 0], world)
+    sizes = hisfrag_row_ranges(n, world)
     if rank + 1 >= len(sizes):
         return n, n  # fewer chunks than ranks: this rank has nothing (the reference would raise IndexError)
     return sizes[rank], sizes[rank + 1]
@@ -175,9 +204,15 @@ def score_puzzles(model, puzzles, n_pieces=None, gather=True, blocks_out=None):
 
 
 @torch.no_grad()
-def score_fragments(model, images, gather=True, resume_path=None, block_rows=64, save_every=5, remove_cache_file=False):
-    """images [N,3,S,S] -> symmetric similarity logits [N, N] fp32 (raw logits, no sigmoid: hisfrag.py:230-231,
+def score_fragments(model, images, gather=True, resume_path=None, block_rows=64, save_every=5, remove_cache_file=False,
+                    xsrc_budget_mb=None):
+    """images [N,3,S,S] fp32, or the uint8 crops [N,S,S,3] of ``pieces.fragments_to_u8_device`` (same scores, a
+    quarter of the memory) -> symmetric similarity logits [N, N] fp32 (raw logits, no sigmoid: hisfrag.py:230-231,
     :281-292). Rows are sharded as DistributedIndicatesSampler does (hisfrag.py:170).
+
+    ``xsrc_budget_mb`` (None: leave the engine's setting) bounds the decoder input states of the grid columns held at
+    once (``OPT_XSRC_BUDGET_MB``, default 32,000 MB = 20,345 Hisfrag fragments); a larger grid is scored in column
+    windows of that size.
 
     ``resume_path`` switches on the crash-resume of the reference's test loop (hisfrag.py:181-195, :243-246): the
     rank's rows are then walked in blocks of ``block_rows`` rows (the reference's x1 batches), after every
@@ -187,10 +222,12 @@ def score_fragments(model, images, gather=True, resume_path=None, block_rows=64,
     written for another grid size or row range is an error, not silently reused."""
     rank, world = _dist_info()
     n = images.shape[0]
+    if xsrc_budget_mb is not None:
+        model.set_option(_lib.OPT_XSRC_BUDGET_MB, xsrc_budget_mb)
     if world == 1:
         ranges = [(0, n)]
     else:
-        sizes = indicates_row_ranges(upper_tri_pairs(n)[:, 0], world)
+        sizes = hisfrag_row_ranges(n, world)
         if any(a > b for a, b in zip(sizes, sizes[1:])):
             # for grids of a dozen items the reference sampler's row snapping (samplers.py:113-134) yields boundaries
             # that run backwards; every rank sees the same `sizes`, so all of them stop here, before any collective

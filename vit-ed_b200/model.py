@@ -334,9 +334,22 @@ class VisionTransformerCustom(nn.Module):
     @torch.no_grad()
     def score_grid(self, images, mode, row_begin=0, row_end=None, out=None):
         """All pairs of grid rows [row_begin, row_end) against all N items -> [rows, N, num_classes] fp32.
-        Replaces the inner loops of evaluation.py:101-114 / hisfrag.py:189-231 (see grid.py for the callers)."""
-        images = self._prep(images)
-        self._check_images(images)
+        Replaces the inner loops of evaluation.py:101-114 / hisfrag.py:189-231 (see grid.py for the callers).
+
+        ``images`` is either the model input [N, in_chans, S, S] (fp32) or the decoded crops [N, S, S, in_chans] as a
+        CUDA uint8 tensor: ToTensor + Normalize(.5, .5) then runs inside the patch embedding (C-ABI
+        ``vited_score_grid_u8``), bit-identical to scoring the normalised fp32 images, at a quarter of their memory."""
+        if images.dtype == torch.uint8:
+            want = (self.img_size, self.img_size, self.in_chans)
+            if images.dim() != 4 or tuple(images.shape[1:]) != want or not images.is_cuda:
+                raise ValueError(f'uint8 images must be a CUDA tensor [N, {want[0]}, {want[1]}, {want[2]}] (HWC crops), '
+                                 f'got {tuple(images.shape)} on {images.device}')
+            images = images.contiguous()
+            entry, name = _lib.lib.vited_score_grid_u8, 'vited_score_grid_u8'
+        else:
+            images = self._prep(images)
+            self._check_images(images)
+            entry, name = _lib.lib.vited_score_grid, 'vited_score_grid'
         n = images.shape[0]
         row_end = n if row_end is None else row_end
         if not (0 <= row_begin <= row_end <= n):
@@ -344,8 +357,8 @@ class VisionTransformerCustom(nn.Module):
         eng = self._ensure_engine(images.device)
         if out is None:
             out = torch.zeros((row_end - row_begin, n, self.num_classes), dtype=torch.float32, device=images.device)
-        _lib.check(_lib.lib.vited_score_grid(eng, images.data_ptr(), n, int(mode), int(row_begin), int(row_end),
-                                             out.data_ptr(), self._stream(images.device)), 'vited_score_grid')
+        _lib.check(entry(eng, images.data_ptr(), n, int(mode), int(row_begin), int(row_end), out.data_ptr(),
+                         self._stream(images.device)), name)
         return out
 
 

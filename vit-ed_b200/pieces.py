@@ -123,6 +123,18 @@ def center_crop_u8(img, size):
     return img[top:top + size, left:left + size]
 
 
+def fragments_to_u8_device(images, img_size=512, device='cuda'):
+    """List of PIL images / [H, W, 3] uint8 arrays -> CUDA uint8 [N, S, S, 3]: the CenterCrop of the Hisfrag20
+    test-time preparation done on the bytes, then one upload. ``model.score_grid`` and ``grid.score_fragments`` take
+    this directly and normalise inside the patch embedding: a quarter of the device memory of the fp32 batch that
+    ``fragments_to_batch_device`` returns, identical scores."""
+    from . import _lib
+    crops = np.stack([center_crop_u8(np.asarray(im), img_size) for im in images])
+    if crops.dtype != np.uint8 or crops.shape[1:] != (img_size, img_size, 3):
+        raise _lib.VitedError(f'fragments_to_u8_device: expected uint8 RGB images, got {crops.dtype} {crops.shape}')
+    return torch.from_numpy(np.ascontiguousarray(crops)).to(torch.device(device))
+
+
 def fragments_to_batch_device(images, img_size=512, device='cuda'):
     """List of PIL images / [H, W, 3] uint8 arrays -> CUDA fp32 [N, 3, S, S]: the Hisfrag20 test-time preparation
     (SURVEY 8a row a6; ``fragment_to_tensor`` is the per-image host version) with the crop done on the bytes and
@@ -130,14 +142,11 @@ def fragments_to_batch_device(images, img_size=512, device='cuda'):
     import ctypes
 
     from . import _lib
-    crops = np.stack([center_crop_u8(np.asarray(im), img_size) for im in images])
-    if crops.dtype != np.uint8 or crops.shape[1:] != (img_size, img_size, 3):
-        raise _lib.VitedError(f'fragments_to_batch_device: expected uint8 RGB images, got {crops.dtype} {crops.shape}')
     dev = torch.device(device)
     with torch.cuda.device(dev):
-        src = torch.from_numpy(np.ascontiguousarray(crops)).to(dev)
-        out = torch.empty((len(crops), 3, img_size, img_size), dtype=torch.float32, device=dev)
-        _lib.check(_lib.lib.vited_normalize_u8(ctypes.c_void_p(src.data_ptr()), len(crops), img_size,
+        src = fragments_to_u8_device(images, img_size, dev)
+        out = torch.empty((src.shape[0], 3, img_size, img_size), dtype=torch.float32, device=dev)
+        _lib.check(_lib.lib.vited_normalize_u8(ctypes.c_void_p(src.data_ptr()), src.shape[0], img_size,
                                                ctypes.c_void_p(out.data_ptr()),
                                                ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)),
                    'vited_normalize_u8')
