@@ -129,6 +129,26 @@ VITED_API int vited_score_grid(vited_engine* e, const float* images, int N, int 
 VITED_API int vited_score_grid_u8(vited_engine* e, const uint8_t* images, int N, int mode, int row_begin, int row_end,
                                   float* out, void* stream);
 
+/* replaces: the `sub_pairs` batches of hisfrag.py:221-229 and a one-shot pass over a pair dataset -- any pair list, with
+ * every item encoded and its decoder input state built once per call, as the grid does.
+ * images [N, in_chans, S, S] f32 (vited_score_pairs) or [N, S, S, in_chans] u8 (vited_score_pairs_u8, the format and
+ * normalisation of vited_score_grid_u8);
+ * pairs  [n_pairs, 2] i32 (device): (context item a, decoder item b), indices into images[0..N);
+ * out    [n_pairs, num_classes] f32: out[p] = logits of model(tokens(images[a]), images[b]), the (a, b) entry of
+ *        vited_score_grid. Any order; duplicates, a == b and a > b are allowed.
+ * Only the items the list references are read and computed: its distinct context items in blocks of at most
+ * VITED_OPT_KV_BUDGET_MB of K/V cache, its distinct decoder items in windows of at most VITED_OPT_XSRC_BUDGET_MB of
+ * decoder input states. Pairs are bucketed by (block, window) on the device with a stable sort, so the same list always
+ * gives the same bits; a dense grid's own pair set in its i-major order gives vited_score_grid's bits.
+ * Synchronises `stream` once (to size its loops); an index outside [0, N) is an error reported before anything is
+ * scored (out untouched), its message names the first such pair. n_pairs == 0 does nothing; n_pairs > INT32_MAX is an
+ * error. Device memory of one call: about 20 bytes per pair (the caller's list and three sorted index arrays), 24 bytes
+ * per item of N, on top of what vited_score_grid holds. */
+VITED_API int vited_score_pairs(vited_engine* e, const float* images, int N, const int32_t* pairs, int64_t n_pairs,
+                                float* out, void* stream);
+VITED_API int vited_score_pairs_u8(vited_engine* e, const uint8_t* images, int N, const int32_t* pairs,
+                                   int64_t n_pairs, float* out, void* stream);
+
 /* number of kernels launched by this engine since creation (bench.py's gpu_launches) */
 VITED_API int64_t vited_launch_count(vited_engine* e);
 /* Per-kernel-class device time since profiling was switched on / last read, as a JSON object

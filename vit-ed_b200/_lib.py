@@ -65,6 +65,8 @@ SIGNATURES = {
     "vited_forward_pairs": (_i, [_vp, _vp, _i, _vp, _vp]),
     "vited_score_grid": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp]),
     "vited_score_grid_u8": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp]),
+    "vited_score_pairs": (_i, [_vp, _vp, _i, _vp, _i64, _vp, _vp]),
+    "vited_score_pairs_u8": (_i, [_vp, _vp, _i, _vp, _i64, _vp, _vp]),
     "vited_profile_json": (ctypes.c_char_p, [_vp, _vp]),
     "vited_launch_count": (_i64, [_vp]),
     "vited_act_dtype": (_i, []),

@@ -108,10 +108,12 @@ struct vited_engine {
   std::string profile_json;
   // workspace
   DevBuf x, h, qkv, o, q, delta, hid, col, tok, xsrc, enc_tok, kv, ci, xj, tmp_tok;
+  DevBuf out_pos, pl_items, pl_hist, pl_info;   // vited_score_pairs: sorted output positions, item maps, sort, info
 
   int64_t workspace_bytes() const {
     return (int64_t)(x.cap + h.cap + qkv.cap + o.cap + q.cap + delta.cap + hid.cap + col.cap + tok.cap + xsrc.cap +
-                     enc_tok.cap + kv.cap + ci.cap + xj.cap + tmp_tok.cap);
+                     enc_tok.cap + kv.cap + ci.cap + xj.cap + tmp_tok.cap + out_pos.cap + pl_items.cap + pl_hist.cap +
+                     pl_info.cap);
   }
 };
 
@@ -389,8 +391,9 @@ static int items_per_batch(vited_engine* e) {
 
 // patch tokens of B images -> e->tok (fp16 [B*Ne, D]); img_stride = elements between consecutive images.
 // `u8`: the images are [B, S, S, in_chans] bytes (ToTensor + Normalize(.5, .5) applied on the way, im2col_u8_patches),
-// otherwise [B, in_chans, S, S] fp32.
-static int patch_tokens(vited_engine* e, const void* images, bool u8, size_t img_stride, int B, cudaStream_t s) {
+// otherwise [B, in_chans, S, S] fp32. `items` (device, [B]) non-null: image b is images[items[b]] of a contiguous set.
+static int patch_tokens(vited_engine* e, const void* images, bool u8, size_t img_stride, int B, cudaStream_t s,
+                        const int* items = nullptr) {
   const vited_config& c = e->cfg;
   const size_t rows = (size_t)B * e->Ne;
   TRY(e->col.ensure(rows * e->Kpe * 2));
@@ -400,11 +403,13 @@ static int patch_tokens(vited_engine* e, const void* images, bool u8, size_t img
     VITED_CHECK(img_stride == img_elems, "patch_tokens: uint8 images must be contiguous");
     prof_mark(e, "im2col_u8", 0.0, (double)rows * e->Kpe * 3.0, s);
     TRY(im2col_u8_patches(static_cast<const uint8_t*>(images), e->col.as<act_t>(), B, c.in_chans, c.img_size,
-                          c.patch_size, s));
+                          c.patch_size, s, items));
   } else if (img_stride == img_elems) {
     prof_mark(e, "im2col", 0.0, (double)rows * e->Kpe * 6.0, s);
-    TRY(im2col_patches(static_cast<const float*>(images), e->col.as<act_t>(), B, c.in_chans, c.img_size, c.patch_size, s));
+    TRY(im2col_patches(static_cast<const float*>(images), e->col.as<act_t>(), B, c.in_chans, c.img_size, c.patch_size, s,
+                       items));
   } else {
+    VITED_CHECK(items == nullptr, "patch_tokens: gathered images must be contiguous");
     for (int b = 0; b < B; ++b) {
       prof_mark(e, "im2col", 0.0, (double)e->Ne * e->Kpe * 6.0, s);
       TRY(im2col_patches(static_cast<const float*>(images) + (size_t)b * img_stride,
@@ -652,7 +657,7 @@ void vited_destroy(vited_engine* e) {
   cudaDeviceSynchronize();
   for (void* p : e->owned) cudaFree(p);
   DevBuf* bufs[] = {&e->x, &e->h, &e->qkv, &e->o, &e->q, &e->delta, &e->hid, &e->col, &e->tok, &e->xsrc, &e->enc_tok,
-                    &e->kv, &e->ci, &e->xj, &e->tmp_tok};
+                    &e->kv, &e->ci, &e->xj, &e->tmp_tok, &e->out_pos, &e->pl_items, &e->pl_hist, &e->pl_info};
   for (DevBuf* b : bufs) b->release();
   for (cudaEvent_t ev : e->ev_pool) cudaEventDestroy(ev);
   delete e;
@@ -780,20 +785,33 @@ int vited_forward_pairs(vited_engine* e, const float* pairs, int B, float* out_l
   return 0;
 }
 
-// decoder input states of items [ca, cb) -> e->xsrc (split layout, cb - ca sequences)
+// decoder input states of items [ca, cb) -> e->xsrc (split layout, cb - ca sequences). `items` non-null: of items
+// items[ca .. cb) (device list) instead.
 static int build_xsrc(vited_engine* e, const char* images, bool u8, size_t img_bytes, int ca, int cb, bool headroom,
-                      cudaStream_t s) {
+                      cudaStream_t s, const int* items = nullptr) {
   const int n_src = cb - ca;
   const size_t img = (size_t)e->cfg.in_chans * e->cfg.img_size * e->cfg.img_size;
   const int step = items_per_batch(e);
   TRY(e->xsrc.ensure((size_t)n_src * e->Nd * e->D * 4, headroom));
   for (int i0 = 0; i0 < n_src; i0 += step) {
     const int n = (n_src - i0 < step) ? (n_src - i0) : step;
-    TRY(patch_tokens(e, images + (size_t)(ca + i0) * img_bytes, u8, img, n, s));
+    if (items) TRY(patch_tokens(e, images, u8, img, n, s, items + ca + i0));
+    else TRY(patch_tokens(e, images + (size_t)(ca + i0) * img_bytes, u8, img, n, s));
     TRY(decoder_item_state(e, n, s));
     TRY(scatter_split(e, e->xsrc.as<float>(), n_src, i0, n, s));
   }
   return 0;
+}
+
+// items whose decoder input states fit OPT_XSRC_BUDGET_MB (columns per window), at least one
+static int64_t xsrc_window_items(vited_engine* e) {
+  const int64_t cw = (int64_t)((size_t)e->xsrc_budget_mb * 1000000 / ((size_t)e->Nd * e->D * 4));
+  return cw < 1 ? 1 : cw;
+}
+// context items whose K/V cache (every decoder layer) fits OPT_KV_BUDGET_MB, at least one
+static int kv_block_items(vited_engine* e) {
+  const int rb = (int)((size_t)e->kv_budget_mb * 1000000 / (e->dec.size() * e->Ne * 2 * e->D * 2));
+  return rb < 1 ? 1 : rb;
 }
 
 // vited_score_grid / vited_score_grid_u8: one grid loop for both image formats
@@ -809,7 +827,7 @@ static int score_grid_impl(vited_engine* e, const void* images_in, bool u8, int 
   const char* images = static_cast<const char*>(images_in);
   const size_t img = (size_t)e->cfg.in_chans * e->cfg.img_size * e->cfg.img_size;
   const size_t img_bytes = img * (u8 ? 1 : 4);
-  const size_t D = e->D, Ne = e->Ne, Nd = e->Nd;
+  const size_t D = e->D, Ne = e->Ne;
   const int step = items_per_batch(e);
   const int pair_mode = mode == VITED_GRID_ORDERED_OFFDIAG ? 0 : 1;
 
@@ -820,17 +838,13 @@ static int score_grid_impl(vited_engine* e, const void* images_in, bool u8, int 
   //    budget, inside the loop over K/V row blocks below; otherwise once, here, for the whole call.
   const int c0 = (mode == VITED_GRID_UPPER_TRI_DIAG) ? row_begin : 0;
   const int n_cols = N - c0;
-  const size_t xsrc_bytes_per_item = Nd * D * 4;
-  int64_t cw = (int64_t)((size_t)e->xsrc_budget_mb * 1000000 / xsrc_bytes_per_item);
-  if (cw < 1) cw = 1;
+  const int64_t cw = xsrc_window_items(e);
   const bool one_window = n_cols <= cw;
   const int win = one_window ? n_cols : (int)cw;
   if (one_window) TRY(build_xsrc(e, images, u8, img_bytes, c0, N, true, s));
 
   // 2) context rows in blocks whose K/V cache stays within the budget (default 8 GB)
-  const size_t kv_bytes_per_item = e->dec.size() * Ne * 2 * D * 2;
-  int rb = (int)((size_t)e->kv_budget_mb * 1000000 / kv_bytes_per_item);
-  if (rb < 1) rb = 1;
+  const int rb = kv_block_items(e);
   const int pairs_per_chunk = items_per_batch(e);
   for (int r0 = row_begin; r0 < row_end; r0 += rb) {
     const int r1 = (r0 + rb < row_end) ? (r0 + rb) : row_end;
@@ -878,6 +892,139 @@ int vited_score_grid(vited_engine* e, const float* images, int N, int mode, int 
 int vited_score_grid_u8(vited_engine* e, const uint8_t* images, int N, int mode, int row_begin, int row_end, float* out,
                         void* stream) {
   return score_grid_impl(e, images, true, N, mode, row_begin, row_end, out, (cudaStream_t)stream);
+}
+
+// vited_score_pairs / vited_score_pairs_u8. The distinct context items of the list take the grid's role of rows (slots
+// in ascending item order, blocks of kv_block_items), its distinct decoder items that of columns (windows of
+// xsrc_window_items); the pairs are bucketed by (block, window) on the device, then the grid's loops run over the cells
+// with pairs, with the decoder writing every logit row to the pair's input position.
+static int score_pairs_impl(vited_engine* e, const void* images_in, bool u8, int N, const int32_t* pairs,
+                            int64_t n_pairs, float* out, cudaStream_t s) {
+  TRY(check_ready(e));
+  DeviceScope scope(e->device);
+  VITED_CHECK(N >= 0, "vited_score_pairs: N = %d", N);
+  VITED_CHECK(n_pairs >= 0 && n_pairs <= INT32_MAX, "vited_score_pairs: n_pairs = %lld outside [0, 2^31)",
+              (long long)n_pairs);
+  if (n_pairs == 0) return 0;
+  VITED_CHECK(pairs && out && (images_in || N == 0), "vited_score_pairs: null pointer");
+  const int P = (int)n_pairs;
+  const char* images = static_cast<const char*>(images_in);
+  const size_t img = (size_t)e->cfg.in_chans * e->cfg.img_size * e->cfg.img_size;
+  const size_t img_bytes = img * (u8 ? 1 : 4);
+  const size_t D = e->D, Ne = e->Ne;
+  const int step = items_per_batch(e);
+
+  // cells: at most min(N, P) distinct items on either side
+  const int64_t cw = xsrc_window_items(e);
+  const int rb = kv_block_items(e);
+  const int64_t m = N < P ? N : P;
+  const int64_t nw = m > 0 ? (m + cw - 1) / cw : 1;
+  const int64_t cells = (m > 0 ? (m + rb - 1) / rb : 1) * nw;
+  const int64_t kMaxSortEntries = 1 << 24;
+  VITED_CHECK(cells <= kMaxSortEntries,
+              "vited_score_pairs: the K/V and decoder-state budgets split %lld items into %lld cells (at most %lld); "
+              "raise VITED_OPT_KV_BUDGET_MB / VITED_OPT_XSRC_BUDGET_MB", (long long)m, (long long)cells,
+              (long long)kMaxSortEntries);
+  // tiles of the counting sort: 1,024 pairs, or more so that the [cells x tiles] histogram stays within 2^24 entries
+  int64_t T = 1024;
+  if (cells * ((P + T - 1) / T) > kMaxSortEntries) T = ((int64_t)P * cells / kMaxSortEntries + 32) / 32 * 32;
+  PairCells pc;
+  pc.rb = rb;
+  pc.cw = (int)(cw < INT32_MAX ? cw : INT32_MAX);
+  pc.nw = (int)nw;
+  pc.T = (int)T;
+  pc.tiles = (int)((P + T - 1) / T);
+  const size_t n_hist = (size_t)cells * pc.tiles;
+  const size_t n_info = PL_CELLS + (size_t)cells + 1;
+  const size_t Nz = N > 0 ? (size_t)N : 1;
+  TRY(e->pl_items.ensure(6 * Nz * sizeof(int)));      // used [2N] | slot [2N] | items [2N]
+  TRY(e->pl_hist.ensure(n_hist * sizeof(int)));
+  TRY(e->pl_info.ensure(n_info * sizeof(int)));
+  TRY(e->ci.ensure((size_t)P * sizeof(int) + 16));
+  TRY(e->xj.ensure((size_t)P * sizeof(int) + 16));
+  TRY(e->out_pos.ensure((size_t)P * sizeof(int) + 16));
+  int* used = e->pl_items.as<int>();
+  int* slot = used + 2 * Nz;
+  int* items = used + 4 * Nz;
+  int* hist = e->pl_hist.as<int>();
+  int* info = e->pl_info.as<int>();
+
+  // 1) mark + validate, 2) compact, 3) bucket; 4) one copy back
+  VITED_CUDA_OK(cudaMemsetAsync(used, 0, 2 * Nz * sizeof(int), s));
+  VITED_CUDA_OK(cudaMemsetAsync(hist, 0, n_hist * sizeof(int), s));
+  VITED_CUDA_OK(cudaMemsetAsync(info, 0, n_info * sizeof(int), s));
+  VITED_CUDA_OK(cudaMemsetAsync(info + PL_FIRST_BAD, 0xff, sizeof(int), s));
+  prof_mark(e, "pair_index", 0.0, (double)P * 8.0, s);
+  TRY(pairs_mark(pairs, P, N, used, info, s));
+  prof_mark(e, "pair_index", 0.0, (double)Nz * 8.0, s);
+  TRY(exclusive_scan(used, slot, N, info + PL_N_CTX, s));
+  prof_mark(e, "pair_index", 0.0, (double)Nz * 8.0, s);
+  TRY(exclusive_scan(used + Nz, slot + Nz, N, info + PL_N_X2, s));
+  prof_mark(e, "pair_index", 0.0, (double)Nz * 16.0, s);
+  TRY(pairs_compact(used, slot, items, N, s));
+  prof_mark(e, "pair_index", 0.0, (double)P * 16.0 + n_hist * 4.0, s);
+  TRY(pairs_bucket_count(pairs, P, N, slot, pc, hist, s));
+  prof_mark(e, "pair_index", 0.0, (double)n_hist * 8.0, s);
+  TRY(exclusive_scan(hist, hist, (int64_t)n_hist, info + PL_CELLS + cells, s));
+  prof_mark(e, "pair_index", 0.0, (double)cells * 8.0, s);
+  TRY(pairs_cell_starts(pairs, hist, pc.tiles, (int)cells, info, s));
+  prof_mark(e, "pair_index", 0.0, (double)P * 28.0, s);
+  TRY(pairs_bucket_scatter(pairs, P, N, slot, pc, hist, e->ci.as<int>(), e->xj.as<int>(), e->out_pos.as<int>(), s));
+  std::vector<int> h(n_info);
+  VITED_CUDA_OK(cudaMemcpyAsync(h.data(), info, n_info * sizeof(int), cudaMemcpyDeviceToHost, s));
+  VITED_CUDA_OK(cudaStreamSynchronize(s));
+  VITED_CHECK(h[PL_N_BAD] == 0, "vited_score_pairs: pair %u = (%d, %d) has an index outside [0, %d) (%d such pairs)",
+              (unsigned)h[PL_FIRST_BAD], h[PL_BAD_A], h[PL_BAD_B], N, h[PL_N_BAD]);
+  const int n_ctx = h[PL_N_CTX], n_x2 = h[PL_N_X2];
+  const int* ctx_items = items;
+  const int* x2_items = items + Nz;
+
+  // 5) the grid's loops over the cells: K/V blocks outer, decoder-state windows inner
+  const bool one_window = n_x2 <= cw;
+  if (one_window) TRY(build_xsrc(e, images, u8, img_bytes, 0, n_x2, true, s, x2_items));
+  const int pairs_per_chunk = items_per_batch(e);
+  for (int blk = 0; (int64_t)blk * rb < n_ctx; ++blk) {
+    const int s0 = blk * rb;
+    const int nr = (n_ctx - s0 < rb) ? (n_ctx - s0) : rb;
+    TRY(e->enc_tok.ensure((size_t)nr * Ne * D * 4));
+    for (int i0 = 0; i0 < nr; i0 += step) {
+      const int n = (nr - i0 < step) ? (nr - i0) : step;
+      TRY(patch_tokens(e, images, u8, img, n, s, ctx_items + s0 + i0));
+      TRY(encoder_stack(e, n, e->enc_tok.as<float>() + (size_t)i0 * Ne * D, s));
+    }
+    TRY(build_kv(e, e->enc_tok.as<float>(), nr, s));
+    for (int w = 0; (int64_t)w * cw < n_x2; ++w) {
+      const int64_t cell = (int64_t)blk * nw + w;
+      const size_t first = (size_t)h[PL_CELLS + cell];
+      const size_t total = (size_t)h[PL_CELLS + cell + 1] - first;
+      if (total == 0) continue;
+      const int ca = (int)(w * cw);
+      const int cb = (int)((ca + cw < n_x2) ? (ca + cw) : n_x2);
+      if (!one_window) TRY(build_xsrc(e, images, u8, img_bytes, ca, cb, false, s, x2_items));
+      // equal chunks, as in score_grid_impl
+      const size_t n_chunks = (total + pairs_per_chunk - 1) / pairs_per_chunk;
+      const size_t chunk = (total + n_chunks - 1) / n_chunks;
+      for (size_t p0 = 0; p0 < total; p0 += chunk) {
+        const int Pc = (int)((total - p0 < chunk) ? (total - p0) : chunk);
+        HeadArgs head = {};
+        head.out = out;
+        head.out_pos = e->out_pos.as<int>() + first + p0;
+        TRY(decode_chunk(e, Pc, e->ci.as<int>() + first + p0, e->xj.as<int>() + first + p0, e->xsrc.as<float>(),
+                         cb - ca, ca, nr, head, s));
+      }
+    }
+  }
+  return 0;
+}
+
+int vited_score_pairs(vited_engine* e, const float* images, int N, const int32_t* pairs, int64_t n_pairs, float* out,
+                      void* stream) {
+  return score_pairs_impl(e, images, false, N, pairs, n_pairs, out, (cudaStream_t)stream);
+}
+
+int vited_score_pairs_u8(vited_engine* e, const uint8_t* images, int N, const int32_t* pairs, int64_t n_pairs,
+                         float* out, void* stream) {
+  return score_pairs_impl(e, images, true, N, pairs, n_pairs, out, (cudaStream_t)stream);
 }
 
 const char* vited_profile_json(vited_engine* e, void* stream) {

@@ -66,11 +66,14 @@ struct ResidLnArgs {
 };
 int resid_ln(const ResidLnArgs& a, cudaStream_t stream);
 
-// images [B,3,S,S] f32 -> patch matrix [B*G*G, 3*p*p] fp16, column = c*p*p + py*p + px (Conv2d weight.view order)
-int im2col_patches(const float* images, act_t* out, int B, int C, int S, int p, cudaStream_t stream);
+// images [B,3,S,S] f32 -> patch matrix [B*G*G, 3*p*p] fp16, column = c*p*p + py*p + px (Conv2d weight.view order).
+// items (device, [B]) non-null: output image b is read from images[items[b]] (a gathered batch, no staging copy).
+int im2col_patches(const float* images, act_t* out, int B, int C, int S, int p, cudaStream_t stream,
+                   const int* items = nullptr);
 // images [B,S,S,C] u8 (HWC bytes) -> the same patch matrix, bit-identical to normalize_u8 + im2col_patches
 // (ToTensor + Normalize(.5, .5) folded in). Built for C = 3 and p in {4, 8, 16, 32}; anything else is an error.
-int im2col_u8_patches(const uint8_t* images, act_t* out, int B, int C, int S, int p, cudaStream_t stream);
+int im2col_u8_patches(const uint8_t* images, act_t* out, int B, int C, int S, int p, cudaStream_t stream,
+                      const int* items = nullptr);
 
 // x0 (f32, split layout, B sequences): patch rows = tok (fp16 [B*Np, D]) + pos[1+t]; cls rows = cls + pos[0]
 int assemble_tokens(const act_t* tok, const float* pos_embed, const float* cls_token, float* x, int B, int n_patch,
@@ -87,6 +90,7 @@ struct HeadArgs {
   float* out;
   const int* ci;        // pair -> ctx item (row of the grid); null => linear output out[p*C + c]
   const int* xj;        // pair -> x2 item (column)
+  const int* out_pos;   // non-null: out[out_pos[p]*C + c] (vited_score_pairs: the pair's position in the caller's list)
   int row_begin, n_items;
   int P, D, C;
   float eps;
@@ -101,6 +105,28 @@ int head_logits(const HeadArgs& a, cudaStream_t stream);
 // The whole grid row is the window [0, N). pair_list_count returns the number of pairs (the caller sizes ci / xj with it).
 __host__ __device__ size_t pair_list_count(int mode, int r0, int r1, int ca, int cb);
 int pair_list(int mode, int r0, int r1, int ca, int cb, int* ci, int* xj, cudaStream_t stream);
+
+// ---- caller-given pair lists (pair_lists.cu): the index work of vited_score_pairs ----
+// info block copied back to the host once per call: the header below, then PL_CELLS + k = first sorted position of cell
+// k (k <= cells, the last entry = number of valid pairs)
+enum { PL_N_BAD = 0, PL_FIRST_BAD, PL_BAD_A, PL_BAD_B, PL_N_CTX, PL_N_X2, PL_CELLS };
+// pairs [P, 2] (context item, decoder item); used [2N] zeroed: used[a] / used[N + b] = 1 for valid pairs; invalid ones
+// counted in info[PL_N_BAD], the lowest such pair index in info[PL_FIRST_BAD] (preset to 0xffffffff)
+int pairs_mark(const int* pairs, int P, int N, int* used, int* info, cudaStream_t stream);
+// exclusive prefix sum of n ints (one block; out may alias in); *total = sum (device)
+int exclusive_scan(const int* in, int* out, int64_t n, int* total, cudaStream_t stream);
+// items[half*N + slot[half*N + i]] = i for the used items of both halves (ascending lists of distinct items)
+int pairs_compact(const int* used, const int* slot, int* items, int N, cudaStream_t stream);
+// cell of a pair = (context slot / rb) * nw + decoder slot / cw; the sort runs on tiles of T pairs, one warp each
+struct PairCells { int rb, cw, nw, T, tiles; };
+// hist [cells * tiles] zeroed -> pairs per (cell, tile)
+int pairs_bucket_count(const int* pairs, int P, int N, const int* slot, const PairCells& c, int* hist,
+                       cudaStream_t stream);
+// info[PL_CELLS + k] = hist[k * tiles] (hist exclusive-scanned) and the offending pair's indices, if any
+int pairs_cell_starts(const int* pairs, const int* hist, int tiles, int cells, int* info, cudaStream_t stream);
+// stable scatter by cell: ci = context slot % rb, xj = decoder slot, out_pos = input position (hist advanced)
+int pairs_bucket_scatter(const int* pairs, int P, int N, const int* slot, const PairCells& c, int* hist, int* ci,
+                         int* xj, int* out_pos, cudaStream_t stream);
 
 // plain copy/convert helpers
 int f32_to_act(const float* in, act_t* out, size_t n, cudaStream_t stream);

@@ -9,7 +9,8 @@ namespace vited {
 // im2col for Conv2d(kernel = stride = p)  (timm PatchEmbed; called from models/vision_transformer.py:383,391)
 // token t = gy*G + gx covers pixels [gy*p:(gy+1)*p, gx*p:(gx+1)*p]; column = c*p*p + py*p + px.
 // ------------------------------------------------------------------------------------------------------------
-__global__ void im2col_kernel(const float* __restrict__ img, act_t* __restrict__ out, int B, int C, int S, int p) {
+__global__ void im2col_kernel(const float* __restrict__ img, act_t* __restrict__ out, int B, int C, int S, int p,
+                              const int* __restrict__ items) {
   const int G = S / p;
   const int K = C * p * p;
   const int segs_per_row = K / 4;  // 4 consecutive px per thread (p % 4 == 0)
@@ -23,8 +24,9 @@ __global__ void im2col_kernel(const float* __restrict__ img, act_t* __restrict__
     const int px = col % p;
     const int t = (int)(row % (G * G));
     const int b = (int)(row / (G * G));
+    const size_t sb = items != nullptr ? (size_t)items[b] : (size_t)b;   // source image
     const int gy = t / G, gx = t % G;
-    const float4 v = *reinterpret_cast<const float4*>(img + (((size_t)b * C + c) * S + (gy * p + py)) * S + gx * p + px);
+    const float4 v = *reinterpret_cast<const float4*>(img + ((sb * C + c) * S + (gy * p + py)) * S + gx * p + px);
     uint2 pk;
     pk.x = pack_act(v.x, v.y);
     pk.y = pack_act(v.z, v.w);
@@ -32,13 +34,13 @@ __global__ void im2col_kernel(const float* __restrict__ img, act_t* __restrict__
   }
 }
 
-int im2col_patches(const float* images, act_t* out, int B, int C, int S, int p, cudaStream_t stream) {
+int im2col_patches(const float* images, act_t* out, int B, int C, int S, int p, cudaStream_t stream, const int* items) {
   VITED_CHECK(p % 4 == 0 && S % p == 0, "im2col: patch size %d must be a multiple of 4 and divide img size %d", p, S);
   const size_t total = (size_t)B * (S / p) * (S / p) * (C * p * p / 4);
   int blocks = (int)((total + 255) / 256);
   if (blocks > 148 * 16) blocks = 148 * 16;
   if (blocks < 1) blocks = 1;
-  im2col_kernel<<<blocks, 256, 0, stream>>>(images, out, B, C, S, p);
+  im2col_kernel<<<blocks, 256, 0, stream>>>(images, out, B, C, S, p, items);
   VITED_CUDA_OK(cudaGetLastError());
   return 0;
 }
@@ -47,12 +49,13 @@ int im2col_patches(const float* images, act_t* out, int B, int C, int S, int p, 
 // normalize_u8_kernel (ToTensor + Normalize(.5, .5), hisfrag.py:89-93) folded in. A byte has 256 values, so every
 // block first evaluates that arithmetic once per value into a shared table of 16-bit results (rounded by pack_act,
 // as im2col_kernel rounds): the output is bit-identical to normalize_u8 followed by im2col_patches.
+// `items` non-null: output image b is read from image items[b] (the engine's gathered batches).
 // One thread = one pixel row of one patch: P*C contiguous bytes (48 at P = 16), loaded as VB-byte vectors and
 // de-interleaved in registers, then P 16-bit values per channel stored contiguously. gx runs fastest across a warp,
 // so a warp reads whole pixel rows and every thread writes whole 32-byte sectors.
 template <int P, int C, int VB>
 __global__ void __launch_bounds__(256) im2col_u8_kernel(const uint8_t* __restrict__ img, act_t* __restrict__ out,
-                                                        int B, int S) {
+                                                        int B, int S, const int* __restrict__ items) {
   __shared__ uint16_t lut[256];
   for (int v = threadIdx.x; v < 256; v += blockDim.x) {
     const float f = __fdiv_rn(__fsub_rn(__fdiv_rn((float)v, 255.0f), 0.5f), 0.5f);
@@ -71,7 +74,8 @@ __global__ void __launch_bounds__(256) im2col_u8_kernel(const uint8_t* __restric
     const size_t b = by / S;
     const int gy = y / P, py = y % P;
     uint32_t w[NB / 4];
-    const uint8_t* src = img + (by * S + (size_t)gx * P) * C;
+    const size_t sb = items != nullptr ? (size_t)items[b] : b;   // source image
+    const uint8_t* src = img + ((sb * S + y) * S + (size_t)gx * P) * C;
 #pragma unroll
     for (int k = 0; k < NB / VB; ++k) {
       if constexpr (VB == 16) {
@@ -105,7 +109,8 @@ __global__ void __launch_bounds__(256) im2col_u8_kernel(const uint8_t* __restric
   }
 }
 
-int im2col_u8_patches(const uint8_t* images, act_t* out, int B, int C, int S, int p, cudaStream_t stream) {
+int im2col_u8_patches(const uint8_t* images, act_t* out, int B, int C, int S, int p, cudaStream_t stream,
+                      const int* items) {
   VITED_CHECK(B >= 0 && p > 0 && S % p == 0, "im2col_u8: patch size %d must divide img size %d", p, S);
   const size_t total = (size_t)B * S * (S / p);
   if (total == 0) return 0;
@@ -116,7 +121,7 @@ int im2col_u8_patches(const uint8_t* images, act_t* out, int B, int C, int S, in
 #define VITED_IM2COL_U8(P_, C_, VB_)                                                                    \
   if (p == P_ && C == C_) {                                                                             \
     VITED_CHECK(a % VB_ == 0, "im2col_u8: images must be %d-byte aligned for patch %d", VB_, P_);       \
-    im2col_u8_kernel<P_, C_, VB_><<<blocks, 256, 0, stream>>>(images, out, B, S);                       \
+    im2col_u8_kernel<P_, C_, VB_><<<blocks, 256, 0, stream>>>(images, out, B, S, items);                \
     VITED_CUDA_OK(cudaGetLastError());                                                                  \
     return 0;                                                                                           \
   }
@@ -335,7 +340,9 @@ __global__ void __launch_bounds__(256) head_kernel(HeadArgs a) {
     }
     const float rstd = rsqrtf(warp_sum(ss) / (float)D + a.eps);
     size_t obase;
-    if (a.ci != nullptr) {
+    if (a.out_pos != nullptr) {
+      obase = (size_t)a.out_pos[p] * a.C;
+    } else if (a.ci != nullptr) {
       obase = ((size_t)(a.ci[p] - a.row_begin) * a.n_items + a.xj[p]) * a.C;
     } else {
       obase = p * a.C;

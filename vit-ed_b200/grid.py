@@ -287,6 +287,99 @@ def _score_fragment_rows_resumable(model, images, lo, hi, path, block_rows, save
     return block
 
 
+# --------------------------------------------------------------------------------------------- pair lists
+def extension_pairs(is_new):
+    """The pairs of ``upper_tri_pairs(N)`` that touch a new item: every (a, b) with a <= b and ``is_new[a] or
+    is_new[b]``, a-major with b ascending, as int32 [P, 2]. What a scored collection of the old items lacks once the new
+    ones are inserted at their sorted positions: N_old * N_new + N_new (N_new + 1) / 2 pairs."""
+    is_new = np.asarray(is_new, dtype=bool)
+    n = len(is_new)
+    new_idx = np.flatnonzero(is_new).astype(np.int32)
+    rows = []
+    for a in range(n):
+        cols = np.arange(a, n, dtype=np.int32) if is_new[a] else new_idx[np.searchsorted(new_idx, a):]
+        if len(cols):
+            rows.append(np.stack([np.full(len(cols), a, dtype=np.int32), cols], axis=1))
+    return np.concatenate(rows) if rows else np.zeros((0, 2), dtype=np.int32)
+
+
+def pair_shares(ctx_items, world):
+    """Sharding of a pair list over ``world`` ranks: the pairs stable-sorted by context item (so that a rank encodes
+    only the context items of its share), then split into contiguous shares of equal pair count. Returns ``order``
+    (sorted position -> input position, int64) and ``bounds`` (rank r takes sorted positions [bounds[r], bounds[r+1]))."""
+    ctx_items = np.asarray(ctx_items)
+    order = np.argsort(ctx_items, kind='stable').astype(np.int64)
+    per = -(-len(ctx_items) // world)
+    bounds = [min(r * per, len(ctx_items)) for r in range(world + 1)]
+    return order, bounds
+
+
+def unpermute_shares(gathered, order, bounds):
+    """Inverse of ``pair_shares``: ``gathered`` [world, longest, ...] holds rank r's scores in its first
+    bounds[r+1] - bounds[r] rows; returns them as [P, ...] in input order."""
+    shares = [gathered[r, :bounds[r + 1] - bounds[r]] for r in range(len(bounds) - 1)]
+    flat = torch.cat(shares) if shares else gathered.new_zeros((0,) + tuple(gathered.shape[2:]))
+    out = torch.empty_like(flat)
+    out[torch.as_tensor(order, device=flat.device)] = flat
+    return out
+
+
+@torch.no_grad()
+def score_pairs(model, images, pairs, gather=True):
+    """Logits of a pair list -> [P, num_classes] fp32 in the list's order (``model.score_pairs`` on every rank's share,
+    see ``pair_shares``), then ONE all-gather of the padded shares. ``images`` (either form of ``score_grid``) are
+    the whole collection on every rank; ``pairs`` a [P, 2] int32 / int64 tensor or array (any device). With several
+    ranks and ``gather=False``, returns this rank's share as (input positions int64 [P_r], logits [P_r, C])."""
+    rank, world = _dist_info()
+    dev = images.device
+    if world == 1:
+        return model.score_pairs(images, torch.as_tensor(pairs).to(dev))
+    pairs_np = (pairs.cpu().numpy() if isinstance(pairs, torch.Tensor) else np.asarray(pairs)).astype(np.int64)
+    if pairs_np.ndim != 2 or pairs_np.shape[1] != 2:
+        raise ValueError(f'pairs must be [P, 2], got {pairs_np.shape}')
+    order, bounds = pair_shares(pairs_np[:, 0], world)
+    lo, hi = bounds[rank], bounds[rank + 1]
+    mine = model.score_pairs(images, torch.from_numpy(pairs_np[order[lo:hi]]).to(dev))
+    if not gather:
+        return torch.from_numpy(order[lo:hi]), mine
+    import torch.distributed as dist
+    longest = max(b - a for a, b in zip(bounds, bounds[1:]))
+    padded = mine.new_zeros((longest, model.num_classes))
+    padded[:hi - lo] = mine
+    gathered = mine.new_empty((world * longest, model.num_classes))
+    dist.all_gather_into_tensor(gathered, padded)
+    return unpermute_shares(gathered.view(world, longest, model.num_classes), order, bounds)
+
+
+@torch.no_grad()
+def extend_fragments(model, images, old_sim, is_new, gather=True):
+    """Similarity logits [N, N] fp32 of a fragment collection grown by new items, without re-scoring the old ones.
+    ``images`` is the whole collection in its sorted order (fp32 or the uint8 crops, as ``score_fragments``);
+    ``is_new[k]`` marks the new items; ``old_sim`` is the ``score_fragments`` matrix of the old items in their relative
+    order. Old x old entries are copied from ``old_sim``; every other entry is scored through
+    ``score_pairs(extension_pairs(is_new))`` and mirrored as ``mirror_upper`` does. With several ranks and
+    ``gather=False``, returns this rank's share of the extension pairs as ``score_pairs`` does."""
+    is_new = np.asarray(is_new, dtype=bool)
+    n = images.shape[0]
+    if is_new.shape != (n,):
+        raise ValueError(f'is_new has shape {is_new.shape}, the collection {n} items')
+    old = np.flatnonzero(~is_new)
+    if tuple(old_sim.shape) != (len(old), len(old)):
+        raise ValueError(f'old_sim is {tuple(old_sim.shape)}, the collection has {len(old)} old items')
+    pairs = extension_pairs(is_new)
+    scores = score_pairs(model, images, pairs, gather=gather)
+    if isinstance(scores, tuple):
+        return scores
+    dev = images.device
+    upper = torch.zeros((n, n), dtype=torch.float32, device=dev)
+    p = torch.from_numpy(pairs).to(dev).long()
+    upper[p[:, 0], p[:, 1]] = scores[:, 0]
+    sim = mirror_upper(upper)
+    o = torch.from_numpy(old).to(dev)
+    sim[o[:, None], o[None, :]] = old_sim.to(device=dev, dtype=torch.float32)
+    return sim
+
+
 def mirror_upper(upper):
     """sim[a, b] = sim[b, a] = score(a, b) for a <= b (hisfrag.py:291-292)."""
     tri = torch.triu(upper)

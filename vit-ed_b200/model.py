@@ -339,17 +339,9 @@ class VisionTransformerCustom(nn.Module):
         ``images`` is either the model input [N, in_chans, S, S] (fp32) or the decoded crops [N, S, S, in_chans] as a
         CUDA uint8 tensor: ToTensor + Normalize(.5, .5) then runs inside the patch embedding (C-ABI
         ``vited_score_grid_u8``), bit-identical to scoring the normalised fp32 images, at a quarter of their memory."""
-        if images.dtype == torch.uint8:
-            want = (self.img_size, self.img_size, self.in_chans)
-            if images.dim() != 4 or tuple(images.shape[1:]) != want or not images.is_cuda:
-                raise ValueError(f'uint8 images must be a CUDA tensor [N, {want[0]}, {want[1]}, {want[2]}] (HWC crops), '
-                                 f'got {tuple(images.shape)} on {images.device}')
-            images = images.contiguous()
-            entry, name = _lib.lib.vited_score_grid_u8, 'vited_score_grid_u8'
-        else:
-            images = self._prep(images)
-            self._check_images(images)
-            entry, name = _lib.lib.vited_score_grid, 'vited_score_grid'
+        images, u8 = self._grid_images(images)
+        entry, name = ((_lib.lib.vited_score_grid_u8, 'vited_score_grid_u8') if u8 else
+                       (_lib.lib.vited_score_grid, 'vited_score_grid'))
         n = images.shape[0]
         row_end = n if row_end is None else row_end
         if not (0 <= row_begin <= row_end <= n):
@@ -358,6 +350,52 @@ class VisionTransformerCustom(nn.Module):
         if out is None:
             out = torch.zeros((row_end - row_begin, n, self.num_classes), dtype=torch.float32, device=images.device)
         _lib.check(entry(eng, images.data_ptr(), n, int(mode), int(row_begin), int(row_end), out.data_ptr(),
+                         self._stream(images.device)), name)
+        return out
+
+    def _grid_images(self, images):
+        """The two image forms of score_grid / score_pairs -> (contiguous tensor, is_uint8)."""
+        if images.dtype == torch.uint8:
+            want = (self.img_size, self.img_size, self.in_chans)
+            if images.dim() != 4 or tuple(images.shape[1:]) != want or not images.is_cuda:
+                raise ValueError(f'uint8 images must be a CUDA tensor [N, {want[0]}, {want[1]}, {want[2]}] (HWC crops), '
+                                 f'got {tuple(images.shape)} on {images.device}')
+            return images.contiguous(), True
+        images = self._prep(images)
+        self._check_images(images)
+        return images, False
+
+    @torch.no_grad()
+    def score_pairs(self, images, pairs, out=None):
+        """Logits of a caller-given pair list -> [P, num_classes] fp32, ``out[p]`` = model(tokens(images[a]), images[b])
+        for ``pairs[p] = (a, b)``: the (a, b) entry of ``score_grid``. Any order; duplicates, a == b and a > b are
+        allowed. Every item the list references is encoded, and its decoder input state built, once per call (C-ABI
+        ``vited_score_pairs``), which is what makes this cheaper than ``model(pairs)`` when items repeat.
+
+        ``images`` takes the two forms of ``score_grid``. ``pairs`` is an int32 / int64 [P, 2] tensor on the images'
+        device. An index outside [0, N) raises ``VitedError`` naming the pair, before anything is scored."""
+        images, u8 = self._grid_images(images)
+        if not isinstance(pairs, torch.Tensor) or pairs.dim() != 2 or pairs.shape[1] != 2:
+            raise ValueError(f'pairs must be a [P, 2] tensor, got {getattr(pairs, "shape", type(pairs))}')
+        if pairs.dtype not in (torch.int32, torch.int64):
+            raise ValueError(f'pairs must be int32 or int64, got {pairs.dtype}')
+        if pairs.device != images.device:
+            raise ValueError(f'pairs are on {pairs.device}, images on {images.device}')
+        if pairs.dtype == torch.int64:      # out-of-range values stay out of range
+            pairs = pairs.clamp(-2 ** 31, 2 ** 31 - 1)
+        pairs = pairs.to(torch.int32).contiguous()
+        n, n_pairs = images.shape[0], pairs.shape[0]
+        if out is None:
+            out = torch.empty((n_pairs, self.num_classes), dtype=torch.float32, device=images.device)
+        elif (out.shape != (n_pairs, self.num_classes) or out.dtype != torch.float32 or out.device != images.device
+              or not out.is_contiguous()):
+            raise ValueError(f'out must be a contiguous fp32 [{n_pairs}, {self.num_classes}] tensor on {images.device}')
+        if n_pairs == 0:
+            return out
+        eng = self._ensure_engine(images.device)
+        entry, name = ((_lib.lib.vited_score_pairs_u8, 'vited_score_pairs_u8') if u8 else
+                       (_lib.lib.vited_score_pairs, 'vited_score_pairs'))
+        _lib.check(entry(eng, images.data_ptr(), n, pairs.data_ptr(), n_pairs, out.data_ptr(),
                          self._stream(images.device)), name)
         return out
 
