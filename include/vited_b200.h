@@ -226,6 +226,45 @@ VITED_API int vited_train_attention(int backward, const void* q, int q_ld, const
 VITED_API int vited_train_bce_logits(const float* logits, const float* labels, int n, float* loss, float* dlogits,
                                      float grad_scale, void* stream);
 
+/* ---- Hisfrag training iteration: overflow detection, gradient clipping, AdamW ----
+ * The 16-bit conversions of this library saturate (fp16 at +-65504) instead of producing inf, so an overflowing
+ * loss-scaled gradient is finite and silently wrong; these entry points let the host detect it, skip the step and back
+ * off the scale (vit-ed_b200/train.py train_iteration). `flag` is one int32 on the device, sticky: entry points set it
+ * to 1 and never clear it.
+ *   range_limit: |x| from which a value does not survive the 16-bit conversion: 65504 (fp16 builds) or +inf (bf16
+ *                builds, where only non-finite values count)
+ *   range_check: *flag = 1 if any of x[0, n) (f32 if is_f32, else h16) is non-finite or has |x| >= limit; any element
+ *                offset and any n >= 0
+ *   attention_chk: vited_train_attention, and in the backward pass *flag = 1 when a dS = P (dP - D) scale value of the
+ *                tensor-core kernels is out of range before its conversion to h16 (|dS| can reach about
+ *                2 |dO_i| max_j |V_j| scale with dO in range). flag NULL = vited_train_attention. The fp32 kernels of
+ *                other head dims convert nothing and leave the flag alone. */
+/* replaces: the found_inf check of GradScaler (torch.amp, misc/engine.py:189-257) */
+VITED_API float vited_train_range_limit(void);
+VITED_API int vited_train_range_check(const void* x, int is_f32, int64_t n, float limit, int32_t* flag, void* stream);
+/* replaces: the backward of the attention (misc/engine.py:189-257 autograd) with GradScaler's overflow check */
+VITED_API int vited_train_attention_chk(int backward, const void* q, int q_ld, const void* k, int k_ld, const void* v,
+                                        int v_ld, void* o, int o_ld, float* lse, const float* d_o, int do_ld, float* dsum,
+                                        float* dq, int dq_ld, float* dk, int dk_ld, float* dv, int dv_ld, int n_seq, int H,
+                                        int hd, int Tq, int Tk, float scale, int32_t* flag, void* stream);
+/* replaces: the total norm of clip_grad_norm_(params, 5.0) (misc/utils.py:206-226).
+ * table [n_tensors, 2] int64 on the device: (pointer to f32 gradient, numel) per tensor. Sum of squares in fp64 over a
+ * fixed partition (n_partials blocks, partials [n_partials] f64 workspace) and a fixed-order final sum: bit-reproducible
+ * for a given table and n_partials. out_sumsq_and_flag: 8 bytes, 8-byte aligned: out[0] = (float) sum of squares, the
+ * int32 after it is a sticky flag set to 1 when that value is non-finite. */
+VITED_API int vited_train_grad_norm(const int64_t* table, int n_tensors, double* partials, int n_partials,
+                                    float* out_sumsq_and_flag, void* stream);
+/* replaces: optimizer.step() of torch.optim.AdamW (misc/optimizer.py:12-46) after clip_grad_norm_.
+ * table [n_tensors, 6] int64 on the device: (param, grad, exp_avg, exp_avg_sq pointers (f32, numel elements each),
+ * numel, weight decay as the bit pattern of a double) per tensor; max_numel = the largest numel. One step of the
+ * single-tensor form of torch.optim.AdamW operation for operation, with g = grad * clip_coef:
+ *   p *= 1 - lr wd;  m = lerp(m, g, 1 - beta1);  v = beta2 v + (1 - beta2) g^2;
+ *   p -= (lr / bias_correction1) m / (sqrt(v) / sqrt(bias_correction2) + eps)
+ * with bias_correction{1,2} = 1 - beta{1,2}^t computed by the caller in double. grad is read, never written. */
+VITED_API int vited_train_adamw(const int64_t* table, int n_tensors, int64_t max_numel, double lr, double beta1,
+                                double beta2, double eps, float clip_coef, double bias_correction1,
+                                double bias_correction2, void* stream);
+
 /* ---- consumer side of the puzzle grid (SURVEY 8f row 3) ----
  * replaces: the tables InterPieceDistance.__init__ fills through 4*N*(N-1) callbacks into evaluation.py:116-131's
  * distance_function -- PieceDistanceInformation.calculate_inter_piece_distances (paikin_tal_solver/

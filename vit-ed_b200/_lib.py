@@ -49,6 +49,7 @@ _vp = ctypes.c_void_p
 _i = ctypes.c_int
 _i64 = ctypes.c_int64
 _f = ctypes.c_float
+_d = ctypes.c_double
 
 # name -> (restype, argtypes); kept in one table so tests can check it against the header
 SIGNATURES = {
@@ -89,6 +90,12 @@ SIGNATURES = {
     "vited_train_attention": (_i, [_i, _vp, _i, _vp, _i, _vp, _i, _vp, _i, _vp, _vp, _i, _vp, _vp, _i, _vp, _i, _vp, _i, _i, _i,
                                    _i, _i, _i, _f, _vp]),
     "vited_train_bce_logits": (_i, [_vp, _vp, _i, _vp, _vp, _f, _vp]),
+    "vited_train_range_limit": (_f, []),
+    "vited_train_range_check": (_i, [_vp, _i, _i64, _f, _vp, _vp]),
+    "vited_train_attention_chk": (_i, [_i, _vp, _i, _vp, _i, _vp, _i, _vp, _i, _vp, _vp, _i, _vp, _vp, _i, _vp, _i, _vp, _i, _i,
+                                       _i, _i, _i, _i, _f, _vp, _vp]),
+    "vited_train_grad_norm": (_i, [_vp, _i, _vp, _i, _vp, _vp]),
+    "vited_train_adamw": (_i, [_vp, _i, _i64, _d, _d, _d, _d, _f, _d, _d, _vp]),
     "vited_op_gemm": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
     "vited_op_gemm_resid_ln": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _f, _vp]),
     "vited_op_mlp_resid_ln": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _f, _vp]),
@@ -126,6 +133,13 @@ def act_dtype():
 
 
 ACT_NAME = 'bf16' if lib.vited_act_dtype() == 1 else 'fp16'
+
+
+def range_limit():
+    """|x| from which a value does not survive this build's 16-bit conversion: 65504.0 (fp16, where conversions
+    saturate) or inf (bf16, where only non-finite values are lost). ``vited_train_range_check`` flags values at or
+    beyond it."""
+    return float(lib.vited_train_range_limit())
 
 
 def last_error() -> str:

@@ -1174,6 +1174,27 @@ int vited_train_bce_logits(const float* logits, const float* labels, int n, floa
                            void* stream) {
   return train_bce_logits(logits, labels, n, loss, dlogits, grad_scale, (cudaStream_t)stream);
 }
+int vited_train_attention_chk(int backward, const void* q, int q_ld, const void* k, int k_ld, const void* v, int v_ld,
+                              void* o, int o_ld, float* lse, const float* d_o, int do_ld, float* dsum, float* dq, int dq_ld,
+                              float* dk, int dk_ld, float* dv, int dv_ld, int n_seq, int H, int hd, int Tq, int Tk,
+                              float scale, int32_t* flag, void* stream) {
+  return train_attention(backward, (const act_t*)q, q_ld, (const act_t*)k, k_ld, (const act_t*)v, v_ld, (act_t*)o, o_ld, lse,
+                         d_o, do_ld, dsum, dq, dq_ld, dk, dk_ld, dv, dv_ld, n_seq, H, hd, Tq, Tk, scale, (cudaStream_t)stream,
+                         flag);
+}
+float vited_train_range_limit(void) { return train_range_limit(); }
+int vited_train_range_check(const void* x, int is_f32, int64_t n, float limit, int32_t* flag, void* stream) {
+  return train_range_check(x, is_f32, n, limit, flag, (cudaStream_t)stream);
+}
+int vited_train_grad_norm(const int64_t* table, int n_tensors, double* partials, int n_partials, float* out_sumsq_and_flag,
+                          void* stream) {
+  return train_grad_norm(table, n_tensors, partials, n_partials, out_sumsq_and_flag, (cudaStream_t)stream);
+}
+int vited_train_adamw(const int64_t* table, int n_tensors, int64_t max_numel, double lr, double beta1, double beta2,
+                      double eps, float clip_coef, double bias_correction1, double bias_correction2, void* stream) {
+  return train_adamw(table, n_tensors, max_numel, lr, beta1, beta2, eps, clip_coef, bias_correction1, bias_correction2,
+                     (cudaStream_t)stream);
+}
 
 int vited_prepare_pieces(const uint8_t* lab_image, int H, int W, int piece_width, int side, int off, int out_size,
                          float* out, int* n_pieces, void* stream) {

@@ -162,15 +162,33 @@ int train_gather_rows(const float* in, const int* idx, float* out, int n_blocks,
                       int in_row_off, int out_block_stride, int out_row_off, int D, int accumulate, cudaStream_t s);
 int train_scatter_add_rows(const float* src, const int* idx, float* dst, int n_blocks, int rows_per, int src_block_stride,
                            int src_row_off, int dst_block_stride, int dst_row_off, int D, float alpha, cudaStream_t s);
+// flag non-null (backward only): *flag = 1 when a dS value of the tensor-core kernels does not survive its conversion to
+// the 16-bit type (kActRangeLimit); the fp32 SIMT kernels convert nothing and never touch it
 int train_attention(int backward, const act_t* q, int q_ld, const act_t* k, int k_ld, const act_t* v, int v_ld, act_t* o,
                     int o_ld, float* lse, const float* d_o, int do_ld, float* dsum, float* dq, int dq_ld, float* dk, int dk_ld,
-                    float* dv, int dv_ld, int n_seq, int H, int hd, int Tq, int Tk, float scale, cudaStream_t s);
+                    float* dv, int dv_ld, int n_seq, int H, int hd, int Tq, int Tk, float scale, cudaStream_t s,
+                    int* flag = nullptr);
 // tensor-core (wmma) version of train_attention for head_dim 32 / 64 (train_attn.cu); the backward pass also reads the
 // forward output o (D_i = do_i . o_i)
 bool train_attention_wmma_supported(int hd);
 int train_attention_wmma(int backward, const act_t* q, int q_ld, const act_t* k, int k_ld, const act_t* v, int v_ld, act_t* o,
                          int o_ld, float* lse, const float* d_o, int do_ld, float* dsum, float* dq, int dq_ld, float* dk,
-                         int dk_ld, float* dv, int dv_ld, int n_seq, int H, int hd, int Tq, int Tk, float scale, cudaStream_t s);
+                         int dk_ld, float* dv, int dv_ld, int n_seq, int H, int hd, int Tq, int Tk, float scale, cudaStream_t s,
+                         int* flag = nullptr);
+
+// ---- the optimiser side of a training iteration (train_optim.cu): see include/vited_b200.h ----
+// |x| from which a value does not survive the conversion to the 16-bit type: fp16 conversions saturate at 65504 (f2act),
+// bf16 has the fp32 exponent range and loses only non-finite values
+#if VITED_ACT_BF16
+constexpr float kActRangeLimit = __builtin_huge_valf();
+#else
+constexpr float kActRangeLimit = 65504.f;
+#endif
+float train_range_limit();
+int train_range_check(const void* x, int is_f32, int64_t n, float limit, int* flag, cudaStream_t s);
+int train_grad_norm(const int64_t* table, int n_tensors, double* partials, int n_partials, float* out, cudaStream_t s);
+int train_adamw(const int64_t* table, int n_tensors, int64_t max_numel, double lr, double beta1, double beta2, double eps,
+                float clip_coef, double bc1, double bc2, cudaStream_t s);
 int train_bce_logits(const float* logits, const float* labels, int n, float* loss, float* dlogits, float grad_scale,
                      cudaStream_t s);
 

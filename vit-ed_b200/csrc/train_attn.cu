@@ -196,13 +196,22 @@ struct BwdSmem {
   static constexpr size_t BYTES = 4 * BR * Ld<HD>::H * 2 + kWarps * kWarpBytes + 2 * BR * 4 + 128;
 };
 
+// CHK: *flag = 1 when a dS value is out of the 16-bit range (|dS| can reach about 2 |dO_i| max_j |V_j| scale even
+// when dO is in range); the flag is the last parameter so that the unchecked form keeps its parameter layout
+template <bool CHK>
+__device__ __forceinline__ void report_out_of_range(bool bad, int* flag) {
+  if constexpr (CHK) {
+    if (__any_sync(0xffffffffu, bad) && (threadIdx.x & 31) == 0) *flag = 1;
+  }
+}
+
 // dK, dV of 64 key rows (16 per warp); streams the query blocks
-template <int HD>
+template <int HD, bool CHK>
 __global__ void __launch_bounds__(32 * kWarps)
 attn_wmma_bwd_dkv_kernel(const act_t* __restrict__ q, int q_ld, const act_t* __restrict__ k, int k_ld,
                          const act_t* __restrict__ v, int v_ld, const float* __restrict__ d_o, int do_ld,
                          const float* __restrict__ lse, const float* __restrict__ dsum, float* __restrict__ dk, int dk_ld,
-                         float* __restrict__ dv, int dv_ld, int H, int Tq, int Tk, float scale) {
+                         float* __restrict__ dv, int dv_ld, int H, int Tq, int Tk, float scale, int* __restrict__ flag) {
   extern __shared__ __align__(128) uint8_t smem_raw[];
   act_t* sK = reinterpret_cast<act_t*>(smem_raw);
   act_t* sV = sK + BR * Ld<HD>::H;
@@ -228,6 +237,7 @@ attn_wmma_bwd_dkv_kernel(const act_t* __restrict__ q, int q_ld, const act_t* __r
   for (int n = 0; n < HD / 16; ++n) { wmma::fill_fragment(acc_dk[n], 0.f); wmma::fill_fragment(acc_dv[n], 0.f); }
   const int r = lane >> 1, half = lane & 1;
   const bool key_ok = k0 + warp * 16 + r < Tk;
+  bool bad = false;
   for (int q0 = 0; q0 < Tq; q0 += BC) {
     __syncthreads();
     load_tile16<HD>(sQ, q + ((size_t)s * Tq + q0) * q_ld + h * HD, q_ld, Tq - q0, threadIdx.x, 32 * kWarps);
@@ -248,6 +258,7 @@ attn_wmma_bwd_dkv_kernel(const act_t* __restrict__ q, int q_ld, const act_t* __r
       if (key_ok && q0 + c < Tq) {
         p = expf(sS[r * LDS_F + c] * scale - sLse[c]);
         ds = p * (sDP[r * LDS_F + c] - sD[c]) * scale;
+        if constexpr (CHK) bad |= !(fabsf(ds) < kActRangeLimit);
       }
       sP[r * LDS_H + c] = f2act(p);
       sDS[r * LDS_H + c] = f2act(ds);
@@ -270,15 +281,16 @@ attn_wmma_bwd_dkv_kernel(const act_t* __restrict__ q, int q_ld, const act_t* __r
     }
     __syncwarp();
   }
+  report_out_of_range<CHK>(bad, flag);
 }
 
 // dQ of 64 query rows (16 per warp); streams the key blocks
-template <int HD>
+template <int HD, bool CHK>
 __global__ void __launch_bounds__(32 * kWarps)
 attn_wmma_bwd_dq_kernel(const act_t* __restrict__ q, int q_ld, const act_t* __restrict__ k, int k_ld,
                         const act_t* __restrict__ v, int v_ld, const float* __restrict__ d_o, int do_ld,
                         const float* __restrict__ lse, const float* __restrict__ dsum, float* __restrict__ dq, int dq_ld,
-                        int H, int Tq, int Tk, float scale) {
+                        int H, int Tq, int Tk, float scale, int* __restrict__ flag) {
   extern __shared__ __align__(128) uint8_t smem_raw[];
   act_t* sQ = reinterpret_cast<act_t*>(smem_raw);
   act_t* sDO = sQ + BR * Ld<HD>::H;
@@ -304,6 +316,7 @@ attn_wmma_bwd_dq_kernel(const act_t* __restrict__ q, int q_ld, const act_t* __re
   FragC acc[HD / 16];
 #pragma unroll
   for (int n = 0; n < HD / 16; ++n) wmma::fill_fragment(acc[n], 0.f);
+  bool bad = false;
   for (int k0 = 0; k0 < Tk; k0 += BC) {
     __syncthreads();
     load_tile16<HD>(sK, k + ((size_t)s * Tk + k0) * k_ld + h * HD, k_ld, Tk - k0, threadIdx.x, 32 * kWarps);
@@ -319,6 +332,7 @@ attn_wmma_bwd_dq_kernel(const act_t* __restrict__ q, int q_ld, const act_t* __re
       if (q_ok && k0 + c < Tk) {
         const float p = expf(sS[r * LDS_F + c] * scale - my_lse);
         ds = p * (sDP[r * LDS_F + c] - my_d) * scale;
+        if constexpr (CHK) bad |= !(fabsf(ds) < kActRangeLimit);
       }
       sDS[r * LDS_H + c] = f2act(ds);
     }
@@ -333,17 +347,18 @@ attn_wmma_bwd_dq_kernel(const act_t* __restrict__ q, int q_ld, const act_t* __re
     float* dst = dq + ((size_t)s * Tq + qi) * dq_ld + h * HD;
     for (int d = half * (HD / 2); d < (half + 1) * (HD / 2); ++d) dst[d] += sT[r * Ld<HD>::F + d];
   }
+  report_out_of_range<CHK>(bad, flag);
 }
 
-template <int HD>
+template <int HD, bool CHK>
 int launch_wmma(int backward, const act_t* q, int q_ld, const act_t* k, int k_ld, const act_t* v, int v_ld, act_t* o,
                 int o_ld, float* lse, const float* d_o, int do_ld, float* dsum, float* dq, int dq_ld, float* dk, int dk_ld,
-                float* dv, int dv_ld, int n_seq, int H, int Tq, int Tk, float scale, cudaStream_t s) {
+                float* dv, int dv_ld, int n_seq, int H, int Tq, int Tk, float scale, cudaStream_t s, int* flag) {
   static PerDeviceOnce once;
   if (once.first()) {
     VITED_CUDA_OK(cudaFuncSetAttribute(attn_wmma_fwd_kernel<HD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FwdSmem<HD>::BYTES));
-    VITED_CUDA_OK(cudaFuncSetAttribute(attn_wmma_bwd_dkv_kernel<HD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BwdSmem<HD>::BYTES));
-    VITED_CUDA_OK(cudaFuncSetAttribute(attn_wmma_bwd_dq_kernel<HD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BwdSmem<HD>::BYTES));
+    VITED_CUDA_OK(cudaFuncSetAttribute(attn_wmma_bwd_dkv_kernel<HD, CHK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BwdSmem<HD>::BYTES));
+    VITED_CUDA_OK(cudaFuncSetAttribute(attn_wmma_bwd_dq_kernel<HD, CHK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BwdSmem<HD>::BYTES));
   }
   const int qblocks = n_seq * H * ((Tq + BR - 1) / BR), kblocks = n_seq * H * ((Tk + BR - 1) / BR);
   if (!backward) {
@@ -354,11 +369,11 @@ int launch_wmma(int backward, const act_t* q, int q_ld, const act_t* k, int k_ld
     if (blocks > 148 * 16) blocks = 148 * 16;
     attn_dsum_kernel<<<blocks, 256, 0, s>>>(d_o, do_ld, o, o_ld, dsum, n_seq, H, HD, Tq);
     VITED_CUDA_OK(cudaGetLastError());
-    attn_wmma_bwd_dkv_kernel<HD><<<kblocks, 32 * kWarps, BwdSmem<HD>::BYTES, s>>>(q, q_ld, k, k_ld, v, v_ld, d_o, do_ld, lse, dsum, dk,
-                                                                                  dk_ld, dv, dv_ld, H, Tq, Tk, scale);
+    attn_wmma_bwd_dkv_kernel<HD, CHK><<<kblocks, 32 * kWarps, BwdSmem<HD>::BYTES, s>>>(q, q_ld, k, k_ld, v, v_ld, d_o, do_ld, lse, dsum,
+                                                                                       dk, dk_ld, dv, dv_ld, H, Tq, Tk, scale, flag);
     VITED_CUDA_OK(cudaGetLastError());
-    attn_wmma_bwd_dq_kernel<HD><<<qblocks, 32 * kWarps, BwdSmem<HD>::BYTES, s>>>(q, q_ld, k, k_ld, v, v_ld, d_o, do_ld, lse, dsum, dq,
-                                                                                 dq_ld, H, Tq, Tk, scale);
+    attn_wmma_bwd_dq_kernel<HD, CHK><<<qblocks, 32 * kWarps, BwdSmem<HD>::BYTES, s>>>(q, q_ld, k, k_ld, v, v_ld, d_o, do_ld, lse, dsum,
+                                                                                      dq, dq_ld, H, Tq, Tk, scale, flag);
   }
   VITED_CUDA_OK(cudaGetLastError());
   return 0;
@@ -371,12 +386,12 @@ bool train_attention_wmma_supported(int hd) { return hd == 32 || hd == 64; }
 // o (16-bit, the forward output) is an INPUT of the backward pass here: D_i = do_i . o_i
 int train_attention_wmma(int backward, const act_t* q, int q_ld, const act_t* k, int k_ld, const act_t* v, int v_ld, act_t* o,
                          int o_ld, float* lse, const float* d_o, int do_ld, float* dsum, float* dq, int dq_ld, float* dk,
-                         int dk_ld, float* dv, int dv_ld, int n_seq, int H, int hd, int Tq, int Tk, float scale, cudaStream_t s) {
-  if (hd == 32)
-    return launch_wmma<32>(backward, q, q_ld, k, k_ld, v, v_ld, o, o_ld, lse, d_o, do_ld, dsum, dq, dq_ld, dk, dk_ld, dv, dv_ld,
-                           n_seq, H, Tq, Tk, scale, s);
-  return launch_wmma<64>(backward, q, q_ld, k, k_ld, v, v_ld, o, o_ld, lse, d_o, do_ld, dsum, dq, dq_ld, dk, dk_ld, dv, dv_ld,
-                         n_seq, H, Tq, Tk, scale, s);
+                         int dk_ld, float* dv, int dv_ld, int n_seq, int H, int hd, int Tq, int Tk, float scale, cudaStream_t s,
+                         int* flag) {
+  auto* launch = hd == 32 ? (flag ? launch_wmma<32, true> : launch_wmma<32, false>)
+                          : (flag ? launch_wmma<64, true> : launch_wmma<64, false>);
+  return launch(backward, q, q_ld, k, k_ld, v, v_ld, o, o_ld, lse, d_o, do_ld, dsum, dq, dq_ld, dk, dk_ld, dv, dv_ld, n_seq, H,
+                Tq, Tk, scale, s, flag);
 }
 
 }  // namespace vited

@@ -461,7 +461,7 @@ int train_scatter_add_rows(const float* src, const int* idx, float* dst, int n_b
 }
 int train_attention(int backward, const act_t* q, int q_ld, const act_t* k, int k_ld, const act_t* v, int v_ld, act_t* o,
                     int o_ld, float* lse, const float* d_o, int do_ld, float* dsum, float* dq, int dq_ld, float* dk, int dk_ld,
-                    float* dv, int dv_ld, int n_seq, int H, int hd, int Tq, int Tk, float scale, cudaStream_t s) {
+                    float* dv, int dv_ld, int n_seq, int H, int hd, int Tq, int Tk, float scale, cudaStream_t s, int* flag) {
   if (n_seq == 0) return 0;
   static const int simt = [] { const char* e = getenv("VITED_TRAIN_ATTN_SIMT"); return e ? atoi(e) : 0; }();
   VITED_CHECK(hd % 8 == 0 && q_ld % 8 == 0 && k_ld % 8 == 0 && v_ld % 8 == 0, "train attention: head_dim / strides must be multiples of 8");
@@ -473,7 +473,7 @@ int train_attention(int backward, const act_t* q, int q_ld, const act_t* k, int 
       VITED_CHECK(d_o && dsum && dq && dk && dv && do_ld % 4 == 0 && (reinterpret_cast<uintptr_t>(d_o) & 15) == 0,
                   "train attention backward: bad arguments");
     return train_attention_wmma(backward, q, q_ld, k, k_ld, v, v_ld, o, o_ld, lse, d_o, do_ld, dsum, dq, dq_ld, dk, dk_ld, dv,
-                                dv_ld, n_seq, H, hd, Tq, Tk, scale, s);
+                                dv_ld, n_seq, H, hd, Tq, Tk, scale, s, flag);
   }
   const int tmax = Tq > Tk ? Tq : Tk;
   const size_t smem = (size_t)kAttnWarps * 2 * tmax * sizeof(float);

@@ -9,12 +9,18 @@ attention (forward and backward), residual adds, gathers / scatter-adds and the 
 csrc/train_ops.cu. Gradients carry a loss scale (default 1024) while they are 16-bit GEMM operands and are unscaled when
 accumulated into the fp32 parameter gradients. There is no PyTorch autograd and no CPU path.
 
+``train_iteration`` completes the reference's iteration (misc/engine.py:189-257, misc/utils.py:206-226) on the device:
+the same step with overflow detection for the loss-scaled 16-bit gradients (``LossScaler``, GradScaler's rule),
+gradient-norm clipping and a fused ``AdamW`` step (csrc/train_optim.cu).
+
 Not built yet (DESIGN.md): tensor-core attention backward (the softmax attention here is a plain fp32 kernel pair),
-DDP gradient all-reduce overlap, the optimiser step.
+DDP gradient all-reduce overlap.
 """
 import ctypes
 import math
+import struct
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -47,14 +53,19 @@ def _p(t):
 
 
 class _Ops:
-    """One object per training step: device, stream, the 16-bit type, the loss scale and the gradient store."""
+    """One object per training step: device, stream, the 16-bit type, the loss scale and the gradient store. With an
+    overflow ``flag`` (one int32 on the device) every loss-scaled gradient that is converted to or from 16 bits is
+    range-checked into it; without one (``train_step``) nothing is checked and no extra kernel runs. ``grads``
+    (name -> zeroed fp32 tensor) makes the step accumulate into caller-owned gradient buffers."""
 
-    def __init__(self, device, loss_scale):
+    def __init__(self, device, loss_scale, flag=None, grads=None):
         self.dev = device
         self.act = _lib.act_dtype()
         self.S = float(loss_scale)
         self.stream = ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream)
-        self.grads = {}
+        self.flag = flag
+        self.limit = _lib.range_limit()
+        self.grads = dict(grads) if grads is not None else {}
         self.w16, self.w16t = {}, {}
         self.launches = 0
         self.profile = None          # {op name: [events]} when train_step(profile=True): per-kernel-class device time
@@ -87,6 +98,14 @@ class _Ops:
 
     def zeros(self, *shape, dtype=torch.float32):
         return torch.zeros(shape, dtype=dtype, device=self.dev)   # (cudaMemset: plumbing, not arithmetic)
+
+    def range_check(self, x):
+        """flag = 1 if the contiguous fp32 / 16-bit buffer x holds a value the 16-bit conversion cannot represent"""
+        if self.flag is None:
+            return
+        assert x.is_contiguous(), x.shape
+        self._chk(_lib.lib.vited_train_range_check(_p(x), 1 if x.dtype == torch.float32 else 0, x.numel(), self.limit,
+                                                   _p(self.flag), self.stream), 'train_range_check')
 
     # ---- casts / adds
     def cast(self, x32, scale=1.0):
@@ -162,10 +181,12 @@ class _Linear:
         inv = 1.0 / ops.S
         gw = ops.grad(self.prefix + '.weight', self.w32)
         gb = ops.grad(self.prefix + '.bias', self.b32)
+        ops.range_check(dy32)                                     # before its 16-bit transpose and cast
         # wgrad: dW[N, K] = dY^T[N, R] X[R, K]  ->  gemm(A = dY^T [N, Rp], W = X^T [K, Rp])
         dyt16 = ops.transpose(dy32)
         xt16 = ops.transpose(self.x16)
         dw16 = ops.gemm(dyt16, xt16, self.zero_bias_in)          # [n_pad, K]
+        ops.range_check(dw16)
         ops.to_f32(dw16[:self.n_out], out=gw.view(self.n_out, -1), alpha=inv, beta=1.0)
         if self.n_pad == self.n_out:
             ops._chk(_lib.lib.vited_train_colsum(_p(dy32), _p(gb), r, self.n_out, inv, ops.stream), 'train_colsum')
@@ -178,6 +199,7 @@ class _Linear:
         # dgrad: dX[R, K] = dY[R, N] W[N, K]  ->  gemm(A = dY16 [R, n_pad], W = W^T [K, n_pad])
         dy16 = ops.cast(dy32)
         dx16 = ops.gemm(dy16, self.w16t, self.zero_bias_in)
+        ops.range_check(dx16)
         return ops.to_f32(dx16)
 
 
@@ -216,9 +238,12 @@ def _attention(ops, backward, q, k, v, n_seq, heads, hd, tq, tk, o=None, lse=Non
         lse = ops.empty(n_seq, heads, tq)
     dsum = ops.empty(n_seq, heads, tq) if backward else None
     ld = lambda t: t.stride(0) if t is not None else 0
-    ops._chk(_lib.lib.vited_train_attention(1 if backward else 0, _p(q), ld(q), _p(k), ld(k), _p(v), ld(v), _p(o), ld(o),
-                                            _p(lse), _p(d_o), ld(d_o), _p(dsum), _p(dq), ld(dq), _p(dk), ld(dk), _p(dv), ld(dv),
-                                            n_seq, heads, hd, tq, tk, scale, ops.stream), 'train_attention')
+    args = (1 if backward else 0, _p(q), ld(q), _p(k), ld(k), _p(v), ld(v), _p(o), ld(o), _p(lse), _p(d_o), ld(d_o), _p(dsum),
+            _p(dq), ld(dq), _p(dk), ld(dk), _p(dv), ld(dv), n_seq, heads, hd, tq, tk, scale)
+    if backward and ops.flag is not None:     # dS = P (dP - D) scale is converted to 16 bits inside the kernel
+        ops._chk(_lib.lib.vited_train_attention_chk(*args, _p(ops.flag), ops.stream), 'train_attention_chk')
+    else:
+        ops._chk(_lib.lib.vited_train_attention(*args, ops.stream), 'train_attention')
     return o, lse
 
 
@@ -372,9 +397,9 @@ def train_step(model, samples, targets, generator=None, loss_scale=1024.0, group
         return out
 
 
-def _train_step(model, samples, groups, labels, loss_scale, profile=False):
+def _train_step(model, samples, groups, labels, loss_scale, profile=False, flag=None, grads=None):
     dev = samples.device
-    ops = _Ops(dev, loss_scale)
+    ops = _Ops(dev, loss_scale, flag, grads)
     if profile:
         ops.profile_begin()
     sd = {k: v.detach().float().contiguous() for k, v in model.state_dict().items()}
@@ -473,3 +498,255 @@ def _train_step(model, samples, groups, labels, loss_scale, profile=False):
     model.train_launches = ops.launches
     model.train_profile = ops.profile_read() if profile else None   # time between consecutive calls, by entry point
     return loss[0], logits, groups, labels
+
+
+# ----------------------------------------------------------------------------------------------------------------
+# the optimiser side of the iteration: loss scaling, gradient clipping, AdamW (csrc/train_optim.cu)
+# ----------------------------------------------------------------------------------------------------------------
+def _f32(x):
+    return float(np.float32(x))
+
+
+class LossScaler:
+    """Dynamic loss scale with ``torch.amp.GradScaler``'s update rule and defaults: after a step with an overflow the
+    scale is multiplied by ``backoff_factor`` and the step is skipped; after ``growth_interval`` consecutive clean steps
+    it is multiplied by ``growth_factor`` (if the result is finite in float32). The scale is a float32 value kept on
+    the host, because every training kernel takes it as a scalar. ``state_dict`` uses GradScaler's keys, so either
+    class loads the other's state."""
+
+    def __init__(self, init_scale=2. ** 16, growth_factor=2., backoff_factor=.5, growth_interval=2000):
+        if not growth_factor > 1.0:
+            raise ValueError('growth_factor must be > 1')
+        if not backoff_factor < 1.0:
+            raise ValueError('backoff_factor must be < 1')
+        self.scale = _f32(init_scale)
+        self.growth_factor, self.backoff_factor = float(growth_factor), float(backoff_factor)
+        self.growth_interval = int(growth_interval)
+        self._growth_tracker = 0
+
+    def update(self, found_inf):
+        """One step of torch's ``_amp_update_scale_`` (float32 scale, double factors)."""
+        if found_inf:
+            self.scale = _f32(self.scale * self.backoff_factor)
+            self._growth_tracker = 0
+            return
+        successful = self._growth_tracker + 1
+        if successful == self.growth_interval:
+            with np.errstate(over='ignore'):
+                grown = np.float32(self.scale * self.growth_factor)
+            if np.isfinite(grown):
+                self.scale = float(grown)
+            self._growth_tracker = 0
+        else:
+            self._growth_tracker = successful
+
+    def state_dict(self):
+        return {'scale': self.scale, 'growth_factor': self.growth_factor, 'backoff_factor': self.backoff_factor,
+                'growth_interval': self.growth_interval, '_growth_tracker': self._growth_tracker}
+
+    def load_state_dict(self, state_dict):
+        if not state_dict:
+            raise RuntimeError('The source state dict is empty, possibly because it was saved from a disabled instance.')
+        self.scale = _f32(state_dict['scale'])
+        self.growth_factor = float(state_dict['growth_factor'])
+        self.backoff_factor = float(state_dict['backoff_factor'])
+        self.growth_interval = int(state_dict['growth_interval'])
+        self._growth_tracker = int(state_dict['_growth_tracker'])
+
+
+def default_no_decay(name, param):
+    """The Swin-style ``set_weight_decay`` rule: 1-D parameters, ``*.bias`` and the model's ``no_weight_decay`` names
+    (``pos_embed``, ``cls_token``) get no weight decay."""
+    return param.dim() == 1 or name.endswith('.bias') or name in ('pos_embed', 'cls_token')
+
+
+def _double_bits(x):
+    return struct.unpack('<q', struct.pack('<d', float(x)))[0]
+
+
+class AdamW:
+    """``torch.optim.AdamW`` (single-tensor form) for the Hisfrag model, as one fused kernel per step over every
+    parameter, with the two parameter groups of the reference's ``build_optimizer`` (misc/optimizer.py:12-46): weight
+    decay ``weight_decay`` and 0 for the parameters ``default_no_decay`` selects. That rule is the Swin-style
+    ``set_weight_decay`` the reference is described as using; it has not been checked against misc/optimizer.py itself.
+    ``no_decay`` (a set of parameter names) replaces it.
+
+    Device state: ``exp_avg`` and ``exp_avg_sq`` in fp32, the gradient buffers ``train_iteration`` accumulates into
+    (one flat buffer with a slot for the overflow flag, so the all-reduce is one collective), and the pointer tables of
+    the norm and AdamW kernels, uploaded once (rebuilt if the parameters move). ``lr`` is an attribute the caller sets
+    before each step (the learning-rate schedule stays with the caller). ``state_dict`` / ``load_state_dict`` use
+    torch.optim.AdamW's format, so optimizer state moves between the two in both directions."""
+
+    N_PARTIALS = 148 * 8       # blocks of the gradient-norm kernel: part of what makes the norm bit-reproducible
+    _ALIGN = 128               # gradient / moment slots start at 512-byte boundaries, as torch allocations do
+
+    def __init__(self, model, lr, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.05, no_decay=None):
+        self.lr, self.betas, self.eps = float(lr), (float(betas[0]), float(betas[1])), float(eps)
+        self.weight_decay = float(weight_decay)
+        params = dict(model.named_parameters())
+        skip = set(no_decay) if no_decay is not None else {n for n, p in params.items() if default_no_decay(n, p)}
+        unknown = skip - set(params)
+        if unknown:
+            raise ValueError(f'no_decay names that are not parameters of the model: {sorted(unknown)[:5]}')
+        self.groups = [[n for n in params if n not in skip], [n for n in params if n in skip]]
+        self.group_decay = [self.weight_decay, 0.0]
+        self.names = self.groups[0] + self.groups[1]     # torch's parameter index order in the state_dict
+        self.t = 0
+        self.params = params
+        self.dev = next(iter(params.values())).device     # the step itself runs in train_iteration, on CUDA only
+        offs, total = [], 0
+        for n in self.names:
+            offs.append(total)
+            total += (params[n].numel() + self._ALIGN - 1) // self._ALIGN * self._ALIGN
+        z = lambda k: torch.zeros(k, dtype=torch.float32, device=self.dev)
+        self._grad_flat, self._m_flat, self._v_flat = z(total + 1), z(total), z(total)   # + 1: the flag's slot
+        view = lambda flat, n, o: flat[o:o + params[n].numel()].view(params[n].shape)
+        self.grads = {n: view(self._grad_flat, n, o) for n, o in zip(self.names, offs)}
+        self.exp_avg = {n: view(self._m_flat, n, o) for n, o in zip(self.names, offs)}
+        self.exp_avg_sq = {n: view(self._v_flat, n, o) for n, o in zip(self.names, offs)}
+        self._status = torch.zeros(2, dtype=torch.int32, device=self.dev)   # (float sum of squares, int32 overflow flag)
+        self._partials = torch.empty(self.N_PARTIALS, dtype=torch.float64, device=self.dev)
+        self._ptrs = None
+        self._tables(model)
+
+    def _tables(self, model):
+        """Validates every (param, grad, exp_avg, exp_avg_sq) and uploads the kernels' tables, unless the parameters
+        are where the current tables point."""
+        params = dict(model.named_parameters())
+        if sorted(params) != sorted(self.names):
+            raise ValueError('the model does not have the parameters this optimizer was built for')
+        self.params = params
+        ptrs = tuple(params[n].data_ptr() for n in self.names)
+        if ptrs == self._ptrs:
+            return
+        norm_rows, adam_rows = [], []
+        decay = {n: self.group_decay[g] for g, names in enumerate(self.groups) for n in names}
+        for n in self.names:
+            p, g, m, v = params[n], self.grads[n], self.exp_avg[n], self.exp_avg_sq[n]
+            for what, t in (('param', p), ('grad', g), ('exp_avg', m), ('exp_avg_sq', v)):
+                if t.device != self.dev or t.dtype != torch.float32 or not t.is_contiguous() or t.data_ptr() == 0:
+                    raise ValueError(f'{n}: {what} must be a contiguous fp32 tensor on {self.dev}')
+                if t.shape != p.shape:
+                    raise ValueError(f'{n}: {what} shape {tuple(t.shape)} != parameter shape {tuple(p.shape)}')
+            norm_rows.append([g.data_ptr(), g.numel()])
+            adam_rows.append([p.data_ptr(), g.data_ptr(), m.data_ptr(), v.data_ptr(), p.numel(), _double_bits(decay[n])])
+        self._norm_table = torch.tensor(norm_rows, dtype=torch.int64).to(self.dev)
+        self._adam_table = torch.tensor(adam_rows, dtype=torch.int64).to(self.dev)
+        self._max_numel = max(r[4] for r in adam_rows)
+        self._ptrs = ptrs
+
+    def _stream(self):
+        return ctypes.c_void_p(torch.cuda.current_stream(self.dev).cuda_stream)
+
+    def _grad_norm(self):
+        """sum of squares of every gradient into _status[0] (float bits), a non-finite one sets the flag _status[1]"""
+        _lib.check(_lib.lib.vited_train_grad_norm(_p(self._norm_table), len(self.names), _p(self._partials),
+                                                  self.N_PARTIALS, _p(self._status), self._stream()),
+                   'vited_train_grad_norm')
+
+    def _step(self, clip_coef):
+        self.t += 1
+        b1, b2 = self.betas
+        _lib.check(_lib.lib.vited_train_adamw(_p(self._adam_table), len(self.names), self._max_numel, self.lr, b1, b2,
+                                              self.eps, clip_coef, 1 - b1 ** float(self.t), 1 - b2 ** float(self.t),
+                                              self._stream()), 'vited_train_adamw')
+
+    def _torch_groups(self, params):
+        return [{'params': [params[n] for n in self.groups[0]], 'weight_decay': self.group_decay[0]},
+                {'params': [params[n] for n in self.groups[1]], 'weight_decay': self.group_decay[1]}]
+
+    def state_dict(self):
+        """torch.optim.AdamW(...).state_dict() of the same groups, hyperparameters, step and moments (copies)."""
+        ref = torch.optim.AdamW(self._torch_groups(self.params), lr=self.lr, betas=self.betas, eps=self.eps,
+                                weight_decay=self.weight_decay, foreach=False, fused=False)
+        sd = ref.state_dict()
+        if self.t > 0:
+            sd['state'] = {i: {'step': torch.tensor(float(self.t)), 'exp_avg': self.exp_avg[n].clone(),
+                               'exp_avg_sq': self.exp_avg_sq[n].clone()} for i, n in enumerate(self.names)}
+        return sd
+
+    def load_state_dict(self, state_dict):
+        """Loads a state_dict of this class or of torch.optim.AdamW over the same two groups."""
+        groups = state_dict['param_groups']
+        if [len(g['params']) for g in groups] != [len(self.groups[0]), len(self.groups[1])]:
+            raise ValueError('the state_dict does not have the decay / no-decay groups of this optimizer')
+        if len({g['lr'] for g in groups}) != 1 or len({tuple(g['betas']) for g in groups}) != 1 \
+                or len({g['eps'] for g in groups}) != 1:
+            raise ValueError('lr, betas and eps must be the same in both groups')
+        if any(g.get('amsgrad') or g.get('maximize') for g in groups):
+            raise ValueError('amsgrad / maximize are not supported')
+        self.lr, self.betas, self.eps = float(groups[0]['lr']), tuple(float(b) for b in groups[0]['betas']), float(groups[0]['eps'])
+        self.group_decay = [float(g['weight_decay']) for g in groups]
+        self.weight_decay = self.group_decay[0]
+        index = {i: n for g, names in zip(groups, self.groups) for i, n in zip(g['params'], names)}
+        state = state_dict['state']
+        steps = {float(s['step']) for s in state.values()}
+        if len(steps) > 1:
+            raise ValueError('all parameters must have taken the same number of steps')
+        if state and len(state) != len(self.names):
+            raise ValueError('the state_dict has state for only some of the parameters')
+        self.t = int(steps.pop()) if steps else 0
+        for n in self.names:
+            self.exp_avg[n].zero_()
+            self.exp_avg_sq[n].zero_()
+        for i, s in state.items():
+            self.exp_avg[index[int(i)]].copy_(s['exp_avg'])
+            self.exp_avg_sq[index[int(i)]].copy_(s['exp_avg_sq'])
+        self._ptrs = None        # the weight decays may have changed: rebuild the tables at the next step
+
+
+def _all_reduce_with_flag(flat, flag):
+    """all_reduce_gradients on the optimizer's flat gradient buffer, whose last slot carries the overflow flag: any
+    rank's overflow becomes every rank's, in the same SUM collective."""
+    import torch.distributed as dist
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size() == 1:
+        return
+    flat[-1:].copy_(flag)                        # (int32 -> fp32 device copy: plumbing)
+    dist.all_reduce(flat, op=dist.ReduceOp.SUM)
+    flat /= dist.get_world_size()
+    flag.copy_(flat[-1:] > 0)
+
+
+@torch.no_grad()
+def train_iteration(model, samples, targets, optimizer, scaler, clip_grad=5.0, generator=None, groups=None, labels=None,
+                    all_reduce=True):
+    """One iteration of the reference's training loop (misc/engine.py:189-257): ``train_step`` at the loss scale
+    ``scaler.scale`` with every 16-bit conversion of a loss-scaled gradient range-checked on the device, the gradient
+    all-reduce (the overflow flag travels in the same bucket), ``clip_grad_norm_(params, clip_grad)`` and an
+    ``optimizer`` (``AdamW``) step -- or, when any rank's gradient overflowed, no step and a smaller scale, as
+    ``GradScaler`` does. One 8-byte device-to-host read per call (GradScaler.step synchronises once too).
+
+    Returns (loss, logits, groups, labels, grad_norm, skipped). ``grad_norm`` is the total norm clip_grad_norm_ returns
+    (a float; inf for a skipped step). ``p.grad`` holds the unclipped averaged gradient afterwards; on a skipped step
+    the parameters, the moments and the step count are untouched."""
+    if not (isinstance(samples, torch.Tensor) and samples.is_cuda):
+        raise _lib.VitedError('train_iteration runs on CUDA (sm_100a) tensors only; there is no CPU fallback')
+    dev = samples.device
+    if groups is None:
+        groups, labels = prepare_pairs(targets, generator)
+    with torch.cuda.device(dev):
+        optimizer._tables(model)
+        status = optimizer._status
+        status.zero_()
+        optimizer._grad_flat.zero_()
+        flag = status[1:]
+        loss, logits, groups, labels = _train_step(model, samples.float().contiguous(), groups, labels, scaler.scale,
+                                                   flag=flag, grads=optimizer.grads)
+        if all_reduce:
+            _all_reduce_with_flag(optimizer._grad_flat, flag)
+        optimizer._grad_norm()
+        host = status.cpu()
+        found_inf = bool(host[1])
+        if found_inf:
+            scaler.update(True)
+            model.train_launches += 2
+            return loss, logits, groups, labels, math.inf, True
+        norm = np.float32(math.sqrt(float(host[:1].view(torch.float32))))
+        clip_coef = min(np.float32(1.0), np.float32(clip_grad) / (norm + np.float32(1e-6)))
+        optimizer._step(float(clip_coef))
+        scaler.update(False)
+        model.train_launches += 3
+        # the kernel wrote the parameters through raw pointers: bump their versions so that the scoring engine, which
+        # re-uploads its packed weights when a parameter's version changes, does not keep the old ones
+        torch.autograd.graph.increment_version(list(model.parameters()))
+        return loss, logits, groups, labels, float(norm), False
