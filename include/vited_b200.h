@@ -334,6 +334,16 @@ VITED_API int vited_op_resid_ln(float* x, const void* delta, const float* ln_w, 
 VITED_API int vited_op_attention(const void* q, int q_ld, const void* k, int k_ld, const void* v, int v_ld, void* o, int o_ld,
                        int n_seq, int n_heads, int head_dim, int nq_patch, int q_has_cls, int nk_patch,
                        int k_has_cls, int n_kv_seq, const int32_t* kv_index, float scale, int impl, void* stream);
+/* class-token query only (the pruned last decoder layer, vision_transformer.py:397-401: only token 0 reaches the head).
+ * q and o are full split-layout buffers of n_seq sequences of nk_patch patch rows + a class token; only their class-token
+ * rows (row n_seq*nk_patch + b) are read and written. k / v as in vited_op_attention. */
+VITED_API int vited_op_attention_cls(const void* q, int q_ld, const void* k, int k_ld, const void* v, int v_ld, void* o,
+                                     int o_ld, int n_seq, int n_heads, int head_dim, int nk_patch, int k_has_cls,
+                                     int n_kv_seq, const int32_t* kv_index, float scale, void* stream);
+/* final LayerNorm + head (vision_transformer.py:400, :417): y = LayerNorm(x[p] + delta[p]) * ln_w + ln_b;
+ * out[p*C + c] = y . head_w[c] + head_b[c]. x [P,D] f32, delta [P,D] h16 or NULL, head_w [C,D] f32, all in fp32 math. */
+VITED_API int vited_op_head(const float* x, const void* delta, const float* ln_w, const float* ln_b, const float* head_w,
+                            const float* head_b, float* out, int P, int D, int C, float eps, void* stream);
 /* images [B,C,S,S] f32 -> [B*(S/p)^2, C*p*p] h16 */
 VITED_API int vited_op_im2col(const float* images, void* out, int B, int C, int S, int p, void* stream);
 /* images [B,S,S,C] u8 -> the same [B*(S/p)^2, C*p*p] h16, bit-identical to vited_normalize_u8 + vited_op_im2col

@@ -103,6 +103,8 @@ SIGNATURES = {
                                          _vp]),
     "vited_op_resid_ln": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _f, _vp]),
     "vited_op_attention": (_i, [_vp, _i, _vp, _i, _vp, _i, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _f, _i, _vp]),
+    "vited_op_attention_cls": (_i, [_vp, _i, _vp, _i, _vp, _i, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _f, _vp]),
+    "vited_op_head": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _f, _vp]),
     "vited_op_im2col": (_i, [_vp, _vp, _i, _i, _i, _i, _vp]),
     "vited_op_im2col_u8": (_i, [_vp, _vp, _i, _i, _i, _i, _vp]),
 }

@@ -1113,6 +1113,26 @@ int vited_op_attention(const void* q, int q_ld, const void* k, int k_ld, const v
   return attention(a, impl, (cudaStream_t)stream);
 }
 
+int vited_op_attention_cls(const void* q, int q_ld, const void* k, int k_ld, const void* v, int v_ld, void* o, int o_ld,
+                           int n_seq, int n_heads, int head_dim, int nk_patch, int k_has_cls, int n_kv_seq,
+                           const int32_t* kv_index, float scale, void* stream) {
+  // the query side as L_attn_cls passes it: full split-layout buffers of nk_patch patch rows + one class token per sequence
+  AttnArgs a;
+  a.q = (const act_t*)q; a.q_ld = q_ld; a.k = (const act_t*)k; a.k_ld = k_ld; a.v = (const act_t*)v; a.v_ld = v_ld;
+  a.o = (act_t*)o; a.o_ld = o_ld; a.n_seq = n_seq; a.n_heads = n_heads; a.head_dim = head_dim;
+  a.nq_patch = nk_patch; a.q_has_cls = 1; a.nk_patch = nk_patch; a.k_has_cls = k_has_cls;
+  a.n_kv_seq = n_kv_seq; a.kv_index = kv_index; a.scale = scale;
+  return attention_cls(a, (cudaStream_t)stream);
+}
+
+int vited_op_head(const float* x, const void* delta, const float* ln_w, const float* ln_b, const float* head_w,
+                  const float* head_b, float* out, int P, int D, int C, float eps, void* stream) {
+  HeadArgs a = {};
+  a.x = x; a.delta = (const act_t*)delta; a.ln_w = ln_w; a.ln_b = ln_b; a.head_w = head_w; a.head_b = head_b;
+  a.out = out; a.P = P; a.D = D; a.C = C; a.eps = eps;
+  return head_logits(a, (cudaStream_t)stream);
+}
+
 int vited_op_im2col(const float* images, void* out, int B, int C, int S, int p, void* stream) {
   return im2col_patches(images, (act_t*)out, B, C, S, p, (cudaStream_t)stream);
 }

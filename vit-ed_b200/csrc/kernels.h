@@ -216,7 +216,8 @@ bool attention_pair_supported(const AttnArgs& a);
 int attention_pair(const AttnArgs& a, cudaStream_t stream);
 bool attention_tc_cls_supported(const AttnArgs& a);
 int attention_tc_cls(const AttnArgs& a, cudaStream_t stream);
-// class-token query only: q is [n_seq, q_ld] (one row per sequence), o likewise; nq_patch / q_has_cls are ignored.
+// class-token query only: q and o are the full split-layout buffers (q_has_cls = 1); only their class-token rows
+// (row n_seq*nq_patch + b) are read / written. The puzzle-shape warp kernel assumes nq_patch = 64.
 int attention_cls(const AttnArgs& a, cudaStream_t stream);
 
 }  // namespace vited
