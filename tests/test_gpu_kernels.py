@@ -2,7 +2,6 @@
 16-bit-rounded operands; fp16 unless the library was built with -DVITED_ACT_BF16=1). Tolerances are stated per test."""
 import ctypes
 import math
-import os
 
 import pytest
 import torch
@@ -47,7 +46,7 @@ GEMM_SHAPES = [
     (128, 128, 64), (256, 384, 384), (1000, 1152, 384), (4160, 384, 384), (777, 1536, 384), (640, 384, 1536),
     (65 * 37, 768, 384), (64 * 9, 384, 192), (300, 384, 768), (5, 32, 32), (130, 96, 3072), (1, 8, 8),
     (129, 1152, 384), (20000, 1152, 384),
-    # large-M, K<=384: the resident-weights variant of the tcgen05 kernel
+    # large M, K <= 384
     (30000, 1536, 384), (26000, 384, 384), (26001, 384, 192), (19999, 768, 384),
 ]
 
@@ -94,82 +93,37 @@ def test_gelu_epilogue_accuracy():
 
 
 @pytest.mark.parametrize('bn', ['128', '192', '256'])
-def test_gemm_tile_shapes_agree(bn, monkeypatch):
-    """Both BLOCK_N variants of the tcgen05 kernel must give the same answer (subprocess: the knob is read once)."""
-    import subprocess, sys, os
-    from tests.conftest import ROOT
-    code = (
-        "import torch, ctypes, math, sys; sys.path.insert(0, %r)\n"
-        "from vited_b200 import _lib as L\n"
-        "g = torch.Generator(device='cuda').manual_seed(1)\n"
-        "M, N, K = 1111, 1536, 384\n"
-        "A = torch.randn(M, K, device='cuda', generator=g).to(L.act_dtype()); W = (torch.randn(N, K, device='cuda', generator=g) / math.sqrt(K)).to(L.act_dtype())\n"
-        "b = torch.randn(N, device='cuda', generator=g); C = torch.zeros(M, N, dtype=L.act_dtype(), device='cuda')\n"
-        "st = L.lib.vited_op_gemm(A.data_ptr(), W.data_ptr(), b.data_ptr(), C.data_ptr(), M, N, K, 0, 0, None)\n"
-        "torch.cuda.synchronize(); assert st == 0, L.last_error()\n"
-        "ref = A.float() @ W.float().t() + b\n"
-        "err = (C.float() - ref).abs().max().item(); print('maxerr', err); assert err < 0.06\n"
-    ) % ROOT
-    env = dict(os.environ, VITED_GEMM_BN=bn)
-    r = subprocess.run([sys.executable, '-c', code], env=env, capture_output=True, text=True, timeout=300)
-    assert r.returncode == 0, r.stdout + r.stderr
+def test_gemm_tile_shapes_agree(bn):
+    """Each tile width of the single-CTA tcgen05 kernel, picked by N (the widest of 256 / 192 / 128 that divides it),
+    against torch."""
+    M, N, K = {'128': (1111, 640, 384), '192': (1111, 1152, 384), '256': (1111, 1536, 384)}[bn]
+    g = torch.Generator(device='cuda').manual_seed(1)
+    A = torch.randn(M, K, device='cuda', generator=g).to(_act())
+    W = (torch.randn(N, K, device='cuda', generator=g) / math.sqrt(K)).to(_act())
+    b = torch.randn(N, device='cuda', generator=g)
+    C = _gemm(A, W, b, 0, 0)
+    ref = A.float() @ W.float().t() + b
+    err = (C.float() - ref).abs().max().item()
+    assert err < 0.06, err
 
 
 def test_gemm_cta_pair_variant():
-    """The cta_group::2 (CTA-pair) variant of the tcgen05 kernel against torch (subprocess: env knob read once)."""
-    import subprocess, sys, os
-    from tests.conftest import ROOT
-    code = (
-        "import torch, math, sys; sys.path.insert(0, %r)\n"
-        "from vited_b200 import _lib as L\n"
-        "g = torch.Generator(device='cuda').manual_seed(1)\n"
-        "for (M, N, K, act) in [(40000, 1536, 384, 1), (40001, 384, 1536, 0), (38001, 1152, 384, 0), (40000, 384, 384, 0), (39990, 768, 384, 0)]:\n"
-        "    A = torch.randn(M, K, device='cuda', generator=g).to(L.act_dtype()); W = (torch.randn(N, K, device='cuda', generator=g) / math.sqrt(K)).to(L.act_dtype())\n"
-        "    b = torch.randn(N, device='cuda', generator=g); C = torch.full((M, N), float('nan'), dtype=L.act_dtype(), device='cuda')\n"
-        "    st = L.lib.vited_op_gemm(A.data_ptr(), W.data_ptr(), b.data_ptr(), C.data_ptr(), M, N, K, act, 0, None)\n"
-        "    torch.cuda.synchronize(); assert st == 0, L.last_error()\n"
-        "    ref = A.float() @ W.float().t() + b\n"
-        "    ref = torch.nn.functional.gelu(ref) if act else ref\n"
-        "    assert torch.isfinite(C.float()).all(), ('nan', M, N, K)\n"
-        "    err = (C.float() - ref).abs(); tol = 1e-2 * ref.abs() + 2e-2\n"
-        "    bad = err > tol\n"
-        "    assert not bad.any(), (M, N, K, int(bad.sum()), float(err.max()), bad.nonzero()[0].tolist())\n"
-        "    print('ok', M, N, K, float(err.max()))\n"
-    ) % ROOT
-    env = dict(os.environ, VITED_GEMM_PAIR='1')
-    r = subprocess.run([sys.executable, '-c', code], env=env, capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
-
-
-def test_gemm_quad_cluster_variant():
-    """The 4-CTA-cluster kernel (two cta_group::2 pairs sharing TMA-multicast weight tiles; a measured negative result
-    that only exists in -DVITED_EXPERIMENTAL builds, tools/build_variants.sh) against torch, including an odd number of
-    256-row blocks (the second pair of the last cluster computes on zero-filled rows)."""
-    import subprocess, sys, os
-    from tests.conftest import ROOT
-    lib = os.path.join(ROOT, 'tools', 'bin', 'experimental', 'libvited_b200.so')
-    if not os.path.exists(lib):
-        pytest.skip('no experimental build (tools/build_variants.sh)')
-    code = (
-        "import torch, math, sys; sys.path.insert(0, %r)\n"
-        "from vited_b200 import _lib as L\n"
-        "g = torch.Generator(device='cuda').manual_seed(1)\n"
-        "for (M, N, K, act) in [(80000, 1536, 384, 1), (80001, 384, 1536, 0), (76001, 1152, 384, 0), (79990, 768, 384, 0)]:\n"
-        "    A = torch.randn(M, K, device='cuda', generator=g).to(L.act_dtype()); W = (torch.randn(N, K, device='cuda', generator=g) / math.sqrt(K)).to(L.act_dtype())\n"
-        "    b = torch.randn(N, device='cuda', generator=g); C = torch.full((M, N), float('nan'), dtype=L.act_dtype(), device='cuda')\n"
-        "    st = L.lib.vited_op_gemm(A.data_ptr(), W.data_ptr(), b.data_ptr(), C.data_ptr(), M, N, K, act, 0, None)\n"
-        "    torch.cuda.synchronize(); assert st == 0, L.last_error()\n"
-        "    ref = A.float() @ W.float().t() + b\n"
-        "    ref = torch.nn.functional.gelu(ref) if act else ref\n"
-        "    assert torch.isfinite(C.float()).all(), ('nan', M, N, K)\n"
-        "    err = (C.float() - ref).abs(); tol = 1e-2 * ref.abs() + 2e-2\n"
-        "    bad = err > tol\n"
-        "    assert not bad.any(), (M, N, K, int(bad.sum()), float(err.max()), bad.nonzero()[0].tolist())\n"
-        "    print('ok', M, N, K, float(err.max()))\n"
-    ) % ROOT
-    env = dict(os.environ, VITED_GEMM_QUAD='1', VITED_LIB=lib)
-    r = subprocess.run([sys.executable, '-c', code], env=env, capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
+    """The cta_group::2 (CTA-pair) variant of the tcgen05 kernel, which takes M of at least two 128-row blocks per SM,
+    against torch."""
+    g = torch.Generator(device='cuda').manual_seed(1)
+    for (M, N, K, act) in [(40000, 1536, 384, 1), (40001, 384, 1536, 0), (38001, 1152, 384, 0), (40000, 384, 384, 0),
+                           (39990, 768, 384, 0)]:
+        A = torch.randn(M, K, device='cuda', generator=g).to(_act())
+        W = (torch.randn(N, K, device='cuda', generator=g) / math.sqrt(K)).to(_act())
+        b = torch.randn(N, device='cuda', generator=g)
+        C = _gemm(A, W, b, act, 0)
+        ref = A.float() @ W.float().t() + b
+        ref = torch.nn.functional.gelu(ref) if act else ref
+        assert torch.isfinite(C.float()).all(), ('nan', M, N, K)
+        err = (C.float() - ref).abs()
+        tol = 1e-2 * ref.abs() + 2e-2
+        bad = err > tol
+        assert not bad.any(), (M, N, K, int(bad.sum()), float(err.max()), bad.nonzero()[0].tolist())
 
 
 @pytest.mark.parametrize('D', [384, 768, 32, 96])
@@ -194,21 +148,12 @@ def test_resid_ln(D, has_cls):
     assert (h.float() - h_ref).abs().max().item() <= (1e-2 * h_ref.abs().max().item() + 1e-3) * _r16()
 
 
-def _epi_variant(epi_warps, monkeypatch):
-    """The 16-warp (four column groups) form of the two full-row epilogues is a measured-neutral variant that only exists
-    in -DVITED_EXPERIMENTAL builds (tools/build_variants.sh; select with VITED_LIB=tools/bin/experimental/...)."""
-    if epi_warps == '16' and 'experimental' not in os.environ.get('VITED_LIB', ''):
-        pytest.skip('16 epilogue warps: experimental build only (VITED_LIB=tools/bin/experimental/libvited_b200.so)')
-    monkeypatch.setenv('VITED_EPI_WARPS', epi_warps)
-
-
 @pytest.mark.parametrize('shape', [(256, 384), (70000, 384), (33333, 1536), (1, 384), (300, 64), (40000, 192)],
                          ids=lambda s: 'x'.join(map(str, s)))
-@pytest.mark.parametrize('epi_warps', ['8', '16'])
-def test_gemm_resid_ln_fused(shape, epi_warps, monkeypatch):
-    """x += A W^T + b; h = LayerNorm(x): the fused tcgen05 epilogue against fp32 torch on the same 16-bit operands,
-    in both epilogue forms (8 warps x 192-column half rows, 16 warps x 96-column quarter rows)."""
-    _epi_variant(epi_warps, monkeypatch)
+@pytest.mark.parametrize('epi_warps', ['8'])
+def test_gemm_resid_ln_fused(shape, epi_warps):
+    """x += A W^T + b; h = LayerNorm(x): the fused tcgen05 epilogue (8 warps x 192-column half rows) against fp32 torch
+    on the same 16-bit operands."""
     L = _lib()
     M, K = shape
     N = 384
@@ -235,13 +180,11 @@ def test_gemm_resid_ln_fused(shape, epi_warps, monkeypatch):
 
 @pytest.mark.parametrize('shape', [(256, 1536), (70000, 1536), (33333, 1536), (1, 1536), (300, 64), (40000, 192),
                                    (262144 + 77, 1536)], ids=lambda s: 'x'.join(map(str, s)))
-@pytest.mark.parametrize('epi_warps', ['8', '16'])
-def test_mlp_resid_ln_fused(shape, epi_warps, monkeypatch):
+@pytest.mark.parametrize('epi_warps', ['8'])
+def test_mlp_resid_ln_fused(shape, epi_warps):
     """x += fc2(GELU(fc1(h))) + b2; h = LayerNorm(x): the fused MLP kernel (hidden activations kept in TMEM, GELU
     output fed to the second MMA as its A operand from TMEM) against fp32 torch on the same 16-bit operands, with the
-    hidden activations rounded to 16 bits where the kernel rounds them. In place: h_out aliases h_in. Both epilogue
-    forms (VITED_EPI_WARPS = 8 / 16)."""
-    _epi_variant(epi_warps, monkeypatch)
+    hidden activations rounded to 16 bits where the kernel rounds them. In place: h_out aliases h_in."""
     L = _lib()
     M, HID = shape
     D = 384
@@ -375,19 +318,6 @@ def test_long_attention_lazy_rescale_paths(impl):
         got = torch.cat([o[n_seq * n_patch:].view(n_seq, 1, D).float(), o[:n_seq * n_patch].view(n_seq, n_patch, D).float()], dim=1)
         assert torch.isfinite(got).all()
         assert (got - ref).abs().max().item() < 2e-2 * _r16(), f'max err {(got - ref).abs().max().item()}'
-
-
-def test_puzzle_attention_two_units_per_tile_variant(monkeypatch):
-    """attention_pair.cu packs two (sequence, head) units into one 128-row tcgen05 tile (block-diagonal scores, the
-    class-token query rows on CUDA-core warps). Correct but slower than the one-unit-per-tile kernel, so it only exists in
-    -DVITED_EXPERIMENTAL builds (select with VITED_LIB=tools/bin/experimental/libvited_b200.so)."""
-    if 'experimental' not in os.environ.get('VITED_LIB', ''):
-        pytest.skip('experimental build only (VITED_LIB=tools/bin/experimental/libvited_b200.so)')
-    monkeypatch.setenv('VITED_P64_PAIR', '1')
-    for cfg in [(333, 12, 32, 64, 1), (150, 5, 32, 64, 0), (3, 5, 32, 64, 1), (1, 1, 32, 64, 1)]:
-        test_self_attention(cfg, 0)
-    for cfg in [(401, 7, 12, 32, 64), (7, 3, 5, 32, 64)]:
-        test_cross_attention(cfg, 0)
 
 
 @pytest.mark.parametrize('cfg', [(3, 3, 64, 8), (2, 3, 512, 16), (5, 3, 64, 32)])

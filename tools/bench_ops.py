@@ -60,15 +60,12 @@ def main():
             fl = 2.0 * M * N * K
             by = 2.0 * (M * K + N * K + M * N)
             out.append(dict(op=f'gemm_{name}', M=M, N=N, K=K, ms=ms, tflops=fl / ms / 1e9, tflops_frac=fl / ms / 1e9 / tf,
-                            gbs=by / ms / 1e6, gbs_frac=by / ms / 1e6 / hbm, bn=os.environ.get('VITED_GEMM_BN', 'auto')))
+                            gbs=by / ms / 1e6, gbs_frac=by / ms / 1e6 / hbm))
             ms = timeit(lambda: torch.matmul(A, W.t(), out=C), flush=flush)
             out.append(dict(op=f'cublas_{name}', M=M, N=N, K=K, ms=ms, tflops=2.0 * M * N * K / ms / 1e9))
     if want('fused'):
-        # the two full-row kernels; the 16-epilogue-warp form only exists in -DVITED_EXPERIMENTAL builds (VITED_EPI_WARPS is
-        # read at every launch)
-        epis = ('8', '16') if 'experimental' in os.environ.get('VITED_LIB', '') else ('8',)
-        for epi, name, K in [(e, n, k) for e in epis for n, k in (('proj', 384), ('fc2', 1536))]:
-            os.environ['VITED_EPI_WARPS'] = epi
+        # the two full-row kernels
+        for name, K in (('proj', 384), ('fc2', 1536)):
             A = torch.randn(M, K, device='cuda').to(L.act_dtype())
             W = (torch.randn(384, K, device='cuda') / math.sqrt(K)).to(L.act_dtype())
             b = torch.randn(384, device='cuda')
@@ -79,7 +76,7 @@ def main():
                                                                       lb.data_ptr(), hh.data_ptr(), M, 384, K, 1e-6, st), 'gemm_ln'), flush=flush)
             fl = 2.0 * M * 384 * K
             by = M * K * 2 + 384 * K * 2 + M * 384 * (4 + 4 + 2)
-            out.append(dict(op=f'gemm_ln_{name}' + ('_epi16' if epi == '16' else ''), M=M, N=384, K=K, ms=ms, tflops=fl / ms / 1e9,
+            out.append(dict(op=f'gemm_ln_{name}', M=M, N=384, K=K, ms=ms, tflops=fl / ms / 1e9,
                             gbs=by / ms / 1e6, gbs_frac=by / ms / 1e6 / hbm))
             del A, W, xx, hh
         # fused MLP sub-block + residual + LayerNorm (fc1 -> GELU -> fc2, hidden activations never written)
@@ -90,16 +87,13 @@ def main():
         xx = torch.randn(M, 384, device='cuda')
         lw = torch.ones(384, device='cuda'); lb = torch.zeros(384, device='cuda')
         hh = torch.empty(M, 384, dtype=L.act_dtype(), device='cuda')
-        for epi in epis:
-            os.environ['VITED_EPI_WARPS'] = epi
-            ms = timeit(lambda: L.check(L.lib.vited_op_mlp_resid_ln(hin.data_ptr(), W1.data_ptr(), b1.data_ptr(), W2.data_ptr(), b2.data_ptr(),
-                                                                     xx.data_ptr(), lw.data_ptr(), lb.data_ptr(), hh.data_ptr(), M, 384, 1536,
-                                                                     1e-6, st), 'mlp_ln'), flush=flush)
-            fl = 4.0 * M * 384 * 1536
-            by = M * 384 * (2 + 4 + 4 + 2) + 4 * 384 * 1536
-            out.append(dict(op='mlp_ln' + ('_epi16' if epi == '16' else ''), M=M, D=384, hidden=1536, ms=ms, tflops=fl / ms / 1e9,
-                            tflops_frac=fl / ms / 1e9 / tf, gbs=by / ms / 1e6, gbs_frac=by / ms / 1e6 / hbm))
-        os.environ.pop('VITED_EPI_WARPS', None)
+        ms = timeit(lambda: L.check(L.lib.vited_op_mlp_resid_ln(hin.data_ptr(), W1.data_ptr(), b1.data_ptr(), W2.data_ptr(), b2.data_ptr(),
+                                                                 xx.data_ptr(), lw.data_ptr(), lb.data_ptr(), hh.data_ptr(), M, 384, 1536,
+                                                                 1e-6, st), 'mlp_ln'), flush=flush)
+        fl = 4.0 * M * 384 * 1536
+        by = M * 384 * (2 + 4 + 4 + 2) + 4 * 384 * 1536
+        out.append(dict(op='mlp_ln', M=M, D=384, hidden=1536, ms=ms, tflops=fl / ms / 1e9,
+                        tflops_frac=fl / ms / 1e9 / tf, gbs=by / ms / 1e6, gbs_frac=by / ms / 1e6 / hbm))
         del hin, xx, hh
         # the decoder's cross projection + residual + norm2 + MLP sub-block in one launch, against the gemm_ln + mlp_ln
         # pair it replaces, at the engine's chunk shape (524,288 rows)
@@ -140,16 +134,12 @@ def main():
         by = M * D * (4 + 2 + 4 + 2)
         out.append(dict(op='resid_ln', rows=M, ms=ms, gbs=by / ms / 1e6, gbs_frac=by / ms / 1e6 / hbm))
     if want('attn'):
-        # attention (puzzle): self and cross. impl0 = tcgen05, impl2 = mma.sync; impl0_pair = two units per tile
-        # (attention_pair.cu, experimental builds only, VITED_P64_PAIR=1 is read at every launch)
+        # attention (puzzle): self and cross. impl0 = tcgen05, impl2 = mma.sync
         P, H, hd, Np = 4032, 12, 32, 64
         qkv = torch.randn(M, 3 * D, device='cuda').to(L.act_dtype())
         o = torch.empty(M, D, dtype=L.act_dtype(), device='cuda')
-        variants = ((0, '0', 'impl0'), (2, '0', 'impl2'))
-        if 'experimental' in os.environ.get('VITED_LIB', ''):
-            variants += ((0, '1', 'impl0_pair'),)
-        for impl, pair, tag in variants:
-            os.environ['VITED_P64_PAIR'] = pair
+        variants = ((0, 'impl0'), (2, 'impl2'))
+        for impl, tag in variants:
             ms = timeit(lambda: L.check(L.lib.vited_op_attention(qkv.data_ptr(), 3 * D, qkv.data_ptr() + 2 * D, 3 * D, qkv.data_ptr() + 4 * D,
                                                                   3 * D, o.data_ptr(), D, P, H, hd, Np, 1, Np, 1, P, None, hd ** -0.5, impl, st),
                                         'attn'), flush=flush)
@@ -159,12 +149,10 @@ def main():
         kv = torch.randn(540 * Np, 2 * D, device='cuda').to(L.act_dtype())
         q = torch.randn(M, D, device='cuda').to(L.act_dtype())
         idx = (torch.arange(P, device='cuda') // 539).int()
-        for impl, pair, tag in variants:
-            os.environ['VITED_P64_PAIR'] = pair
+        for impl, tag in variants:
             ms = timeit(lambda: L.check(L.lib.vited_op_attention(q.data_ptr(), D, kv.data_ptr(), 2 * D, kv.data_ptr() + 2 * D, 2 * D, o.data_ptr(), D,
                                                                   P, H, hd, Np, 1, Np, 0, 540, idx.data_ptr(), hd ** -0.5, impl, st), 'attn'), flush=flush)
             out.append(dict(op=f'attn_cross_{tag}', ms=ms, tflops=4.0 * P * H * 65 * 64 * hd / ms / 1e9, gbs=M * D * 2 * 2 / ms / 1e6))
-        os.environ.pop('VITED_P64_PAIR', None)
     for r in out:
         r['peaks'] = src
         print(json.dumps(r))

@@ -3,12 +3,9 @@
 #   bf16    -DVITED_ACT_BF16=1                      bf16 operands instead of fp16 (tools/gpu_fp16.sh, tests/analysis/*)
 #   jitter  -DVITED_JITTER                          random 0..4 us sleeps in front of mbarrier waits (timing fuzzer)
 #   trace   -DVITED_LN_TRACE -DVITED_ATTN_TRACE     clock64 trace points (tools/trace_*.py)
-#   experimental  -DVITED_EXPERIMENTAL              the measured-negative GEMM variants (4-CTA-cluster multicast kernel,
-#                                                   resident-weights kernel) that the product library leaves out
 # Select one with VITED_LIB=$PWD/tools/bin/<variant>/libvited_b200.so
 set -euo pipefail
 cd "$(dirname "$0")/.."
 VITED_OUT_DIR=$PWD/tools/bin/bf16 VITED_EXTRA_FLAGS="-DVITED_ACT_BF16=1" bash vit-ed_b200/csrc/build.sh
 VITED_OUT_DIR=$PWD/tools/bin/jitter VITED_EXTRA_FLAGS="-DVITED_JITTER" bash vit-ed_b200/csrc/build.sh
 VITED_OUT_DIR=$PWD/tools/bin/trace VITED_EXTRA_FLAGS="-DVITED_LN_TRACE -DVITED_ATTN_TRACE -DVITED_MLP_TRACE" bash vit-ed_b200/csrc/build.sh
-VITED_OUT_DIR=$PWD/tools/bin/experimental VITED_EXTRA_FLAGS="-DVITED_EXPERIMENTAL" bash vit-ed_b200/csrc/build.sh

@@ -8,7 +8,6 @@
 //
 // Token rows live in the "split" layout: n_seq*n_patch patch rows, then n_seq cls rows.
 #include "kernels.h"
-#include <cstdlib>
 
 namespace vited {
 
@@ -487,24 +486,13 @@ int attention_cls(const AttnArgs& a, cudaStream_t stream) {
   VITED_CHECK(a.head_dim == 32 || a.head_dim == 64, "attention_cls: head_dim %d not supported (32 or 64)", a.head_dim);
   VITED_CHECK(a.q_has_cls, "attention_cls: the query sequences have no class token");
   if (a.n_seq == 0) return 0;
-  {
-    static int use_warp = -1;   // VITED_ATTN_CLS_WARP=0: back to the tile kernels (A/B measurements)
-    if (use_warp < 0) {
-      const char* e = getenv("VITED_ATTN_CLS_WARP");
-      use_warp = e ? atoi(e) : 1;
-    }
-    if (use_warp && attn_cls_warp_supported(a)) {
-      const int units = a.n_seq * a.n_heads;
-      int blocks = (units + 7) / 8;
-      if (blocks > 148 * 8) blocks = 148 * 8;
-      attn_cls_warp_kernel<<<blocks, 256, 0, stream>>>(a);
-      VITED_CUDA_OK(cudaGetLastError());
-      return 0;
-    }
-  }
-  {
-    const char* e = getenv("VITED_ATTN_TC");
-    if ((!e || atoi(e) != 0) && attention_tc_cls_supported(a)) return attention_tc_cls(a, stream);
+  if (attn_cls_warp_supported(a)) {
+    const int units = a.n_seq * a.n_heads;
+    int blocks = (units + 7) / 8;
+    if (blocks > 148 * 8) blocks = 148 * 8;
+    attn_cls_warp_kernel<<<blocks, 256, 0, stream>>>(a);
+    VITED_CUDA_OK(cudaGetLastError());
+    return 0;
   }
   return attention_launch(a, 1, stream);
 }
@@ -521,12 +509,7 @@ int attention(const AttnArgs& a, int impl, cudaStream_t stream) {
     if (a.head_dim == 32) attn_simt_kernel<32><<<grid, 128, 0, stream>>>(a);
     else attn_simt_kernel<64><<<grid, 128, 0, stream>>>(a);
   } else {
-    static int use_tc = -1;   // VITED_ATTN_TC=0 keeps everything on the mma.sync kernel (A/B measurements)
-    if (use_tc < 0) {
-      const char* e = getenv("VITED_ATTN_TC");
-      use_tc = e ? atoi(e) : 1;
-    }
-    if (impl == IMPL_FAST && use_tc && attention_tc_supported(a)) return attention_tc(a, stream);
+    if (impl == IMPL_FAST && attention_tc_supported(a)) return attention_tc(a, stream);
     return attention_launch(a, 0, stream);
   }
   VITED_CUDA_OK(cudaGetLastError());

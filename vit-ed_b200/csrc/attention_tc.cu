@@ -52,13 +52,8 @@ struct P64Maps {
 };
 
 __global__ void __launch_bounds__(P64::THREADS, 1)
-attn_p64_kernel(AttnArgs a, const __grid_constant__ P64Maps maps, int n_units, int mode) {
+attn_p64_kernel(AttnArgs a, const __grid_constant__ P64Maps maps, int n_units) {
   using C = P64;
-  const int cls_only = mode & 1;
-  // mode bit 1 -- MEASUREMENT ONLY (VITED_P64_KV_ONCE=1, results are wrong): K/V tiles are fetched only the first time
-  // a ring slot is used, every later unit reuses whatever the slot holds. The launch then moves Q and O only: the
-  // upper bound of what a design that keeps a context piece's K/V resident in shared memory could gain.
-  const bool kv_once = (mode & 2) != 0;
   extern __shared__ uint8_t attn_tc_smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(attn_tc_smem_raw) + 1023) & ~uintptr_t(1023));
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + C::NS * C::STAGE);
@@ -100,8 +95,6 @@ attn_p64_kernel(AttnArgs a, const __grid_constant__ P64Maps maps, int n_units, i
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_holder;
-  pdl_launch_dependents();
-  pdl_wait();           // the prologue above overlapped the previous kernel's tail; global memory only from here on
 
   if (quarter == 3) {
     if (group == 0) {
@@ -118,18 +111,13 @@ attn_p64_kernel(AttnArgs a, const __grid_constant__ P64Maps maps, int n_units, i
         const int col = h * C::HD;
         mbar_wait(&empty[s], ph ^ 1, 50);
         uint8_t* st = smem + s * C::STAGE;
-        // cls_only (last decoder layer, only the class-token row reaches the head): the 64 patch queries are not loaded
-        const bool load_kv = !kv_once || i < C::NS;
-        const uint32_t bytes = ((cls_only ? 0 : 1) + (load_kv ? 2 : 0)) * 64 * C::RB + (a.q_has_cls ? C::RB : 0) +
-                               (a.k_has_cls && load_kv ? 2 * C::RB : 0);
+        const uint32_t bytes = 3 * 64 * C::RB + (a.q_has_cls ? C::RB : 0) + (a.k_has_cls ? 2 * C::RB : 0);
         mbar_arrive_expect_tx(&full[s], bytes);
-        if (!cls_only) tma_load_2d(&maps.q_tile, &full[s], st, col, b * 64);
+        tma_load_2d(&maps.q_tile, &full[s], st, col, b * 64);
         if (a.q_has_cls) tma_load_2d(&maps.q_row, &full[s], st + 64 * C::RB, col, a.n_seq * 64 + b);
-        if (load_kv) {
-          tma_load_2d(&maps.k_tile, &full[s], st + C::TB, col, kvb * 64);
-          tma_load_2d(&maps.v_tile, &full[s], st + 2 * C::TB, col, kvb * 64);
-        }
-        if (a.k_has_cls && load_kv) {
+        tma_load_2d(&maps.k_tile, &full[s], st + C::TB, col, kvb * 64);
+        tma_load_2d(&maps.v_tile, &full[s], st + 2 * C::TB, col, kvb * 64);
+        if (a.k_has_cls) {
           tma_load_2d(&maps.k_row, &full[s], st + C::TB + 64 * C::RB, col, a.n_kv_seq * 64 + kvb);
           tma_load_2d(&maps.v_row, &full[s], st + 2 * C::TB + 64 * C::RB, col, a.n_kv_seq * 64 + kvb);
         }
@@ -202,8 +190,8 @@ attn_p64_kernel(AttnArgs a, const __grid_constant__ P64Maps maps, int n_units, i
     // The group owns TMEM stage `group`: scores -> probabilities (packed fp16 over S) -> signal the issuer -> read O.
     const float sl2 = a.scale * kLog2e;
     const int row = quarter * 32 + lane;                  // query row of the unit's tile
-    // quarter 2 only carries the class-token query (row 64); in cls_only mode it is the only live row
-    const bool warp_active = quarter < 2 ? !cls_only : a.q_has_cls != 0;
+    // quarter 2 only carries the class-token query (row 64)
+    const bool warp_active = quarter < 2 || a.q_has_cls != 0;
     const uint32_t t_col = tmem_base + group * C::TCOLS;
     const uint32_t t_stage = t_col + (static_cast<uint32_t>(quarter * 32) << 16);
     uint32_t ph = 0;
@@ -233,7 +221,6 @@ attn_p64_kernel(AttnArgs a, const __grid_constant__ P64Maps maps, int n_units, i
         const float mneg = -mxa * sl2;
         float sum[4] = {0.f, 0.f, 0.f, 0.f};
         uint32_t pk[32];
-#if VITED_SOFTMAX_PACKED
         {
           uint64_t sum2[2] = {0ull, 0ull};
           softmax_exp_pairs<16>(v0, sl2, mneg, pk, sum2);
@@ -241,22 +228,6 @@ attn_p64_kernel(AttnArgs a, const __grid_constant__ P64Maps maps, int n_units, i
           f2_unpack(sum2[0], sum[0], sum[1]);
           f2_unpack(sum2[1], sum[2], sum[3]);
         }
-#else
-#pragma unroll
-        for (int j = 0; j < 16; ++j) {
-          const float p0 = ex2_ftz(fmaf(__uint_as_float(v0[2 * j]), sl2, mneg));
-          const float p1 = ex2_ftz(fmaf(__uint_as_float(v0[2 * j + 1]), sl2, mneg));
-          sum[(2 * j) & 3] += p0; sum[(2 * j + 1) & 3] += p1;
-          pk[j] = pack_act(p0, p1);
-        }
-#pragma unroll
-        for (int j = 0; j < 16; ++j) {
-          const float p0 = ex2_ftz(fmaf(__uint_as_float(v1[2 * j]), sl2, mneg));
-          const float p1 = ex2_ftz(fmaf(__uint_as_float(v1[2 * j + 1]), sl2, mneg));
-          sum[(2 * j) & 3] += p0; sum[(2 * j + 1) & 3] += p1;
-          pk[16 + j] = pack_act(p0, p1);
-        }
-#endif
         tmem_st_32x32b_x32(t_stage, pk);
         if (a.k_has_cls) {
           const float pc = ex2_ftz(fmaf(__uint_as_float(vc[0]), sl2, mneg));
@@ -281,7 +252,7 @@ attn_p64_kernel(AttnArgs a, const __grid_constant__ P64Maps maps, int n_units, i
         const float inv = 1.f / l;
         size_t orow;
         bool valid = true;
-        if (row < 64) { orow = (size_t)b * 64 + row; valid = !cls_only; }
+        if (row < 64) orow = (size_t)b * 64 + row;
         else if (row == 64 && a.q_has_cls) orow = (size_t)a.n_seq * 64 + b;
         else { valid = false; orow = 0; }
         if (valid) {
@@ -402,8 +373,6 @@ attn_l64_kernel(AttnArgs a, const __grid_constant__ L64Maps maps, int n_items) {
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_holder;
-  pdl_launch_dependents();
-  pdl_wait();           // the prologue above overlapped the previous kernel's tail; global memory only from here on
   auto is_cls_item = [&](int i) { return (((int)blockIdx.x + i * (int)gridDim.x) % per_bh) == n_qp; };
 
   if (warp == 8) {
@@ -593,7 +562,6 @@ attn_l64_kernel(AttnArgs a, const __grid_constant__ L64Maps maps, int n_items) {
           }
           const float mneg = -m;
           float sum[4] = {0.f, 0.f, 0.f, 0.f};
-#if VITED_SOFTMAX_PACKED
           {
             uint64_t sum2[2] = {0ull, 0ull};
             {
@@ -609,30 +577,6 @@ attn_l64_kernel(AttnArgs a, const __grid_constant__ L64Maps maps, int n_items) {
             f2_unpack(sum2[0], sum[0], sum[1]);
             f2_unpack(sum2[1], sum[2], sum[3]);
           }
-#else
-          {
-            uint32_t pk[16];
-#pragma unroll
-            for (int e = 0; e < 16; ++e) {
-              const float p0 = ex2_ftz(fmaf(__uint_as_float(v0[2 * e]), sl2, mneg));
-              const float p1 = ex2_ftz(fmaf(__uint_as_float(v0[2 * e + 1]), sl2, mneg));
-              sum[(2 * e) & 3] += p0; sum[(2 * e + 1) & 3] += p1;
-              pk[e] = pack_act(p0, p1);
-            }
-            tmem_st_32x32b_x16(t_s, pk);
-          }
-          {
-            uint32_t pk[16];
-#pragma unroll
-            for (int e = 0; e < 16; ++e) {
-              const float p0 = ex2_ftz(fmaf(__uint_as_float(v1[2 * e]), sl2, mneg));
-              const float p1 = ex2_ftz(fmaf(__uint_as_float(v1[2 * e + 1]), sl2, mneg));
-              sum[(2 * e) & 3] += p0; sum[(2 * e + 1) & 3] += p1;
-              pk[e] = pack_act(p0, p1);
-            }
-            tmem_st_32x32b_x16(t_s + 16, pk);
-          }
-#endif
           l += (sum[0] + sum[1]) + (sum[2] + sum[3]);
         } else {
           // class-token key half tile: column 0 is the only real key
@@ -723,33 +667,12 @@ static int attention_tc_l64(const AttnArgs& a, cudaStream_t stream) {
   if (make_tmap_act_2d(&maps.v_tile, a.v, cols, k_rows, (uint64_t)a.v_ld * 2, 64, 128, 128)) return 1;
   if (make_tmap_act_2d(&maps.v_row, a.v, cols, k_rows, (uint64_t)a.v_ld * 2, 64, 1, 128)) return 1;
   const unsigned grid = (unsigned)(items < (size_t)sms ? items : (size_t)sms);
-  VITED_CUDA_OK(launch_pdl(attn_l64_kernel, dim3(grid), dim3(L64::THREADS), L64::BYTES, stream, a, maps, (int)items));
+  attn_l64_kernel<<<grid, L64::THREADS, L64::BYTES, stream>>>(a, maps, (int)items);
   VITED_CUDA_OK(cudaGetLastError());
   return 0;
 }
 
-static int attention_tc_p64(const AttnArgs& a, int cls_only, cudaStream_t stream);
-
-int attention_tc(const AttnArgs& a, cudaStream_t stream) {
-  VITED_CHECK(attention_tc_supported(a), "attention_tc: unsupported shape");
-  if (l64_shape(a)) return attention_tc_l64(a, stream);
-#ifdef VITED_EXPERIMENTAL
-  // two units per 128-row tile (attention_pair.cu): correct, 30 % slower (profiles/README.md) -- experimental builds
-  // only, selected with VITED_P64_PAIR=1 (read at every launch: A/B runs)
-  const char* pr = getenv("VITED_P64_PAIR");
-  if (pr != nullptr && atoi(pr) != 0 && attention_pair_supported(a)) return attention_pair(a, stream);
-#endif
-  return attention_tc_p64(a, 0, stream);
-}
-
-// class-token query only (last decoder layer), puzzle shape
-bool attention_tc_cls_supported(const AttnArgs& a) { return a.n_heads >= 1 && p64_shape(a) && a.q_has_cls; }
-int attention_tc_cls(const AttnArgs& a, cudaStream_t stream) {
-  VITED_CHECK(attention_tc_cls_supported(a), "attention_tc_cls: unsupported shape");
-  return attention_tc_p64(a, 1, stream);
-}
-
-static int attention_tc_p64(const AttnArgs& a, int cls_only, cudaStream_t stream) {
+static int attention_tc_p64(const AttnArgs& a, cudaStream_t stream) {
   const size_t units = (size_t)a.n_seq * a.n_heads;
   VITED_CHECK(units < ((size_t)1 << 31), "attention_tc: too many work units");
   static PerDeviceOnce once;
@@ -767,11 +690,15 @@ static int attention_tc_p64(const AttnArgs& a, int cls_only, cudaStream_t stream
   if (make_tmap_act_2d(&maps.v_tile, a.v, cols, k_rows, (uint64_t)a.v_ld * 2, 32, 64, 64)) return 1;
   if (make_tmap_act_2d(&maps.v_row, a.v, cols, k_rows, (uint64_t)a.v_ld * 2, 32, 1, 64)) return 1;
   const unsigned grid = (unsigned)(units < (size_t)sms ? units : (size_t)sms);
-  static const int kv_once = [] { const char* v = getenv("VITED_P64_KV_ONCE"); return v ? atoi(v) : 0; }();
-  VITED_CUDA_OK(launch_pdl(attn_p64_kernel, dim3(grid), dim3(P64::THREADS), P64::BYTES, stream, a, maps, (int)units,
-                           cls_only | (kv_once ? 2 : 0)));
+  attn_p64_kernel<<<grid, P64::THREADS, P64::BYTES, stream>>>(a, maps, (int)units);
   VITED_CUDA_OK(cudaGetLastError());
   return 0;
+}
+
+int attention_tc(const AttnArgs& a, cudaStream_t stream) {
+  VITED_CHECK(attention_tc_supported(a), "attention_tc: unsupported shape");
+  if (l64_shape(a)) return attention_tc_l64(a, stream);
+  return attention_tc_p64(a, stream);
 }
 
 }  // namespace vited

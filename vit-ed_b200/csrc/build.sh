@@ -9,5 +9,5 @@ NVCC="${NVCC:-/usr/local/cuda/bin/nvcc}"
   -Xcompiler -fPIC -Xcompiler -fvisibility=hidden -shared -cudart static \
   ${VITED_PTXAS_V:+-Xptxas -v} ${VITED_EXTRA_FLAGS:-} \
   -o "$OUT/libvited_b200.so" \
-  "$HERE/engine.cu" "$HERE/gemm_tc.cu" "$HERE/gemm_ln.cu" "$HERE/mlp_ln.cu" "$HERE/attention.cu" "$HERE/attention_tc.cu" "$HERE/attention_pair.cu" "$HERE/rowops.cu" "$HERE/pair_lists.cu" "$HERE/train_ops.cu" "$HERE/train_attn.cu" "$HERE/train_optim.cu" "$HERE/solver_tables.cu" "$HERE/piece_prep.cu" "$HERE/retrieval_metrics.cu"
+  "$HERE/engine.cu" "$HERE/gemm_tc.cu" "$HERE/gemm_ln.cu" "$HERE/mlp_ln.cu" "$HERE/attention.cu" "$HERE/attention_tc.cu" "$HERE/rowops.cu" "$HERE/pair_lists.cu" "$HERE/train_ops.cu" "$HERE/train_attn.cu" "$HERE/train_optim.cu" "$HERE/solver_tables.cu" "$HERE/piece_prep.cu" "$HERE/retrieval_metrics.cu"
 echo "built $OUT/libvited_b200.so"

@@ -2,7 +2,6 @@
 // PTX wrappers: mbarrier, TMA (cp.async.bulk.tensor), tcgen05 (alloc / mma / commit / ld), ldmatrix, mma.sync.
 #pragma once
 #include <cuda_runtime.h>
-#include <utility>
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include <cuda.h>
@@ -30,7 +29,6 @@ typedef __half act_t;
 // host side error plumbing (no exceptions cross the C-ABI; see include/vited_b200.h)
 // ---------------------------------------------------------------------------------------------
 void set_error(const char* fmt, ...);
-bool pdl_enabled();   // VITED_PDL=1 (default off: measured neutral, see profiles/README.md); engine.cu
 const char* get_error();
 
 #define VITED_CUDA_OK(expr)                                                                     \
@@ -65,30 +63,8 @@ struct PerDeviceOnce {
   }
 };
 int device_sm_count();   // SM count of the CURRENT device (cached per device); gemm_tc.cu
-// Epilogue warps per CTA of the two full-row kernels (gemm_ln.cu, mlp_ln.cu): 8 (two column groups) or, in
-// -DVITED_EXPERIMENTAL builds, 16 (four; measured neutral). VITED_EPI_WARPS=8|16 is read at every launch so that tests
-// and A/B runs can switch in-process.
-int epilogue_warps();    // gemm_tc.cu
 
 #ifdef __CUDACC__
-// Launch `kernel` so that it may overlap the tail of the previous kernel in `stream` (see pdl_wait below). Only for
-// kernels that call pdl_wait() before their first global-memory access.
-template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
-                              Args&&... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute at;
-  at.id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at.val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = &at;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
-}
-
 // ---------------------------------------------------------------------------------------------
 // small device helpers
 // ---------------------------------------------------------------------------------------------
@@ -146,15 +122,6 @@ __device__ __forceinline__ act_t f2act(float v) {
   return __float2half_rn(fminf(fmaxf(v, -65504.f), 65504.f));
 #endif
 }
-
-// Programmatic dependent launch (PDL). A kernel launched through launch_pdl() may become resident while the previous
-// kernel of the stream is still draining: its prologue (barrier init, TMEM allocation, descriptor prefetch) then
-// overlaps the predecessor's tail and the launch latency. pdl_wait() blocks until every earlier kernel has completed
-// and its writes are visible; NOTHING may touch global memory before it. pdl_launch_dependents() lets the NEXT
-// kernel do the same with respect to this one (it still cannot pass its own pdl_wait() before this grid is done).
-// Both are no-ops in a kernel launched the ordinary way.
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
 // one lane of a converged warp (always the same one: lane 0 for a full mask). Issuing tcgen05.mma / commit under this
 // predicate from WARP-UNIFORM code lets the compiler keep descriptors in uniform registers; issuing from a divergent
@@ -284,14 +251,11 @@ __device__ __forceinline__ uint64_t gelu2x_fast2(uint64_t x2) {
   return f2_add(x2, f2_fma(f2_pack(-fabsf(x0), -fabsf(x1)), e2, a2));
 }
 // The exponentials of NP score pairs of one softmax row: pk[j] = fp16x2(2^(v[2j] sl2 + mneg), 2^(v[2j+1] sl2 + mneg)),
-// probabilities accumulated into two packed sums (four chains). -DVITED_SOFTMAX_PACKED=0 keeps the scalar form
-// (FFMA / FADD per element); -DVITED_EXP_POLY=n computes n of every 8 pairs with ex2_poly2 on the FMA pipe.
-#ifndef VITED_SOFTMAX_PACKED
-#define VITED_SOFTMAX_PACKED 1
-#endif
-#ifndef VITED_EXP_POLY
-#define VITED_EXP_POLY 2   // measured on B200 (profiles/r02b_softmax_variants.jsonl): long-sequence attention 0.742 ms scalar,
-#endif                     // 0.712 packed, 0.679 / 0.674 / 0.663 with 1 / 2 / 3 of 8; in the step 2 of 8 is best (power cap)
+// probabilities accumulated into two packed sums (four chains). kExpPoly of every 8 pairs are computed with ex2_poly2
+// on the FMA pipe, the rest with MUFU.EX2.
+// Measured on B200 (profiles/r02b_softmax_variants.jsonl): long-sequence attention 0.742 ms scalar, 0.712 packed, 0.679 /
+// 0.674 / 0.663 with 1 / 2 / 3 of 8; in the step 2 of 8 is best (power cap).
+constexpr int kExpPoly = 2;
 template <int NP>
 __device__ __forceinline__ void softmax_exp_pairs(const uint32_t* v, float sl2, float mneg, uint32_t* pk, uint64_t (&sum2)[2]) {
   const uint64_t s2 = f2_pack(sl2, sl2), m2 = f2_pack(mneg, mneg);
@@ -300,7 +264,7 @@ __device__ __forceinline__ void softmax_exp_pairs(const uint32_t* v, float sl2, 
     const uint64_t x = f2_fma(f2_pack(__uint_as_float(v[2 * j]), __uint_as_float(v[2 * j + 1])), s2, m2);
     uint64_t p;
     float p0, p1;
-    if ((j & 7) < VITED_EXP_POLY) {
+    if ((j & 7) < kExpPoly) {
       p = ex2_poly2(x);
       f2_unpack(p, p0, p1);
     } else {
@@ -565,17 +529,6 @@ __device__ __forceinline__ void tma_load_2d_2cta(const CUtensorMap* tm, uint64_t
       ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(tm)), "r"(smem_u32(bar) & kPeerBitMask), "r"(c0), "r"(c1)
       : "memory");
 }
-// Same, multicast: the box lands at this shared-memory offset in every CTA of `cta_mask` (cluster ranks) and each
-// destination counts the bytes on the barrier at this offset in ITS pair's leader CTA (the peer bit is relative to the
-// destination). Used to share one weight stream between the two CTA pairs of a 4-CTA cluster.
-__device__ __forceinline__ void tma_load_2d_2cta_mc(const CUtensorMap* tm, uint64_t* bar, void* smem_dst, int c0, int c1,
-                                                    uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;"
-      ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(tm)), "r"(smem_u32(bar) & kPeerBitMask), "r"(c0), "r"(c1),
-      "h"(cta_mask)
-      : "memory");
-}
 // D[tmem, both CTAs] (+)= A * B with M = 256 split over the pair; issued by ONE thread of the leader CTA
 __device__ __forceinline__ void umma_f16_2cta(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
                                                uint32_t accumulate) {
@@ -601,13 +554,6 @@ __device__ __forceinline__ void umma_f16_ts_2cta(uint32_t tmem_d, uint32_t tmem_
       : "memory");
 }
 // arrive on the mbarrier at this shared-memory offset in BOTH CTAs once the issued cta_group::2 MMAs have completed
-__device__ __forceinline__ void umma_commit_2cta_mask(uint64_t* bar, uint16_t mask) {   // explicit cluster-rank mask
-  asm volatile(
-      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-          smem_u32(bar)),
-      "h"(mask)
-      : "memory");
-}
 __device__ __forceinline__ void umma_commit_2cta(uint64_t* bar) {
   const uint16_t mask = 3;
   asm volatile(

@@ -613,13 +613,6 @@ static int build_pair_list(vited_engine* e, int mode, int r0, int r1, int ca, in
 // =====================================================================================================================
 // C-ABI
 // =====================================================================================================================
-namespace vited {
-bool pdl_enabled() {
-  static const int on = [] { const char* v = getenv("VITED_PDL"); return v == nullptr ? 0 : atoi(v); }();
-  return on != 0;
-}
-}  // namespace vited
-
 extern "C" {
 
 const char* vited_last_error(void) { return get_error(); }
@@ -639,10 +632,6 @@ int vited_create(const vited_config* cfg, int device, vited_engine** out) {
   vited_engine* e = new vited_engine();
   e->cfg = *cfg;
   e->device = device;
-  const char* cr = getenv("VITED_CHUNK_ROWS");
-  if (cr && atoll(cr) > 0) e->chunk_rows = atoll(cr);
-  const char* fm = getenv("VITED_FUSE_MLP");   // A/B runs of bench.py; vited_set_option(VITED_OPT_FUSE_MLP) is the API
-  if (fm) e->fuse_mlp = atoi(fm) ? 1 : 0;
   if (build(e) != 0) {
     vited_destroy(e);
     return 1;

@@ -8,10 +8,9 @@
 //
 // Structure = gemm_tc_pair_kernel (cta_group::2, TMA ring, one MMA thread) with N = 384 issued as two N = 192 MMAs per
 // k-step and a full-row epilogue: 4 * CG epilogue warps per CTA, warp (q, c) owns TMEM lane quarter q (32 rows) and
-// column group c of CG (CG = 2: 192-column halves, 8 warps; CG = 4: 96-column quarters, 16 warps -- the same bytes in
-// half-width boxes, twice as many independent TMEM -> math -> shared memory -> TMA chains in flight per SM); one thread =
-// one row part. Row statistics use the shifted one-pass form (pivot = first element of the row part) and Chan's
-// combination across the CG parts.
+// column group c of CG; one thread = one row part. Row statistics use the shifted one-pass form (pivot = first element
+// of the row part) and Chan's combination across the CG parts. The library instantiates CG = 2 (192-column halves,
+// 8 warps); CG = 4 (96-column quarters, 16 warps) was measured neutral (profiles/README.md) and is not built.
 #include "kernels.h"
 
 namespace vited {
@@ -118,8 +117,6 @@ gemm_ln_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
   cluster_sync_all();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_holder;
-  pdl_launch_dependents();
-  pdl_wait();           // the prologue above overlapped the previous kernel's tail; global memory only from here on
 
   if (warp == 0) {
     // ===================== TMA producer (both CTAs): own 128 activation rows + 2 x 96 weight rows per k-block ========
@@ -360,15 +357,17 @@ gemm_ln_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
 
 bool gemm_resid_ln_supported(int M, int N, int K) { return N == LN_N && K % 8 == 0 && K >= 8 && M >= 1; }
 
-template <int CG>
-static int gemm_resid_ln_launch(const act_t* A, const act_t* W, const float* bias, float* x, const float* ln_w,
-                                const float* ln_b, act_t* h, int M, int N, int K, float eps, cudaStream_t stream) {
-  using Cfg = LnCfg<CG>;
+int gemm_resid_ln(const act_t* A, const act_t* W, const float* bias, float* x, const float* ln_w, const float* ln_b,
+                  act_t* h, int M, int N, int K, float eps, cudaStream_t stream) {
+  VITED_CHECK(gemm_resid_ln_supported(M, N, K), "gemm_resid_ln: unsupported shape M=%d N=%d K=%d (N must be 384)", M, N, K);
+  VITED_CHECK(((reinterpret_cast<uintptr_t>(A) | reinterpret_cast<uintptr_t>(W) | reinterpret_cast<uintptr_t>(x) |
+                reinterpret_cast<uintptr_t>(h)) & 15) == 0, "gemm_resid_ln: operands must be 16-byte aligned");
+  using Cfg = LnCfg<2>;
   const int sms = gemm_num_sms();
   VITED_CHECK(sms >= 2, "gemm_resid_ln: no device");
   static PerDeviceOnce once;
   if (once.first())
-    VITED_CUDA_OK(cudaFuncSetAttribute(gemm_ln_pair_kernel<CG>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    VITED_CUDA_OK(cudaFuncSetAttribute(gemm_ln_pair_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)Cfg::SMEM_BYTES));
   CUtensorMap tA, tB, tX, tH;
   if (make_tmap_act_2d(&tA, A, (uint64_t)K, (uint64_t)M, (uint64_t)K * 2, 64, BM, 128)) return 1;
@@ -378,20 +377,10 @@ static int gemm_resid_ln_launch(const act_t* A, const act_t* W, const float* bia
   const int tiles = (M + 2 * BM - 1) / (2 * BM);
   int pairs = sms / 2;
   if (pairs > tiles) pairs = tiles;
-  VITED_CUDA_OK(launch_pdl(gemm_ln_pair_kernel<CG>, dim3(2 * pairs), dim3(Cfg::kThreads), Cfg::SMEM_BYTES, stream, tA, tB, tX,
-                           tH, bias, ln_w, ln_b, M, K, eps));
+  gemm_ln_pair_kernel<2><<<2 * pairs, Cfg::kThreads, Cfg::SMEM_BYTES, stream>>>(tA, tB, tX, tH, bias, ln_w, ln_b, M, K,
+                                                                                  eps);
+  VITED_CUDA_OK(cudaGetLastError());
   return 0;
-}
-
-int gemm_resid_ln(const act_t* A, const act_t* W, const float* bias, float* x, const float* ln_w, const float* ln_b,
-                  act_t* h, int M, int N, int K, float eps, cudaStream_t stream) {
-  VITED_CHECK(gemm_resid_ln_supported(M, N, K), "gemm_resid_ln: unsupported shape M=%d N=%d K=%d (N must be 384)", M, N, K);
-  VITED_CHECK(((reinterpret_cast<uintptr_t>(A) | reinterpret_cast<uintptr_t>(W) | reinterpret_cast<uintptr_t>(x) |
-                reinterpret_cast<uintptr_t>(h)) & 15) == 0, "gemm_resid_ln: operands must be 16-byte aligned");
-#ifdef VITED_EXPERIMENTAL   // measured neutral (profiles/README.md): not in the product library
-  if (epilogue_warps() == 16) return gemm_resid_ln_launch<4>(A, W, bias, x, ln_w, ln_b, h, M, N, K, eps, stream);
-#endif
-  return gemm_resid_ln_launch<2>(A, W, bias, x, ln_w, ln_b, h, M, N, K, eps, stream);
 }
 
 }  // namespace vited

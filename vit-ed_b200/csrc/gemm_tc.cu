@@ -11,7 +11,6 @@
 //                                             and the 64-column slab sl, stages its 32x64 fp16 sub-tile in a private
 //                                             4 KB swizzled buffer and TMA-stores it itself (no CTA-wide barrier).
 #include "kernels.h"
-#include <cstdlib>
 #include <cudaTypedefs.h>
 #include <mutex>
 
@@ -46,12 +45,6 @@ static void init_driver_once() {
 int gemm_num_sms() {
   std::call_once(g_once, init_driver_once);
   return device_sm_count();
-}
-
-int epilogue_warps() {
-  const char* v = getenv("VITED_EPI_WARPS");
-  if (v != nullptr && v[0] != 0) return atoi(v) == 16 ? 16 : 8;
-  return 8;
 }
 
 // Every launch needs 3-6 tensor maps and a step makes ~7,500 launches over a handful of buffers and shapes that repeat
@@ -125,23 +118,18 @@ int make_tmap_f32_2d(CUtensorMap* tm, const void* ptr, uint64_t cols, uint64_t r
 constexpr int BM = 128;
 constexpr int BK = 64;
 
-// KB_RES == 0: both operands stream through the ring (any K).
-// KB_RES  > 0: "resident weights": the CTA keeps its [BN x K] weight panel (K <= 64*KB_RES) in shared memory for its
-//              whole life and only the activation tiles stream; this halves the L2->SM traffic of the K=384 layers,
-//              which is what bounds them (a 128xBN tile with K=384 needs only 24 MMAs per 240 KB of operands).
-template <int BN, int KB_RES>
+template <int BN>
 struct GemmCfg {
   static constexpr int kEpiWarps = 4 * (BN / 64);
   static constexpr int kThreads = 128 + 32 * kEpiWarps;
   static constexpr uint32_t A_BYTES = BM * BK * 2;
   static constexpr uint32_t B_BYTES = BN * BK * 2;
-  static constexpr uint32_t STAGE_BYTES = KB_RES > 0 ? A_BYTES : A_BYTES + B_BYTES;
-  static constexpr uint32_t PANEL_BYTES = KB_RES * B_BYTES;
+  static constexpr uint32_t STAGE_BYTES = A_BYTES + B_BYTES;
   static constexpr uint32_t C_BYTES = kEpiWarps * 4096;  // one 32-row x 128-byte swizzled box per epilogue warp
-  static constexpr int kStagesMax = (232448 - 1024 - 256 - (int)C_BYTES - (int)PANEL_BYTES) / (int)STAGE_BYTES;
+  static constexpr int kStagesMax = (232448 - 1024 - 256 - (int)C_BYTES) / (int)STAGE_BYTES;
   static constexpr int kStages = kStagesMax > 8 ? 8 : kStagesMax;
   static constexpr uint32_t TMEM_COLS = (2 * BN <= 256) ? 256 : 512;
-  static constexpr uint32_t SMEM_BYTES = 1024 + PANEL_BYTES + kStages * STAGE_BYTES + C_BYTES + 256;
+  static constexpr uint32_t SMEM_BYTES = 1024 + kStages * STAGE_BYTES + C_BYTES + 256;
   static_assert(BN % 64 == 0 && BN <= 256, "BN must be a multiple of 64 up to 256");
   static_assert(kStages >= 3, "not enough shared memory for the pipeline");
 };
@@ -187,27 +175,22 @@ __device__ __forceinline__ void epilogue_tile(const uint32_t (&v0)[32], const ui
   }
 }
 
-template <int BN, int ACT, int KB_RES>
-__global__ void __launch_bounds__(GemmCfg<BN, KB_RES>::kThreads, 1)
+template <int BN, int ACT>
+__global__ void __launch_bounds__(GemmCfg<BN>::kThreads, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-               const __grid_constant__ CUtensorMap tmC, const float* __restrict__ bias, int M, int N, int K,
-               int order) {
-  using Cfg = GemmCfg<BN, KB_RES>;
+               const __grid_constant__ CUtensorMap tmC, const float* __restrict__ bias, int M, int N, int K) {
+  using Cfg = GemmCfg<BN>;
   constexpr int kStages = Cfg::kStages;
   constexpr int kEpiWarps = Cfg::kEpiWarps;
-  constexpr bool kResident = KB_RES > 0;
   extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem_base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* sPanel = smem_base;                      // resident weight panel: KB_RES boxes of [BN x 64] (may be empty)
-  uint8_t* smem = smem_base + Cfg::PANEL_BYTES;     // operand ring
+  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* sC = smem + kStages * Cfg::STAGE_BYTES;
   uint64_t* bars = reinterpret_cast<uint64_t*>(sC + Cfg::C_BYTES);
   uint64_t* full = bars;
   uint64_t* empty = bars + kStages;
   uint64_t* tfull = bars + 2 * kStages;
   uint64_t* tempty = bars + 2 * kStages + 2;
-  uint64_t* pfull = bars + 2 * kStages + 4;
-  uint32_t* tmem_holder = reinterpret_cast<uint32_t*>(bars + 2 * kStages + 5);
+  uint32_t* tmem_holder = reinterpret_cast<uint32_t*>(bars + 2 * kStages + 4);
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -215,25 +198,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   const int m_blks = (M + BM - 1) / BM;
   const int n_blks = (N + BN - 1) / BN;
   const int num_kb = (K + BK - 1) / BK;
-  // Tile schedule. Streaming: tile = blockIdx.x + i*gridDim.x, n fastest. Resident: the CTA owns ONE n-block
-  // (blockIdx.x % n_blks) and walks the m-blocks (blockIdx.x / n_blks) + i*(gridDim.x / n_blks); the host launches a
-  // grid that is a multiple of n_blks.
-  //   order 1 (streaming, large M): the CTA owns an m-block and runs its n-blocks back to back, so the activation
-  //   tile comes from HBM once and from L2 (short latency) for the remaining n-blocks, and CTAs do not miss in step.
-  const int my_n = kResident ? (int)(blockIdx.x % n_blks) : 0;
-  const int tile0 = kResident ? (int)(blockIdx.x / n_blks) : (int)blockIdx.x;
-  const int tile_step = kResident ? (int)(gridDim.x / n_blks) : (int)gridDim.x;
+  // Tile schedule: tile = blockIdx.x + i*gridDim.x, n fastest.
   auto coords = [&](int it, int& m_blk, int& n_blk) -> bool {
-    if (kResident) {
-      m_blk = tile0 + it * tile_step;
-      n_blk = my_n;
-      return m_blk < m_blks;
-    }
-    if (order == 1) {
-      m_blk = (int)blockIdx.x + (it / n_blks) * (int)gridDim.x;
-      n_blk = it % n_blks;
-      return m_blk < m_blks;
-    }
     const int tile = (int)blockIdx.x + it * (int)gridDim.x;
     m_blk = tile / n_blks;
     n_blk = tile % n_blks;
@@ -253,7 +219,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       mbar_init(&tfull[s], 1);
       mbar_init(&tempty[s], kEpiWarps);
     }
-    mbar_init(pfull, 1);
     fence_mbar_init();
   } else if (warp == 2) {
     tmem_alloc(tmem_holder, Cfg::TMEM_COLS);
@@ -268,10 +233,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     // ===================== TMA producer =====================
     if (lane == 0) {
       uint32_t stage = 0, phase = 0;
-      if (kResident && tile0 < m_blks) {
-        mbar_arrive_expect_tx(pfull, (uint32_t)num_kb * Cfg::B_BYTES);
-        for (int kb = 0; kb < num_kb; ++kb) tma_load_2d(&tmB, pfull, sPanel + kb * Cfg::B_BYTES, kb * BK, my_n * BN);
-      }
       int m_blk, n_blk;
       for (int it = 0; coords(it, m_blk, n_blk); ++it) {
         for (int kb = 0; kb < num_kb; ++kb) {
@@ -279,7 +240,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           uint8_t* a_dst = smem + stage * Cfg::STAGE_BYTES;
           mbar_arrive_expect_tx(&full[stage], Cfg::STAGE_BYTES);
           tma_load_2d(&tmA, &full[stage], a_dst, kb * BK, m_blk * BM);
-          if (!kResident) tma_load_2d(&tmB, &full[stage], a_dst + Cfg::A_BYTES, kb * BK, n_blk * BN);
+          tma_load_2d(&tmB, &full[stage], a_dst + Cfg::A_BYTES, kb * BK, n_blk * BN);
           if (++stage == kStages) { stage = 0; phase ^= 1; }
         }
       }
@@ -290,7 +251,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     {
       constexpr uint32_t idesc = umma_idesc_f16(BM, BN);
       uint32_t stage = 0, phase = 0, as = 0, aphase = 0;
-      if (kResident && tile0 < m_blks) mbar_wait(pfull, 0, 22);
       int m_blk, n_blk;
       for (int it = 0; coords(it, m_blk, n_blk); ++it) {
         mbar_wait(&tempty[as], aphase ^ 1, 20);
@@ -300,8 +260,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           mbar_wait(&full[stage], phase, 21);
           tc_fence_after();
           const uint32_t lo_a = umma_desc_sw128_lo(smem_u32(smem)) + stage * (Cfg::STAGE_BYTES >> 4);
-          const uint32_t lo_b = kResident ? umma_desc_sw128_lo(smem_u32(sPanel)) + kb * (Cfg::B_BYTES >> 4)
-                                          : lo_a + (Cfg::A_BYTES >> 4);
+          const uint32_t lo_b = lo_a + (Cfg::A_BYTES >> 4);
           if (elect_one_sync()) {
 #pragma unroll
             for (int k = 0; k < BK / 16; ++k) {
@@ -441,8 +400,6 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
   cluster_sync_all();   // the peer's barriers exist before anything is signalled across the pair
   tc_fence_after();
   const uint32_t tmem_base = *tmem_holder;
-  pdl_launch_dependents();
-  pdl_wait();           // everything above overlapped the previous kernel's tail; global memory only from here on
 
   if (warp == 0) {
     // ===================== TMA producer (both CTAs) =====================
@@ -540,204 +497,6 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
   }
 }
 
-#ifdef VITED_EXPERIMENTAL   // measured negative results, kept as a record (profiles/README.md): not in the product library
-// =====================================================================================================================
-// Quad variant: a cluster of FOUR CTAs = two cta_group::2 pairs that compute two different 256-row tiles against the
-// SAME weight tile. Every GEMM of the step moves 7.5-9.4 TB/s through L2 (profiles/): the weight tile is re-read from L2
-// for every 256 output rows. Here each CTA fetches only a QUARTER of the weight tile per k-block and TMA-multicasts it
-// to the CTA with the same pair rank in the other pair, so one L2 read serves 512 output rows. The shared stage is
-// released only when BOTH pairs' MMAs have read it (the leaders' commits are multicast to all four CTAs).
-// =====================================================================================================================
-template <int BN, int ACT>
-__global__ void __cluster_dims__(4, 1, 1) __launch_bounds__(PairCfg<BN>::kThreads, 1)
-gemm_tc_quad_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-                    const __grid_constant__ CUtensorMap tmC, const float* __restrict__ bias, int M, int N, int K) {
-  using Cfg = PairCfg<BN>;
-  constexpr int kStages = Cfg::kStages;
-  constexpr int kEpiWarps = Cfg::kEpiWarps;
-  constexpr uint32_t BQ_BYTES = Cfg::BH_BYTES / 2;   // the quarter of the weight tile this CTA fetches
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* sC = smem + kStages * Cfg::STAGE_BYTES;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sC + Cfg::C_BYTES);
-  uint64_t* full = bars;                     // pair leader: TMA bytes of both CTAs of the pair
-  uint64_t* empty = bars + kStages;          // per CTA: BOTH pair leaders' commits (count 2)
-  uint64_t* tfull = bars + 2 * kStages;      // per CTA: own pair's commit
-  uint64_t* tempty = bars + 2 * kStages + 2; // pair leader: epilogue warps of both CTAs of the pair
-  uint32_t* tmem_holder = reinterpret_cast<uint32_t*>(bars + 2 * kStages + 4);
-
-  const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
-  const uint32_t rank4 = cluster_ctarank();
-  const uint32_t r = rank4 & 1, p = rank4 >> 1;     // rank inside the pair, pair inside the cluster
-  const int cluster = (int)(blockIdx.x >> 2);
-  const int num_clusters = (int)(gridDim.x >> 2);
-
-  const int m2_blks = (M + 2 * BM - 1) / (2 * BM);
-  const int m4_blks = (m2_blks + 1) / 2;            // the two pairs of a cluster take 256-row blocks 2*m4 and 2*m4 + 1
-  const int n_blks = (N + BN - 1) / BN;
-  const int num_tiles = m4_blks * n_blks;           // (an odd tail block is computed on zero-filled rows, stores clipped)
-  const int num_kb = (K + BK - 1) / BK;
-
-  if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&tmA);
-    tma_prefetch_desc(&tmB);
-    tma_prefetch_desc(&tmC);
-  } else if (warp == 1 && lane == 0) {
-    for (int s = 0; s < kStages; ++s) {
-      mbar_init(&full[s], 1);
-      mbar_init(&empty[s], 2);
-    }
-    for (int s = 0; s < 2; ++s) {
-      mbar_init(&tfull[s], 1);
-      mbar_init(&tempty[s], 2 * kEpiWarps);
-    }
-    fence_mbar_init();
-  } else if (warp == 2) {
-    tmem_alloc_2cta(tmem_holder, Cfg::TMEM_COLS);
-    tmem_relinquish_2cta();
-  }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_holder;
-
-  if (warp == 0) {
-    // ===================== TMA producer (all four CTAs) =====================
-    if (lane == 0) {
-      uint32_t stage = 0, phase = 0;
-      const uint16_t mc_mask = (uint16_t)((1u << r) | (1u << (r + 2)));   // same pair rank in both pairs
-      for (int tile = cluster; tile < num_tiles; tile += num_clusters) {
-        const int m4 = tile / n_blks, n_blk = tile % n_blks;
-        const int row0 = (2 * m4 + (int)p) * 2 * BM + (int)r * BM;
-        for (int kb = 0; kb < num_kb; ++kb) {
-          mbar_wait(&empty[stage], phase ^ 1, 10);
-          uint8_t* a_dst = smem + stage * Cfg::STAGE_BYTES;
-          if (r == 0) mbar_arrive_expect_tx(&full[stage], 2 * Cfg::STAGE_BYTES);
-          tma_load_2d_2cta(&tmA, &full[stage], a_dst, kb * BK, row0);
-          tma_load_2d_2cta_mc(&tmB, &full[stage], a_dst + Cfg::A_BYTES + p * BQ_BYTES, kb * BK,
-                              n_blk * BN + (int)r * (BN / 2) + (int)p * (BN / 4), mc_mask);
-          if (++stage == kStages) { stage = 0; phase ^= 1; }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ===================== MMA issuer (leader CTA of each pair; warp-uniform, elected lane) =====================
-    if (r == 0) {
-      constexpr uint32_t idesc = umma_idesc_f16(2 * BM, BN);
-      const uint16_t pair_mask = (uint16_t)(3u << (2 * p));
-      uint32_t stage = 0, phase = 0, as = 0, aphase = 0;
-      for (int tile = cluster; tile < num_tiles; tile += num_clusters) {
-        mbar_wait(&tempty[as], aphase ^ 1, 20);
-        tc_fence_after();
-        const uint32_t d_tmem = tmem_base + as * BN;
-        for (int kb = 0; kb < num_kb; ++kb) {
-          mbar_wait(&full[stage], phase, 21);
-          tc_fence_after();
-          const uint32_t lo_a = umma_desc_sw128_lo(smem_u32(smem)) + stage * (Cfg::STAGE_BYTES >> 4);
-          if (elect_one_sync()) {
-#pragma unroll
-            for (int k = 0; k < BK / 16; ++k)
-              umma_f16_2cta(d_tmem, umma_desc_pack(lo_a + 2 * k, kUmmaDescSw128Hi),
-                             umma_desc_pack(lo_a + (Cfg::A_BYTES >> 4) + 2 * k, kUmmaDescSw128Hi), idesc, (kb | k) != 0 ? 1u : 0u);
-            umma_commit_2cta_mask(&empty[stage], 0xF);   // this pair is done with the stage: tell all four CTAs
-          }
-          __syncwarp();
-          if (++stage == kStages) { stage = 0; phase ^= 1; }
-        }
-        if (elect_one_sync()) umma_commit_2cta_mask(&tfull[as], pair_mask);
-        __syncwarp();
-        if (++as == 2) { as = 0; aphase ^= 1; }
-      }
-    }
-  } else if (warp >= 4) {
-    // ===================== epilogue (every CTA, own 128 rows) =====================
-    const int ew = warp - 4;
-    const int q = warp & 3;
-    const int sl = ew >> 2;
-    uint8_t* my_stage = sC + ew * 4096;
-    uint8_t* rowp = my_stage + lane * 128;
-    uint32_t as = 0, aphase = 0;
-    bool store_pending = false;
-    for (int tile = cluster; tile < num_tiles; tile += num_clusters) {
-      const int m4 = tile / n_blks, n_blk = tile % n_blks;
-      const int row0 = (2 * m4 + (int)p) * 2 * BM + (int)r * BM;
-      const int n0 = n_blk * BN + sl * 64;
-      mbar_wait(&tfull[as], aphase, 30);
-      tc_fence_after();
-      uint32_t v0[32], v1[32];
-      const uint32_t taddr = tmem_base + as * BN + sl * 64 + (static_cast<uint32_t>(q * 32) << 16);
-      tmem_ld_32x32b_x32(taddr, v0);
-      tmem_ld_32x32b_x32(taddr + 32, v1);
-      tmem_ld_wait();
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive_leader(&tempty[as]);
-      if (store_pending) {
-        if (lane == 0) tma_store_wait_read();
-        __syncwarp();
-      }
-      epilogue_tile<ACT>(v0, v1, bias, n0, N, rowp, lane);
-      fence_proxy_async_smem();
-      __syncwarp();
-      if (lane == 0 && n0 < N && row0 < M) {
-        tma_store_2d(&tmC, my_stage, n0, row0 + q * 32);
-        tma_store_commit();
-      }
-      store_pending = true;
-      if (++as == 2) { as = 0; aphase ^= 1; }
-    }
-    if (lane == 0) tma_store_wait_all();
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  if (warp == 2) {
-    tc_fence_after();
-    tmem_dealloc_2cta(tmem_base, Cfg::TMEM_COLS);
-  }
-}
-
-template <int BN, int ACT>
-static int launch_quad(const CUtensorMap& tA, const CUtensorMap& tB, const CUtensorMap& tC, const float* bias, int M,
-                       int N, int K, cudaStream_t stream) {
-  using Cfg = PairCfg<BN>;
-  static PerDeviceOnce once;
-  static int max_clusters_dev[64];
-  int dev_id = 0;
-  cudaGetDevice(&dev_id);
-  int& max_clusters = max_clusters_dev[dev_id & 63];
-  if (once.first()) {
-    VITED_CUDA_OK(cudaFuncSetAttribute(gemm_tc_quad_kernel<BN, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)Cfg::SMEM_BYTES));
-    // how many 4-CTA clusters the device can hold at once (GPC sizes that are not multiples of 4 strand a few SMs)
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(4 * (g_num_sms / 4));
-    cfg.blockDim = dim3(Cfg::kThreads);
-    cfg.dynamicSmemBytes = Cfg::SMEM_BYTES;
-    cudaLaunchAttribute at;
-    at.id = cudaLaunchAttributeClusterDimension;
-    at.val.clusterDim.x = 4; at.val.clusterDim.y = 1; at.val.clusterDim.z = 1;
-    cfg.attrs = &at;
-    cfg.numAttrs = 1;
-    int n = 0;
-    VITED_CUDA_OK(cudaOccupancyMaxActiveClusters(&n, gemm_tc_quad_kernel<BN, ACT>, &cfg));
-    max_clusters = n > 0 ? n : 1;
-  }
-  const int m2_blks = (M + 2 * BM - 1) / (2 * BM);
-  const int tiles = ((m2_blks + 1) / 2) * ((N + BN - 1) / BN);
-  int clusters = max_clusters;
-  if (clusters > g_num_sms / 4) clusters = g_num_sms / 4;
-  if (clusters > tiles) clusters = tiles;
-  gemm_tc_quad_kernel<BN, ACT><<<4 * clusters, Cfg::kThreads, Cfg::SMEM_BYTES, stream>>>(tA, tB, tC, bias, M, N, K);
-  VITED_CUDA_OK(cudaGetLastError());
-  return 0;
-}
-
-#endif  // VITED_EXPERIMENTAL
-
 template <int BN, int ACT>
 static int launch_pair(const CUtensorMap& tA, const CUtensorMap& tB, const CUtensorMap& tC, const float* bias, int M,
                        int N, int K, cudaStream_t stream) {
@@ -749,53 +508,35 @@ static int launch_pair(const CUtensorMap& tA, const CUtensorMap& tB, const CUten
   const int tiles = ((M + 2 * BM - 1) / (2 * BM)) * ((N + BN - 1) / BN);
   int pairs = g_num_sms / 2;
   if (pairs > tiles) pairs = tiles;
-  VITED_CUDA_OK(launch_pdl(gemm_tc_pair_kernel<BN, ACT>, dim3(2 * pairs), dim3(Cfg::kThreads), Cfg::SMEM_BYTES, stream, tA, tB,
-                           tC, bias, M, N, K));
-  return 0;
-}
-
-static int g_order = 0;     // VITED_GEMM_ORDER=1: every CTA owns an m-block (measured ~4 % slower: off by default)
-
-template <int BN, int ACT, int KB_RES>
-static int launch_tc(const CUtensorMap& tA, const CUtensorMap& tB, const CUtensorMap& tC, const float* bias, int M,
-                     int N, int K, cudaStream_t stream) {
-  using Cfg = GemmCfg<BN, KB_RES>;
-  static PerDeviceOnce once;
-  if (once.first())
-    VITED_CUDA_OK(cudaFuncSetAttribute(gemm_tc_kernel<BN, ACT, KB_RES>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)Cfg::SMEM_BYTES));
-  const int m_blks = (M + BM - 1) / BM, n_blks = (N + BN - 1) / BN;
-  int grid, order = 0;
-  if (KB_RES > 0) {
-    int per_n = g_num_sms / n_blks;   // CTAs per weight panel
-    if (per_n > m_blks) per_n = m_blks;
-    grid = per_n * n_blks;
-  } else {
-    const int tiles = m_blks * n_blks;
-    grid = tiles < g_num_sms ? tiles : g_num_sms;
-    if (g_order != 0 && n_blks > 1 && m_blks >= 4 * g_num_sms) order = 1;
-  }
-  gemm_tc_kernel<BN, ACT, KB_RES><<<grid, Cfg::kThreads, Cfg::SMEM_BYTES, stream>>>(tA, tB, tC, bias, M, N, K, order);
+  gemm_tc_pair_kernel<BN, ACT><<<2 * pairs, Cfg::kThreads, Cfg::SMEM_BYTES, stream>>>(tA, tB, tC, bias, M, N, K);
   VITED_CUDA_OK(cudaGetLastError());
   return 0;
 }
 
-template <int BN, int KB_RES>
+template <int BN, int ACT>
+static int launch_tc(const CUtensorMap& tA, const CUtensorMap& tB, const CUtensorMap& tC, const float* bias, int M,
+                     int N, int K, cudaStream_t stream) {
+  using Cfg = GemmCfg<BN>;
+  static PerDeviceOnce once;
+  if (once.first())
+    VITED_CUDA_OK(cudaFuncSetAttribute(gemm_tc_kernel<BN, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)Cfg::SMEM_BYTES));
+  const int tiles = ((M + BM - 1) / BM) * ((N + BN - 1) / BN);
+  const int grid = tiles < g_num_sms ? tiles : g_num_sms;
+  gemm_tc_kernel<BN, ACT><<<grid, Cfg::kThreads, Cfg::SMEM_BYTES, stream>>>(tA, tB, tC, bias, M, N, K);
+  VITED_CUDA_OK(cudaGetLastError());
+  return 0;
+}
+
+template <int BN>
 static int launch_act(const CUtensorMap& tA, const CUtensorMap& tB, const CUtensorMap& tC, const float* bias, int M,
                       int N, int K, int act, cudaStream_t stream) {
-  return act == ACT_GELU ? launch_tc<BN, ACT_GELU, KB_RES>(tA, tB, tC, bias, M, N, K, stream)
-                         : launch_tc<BN, ACT_NONE, KB_RES>(tA, tB, tC, bias, M, N, K, stream);
+  return act == ACT_GELU ? launch_tc<BN, ACT_GELU>(tA, tB, tC, bias, M, N, K, stream)
+                         : launch_tc<BN, ACT_NONE>(tA, tB, tC, bias, M, N, K, stream);
 }
 
 int gemm_simt(const act_t* A, const act_t* W, const float* bias, act_t* C, int M, int N, int K, int act,
               cudaStream_t stream);
-
-static int g_block_n = 0;   // 0 = unread; VITED_GEMM_BN=128|192|256 overrides the automatic tile width (tuning knob)
-static int g_pair = -1;     // VITED_GEMM_PAIR=0 disables the CTA-pair (cta_group::2) kernel (used for large M by default)
-#ifdef VITED_EXPERIMENTAL
-static int g_quad = -1;     // VITED_GEMM_QUAD=1 enables the 4-CTA-cluster kernel with multicast weight tiles (large M)
-static int g_resident = -1; // VITED_GEMM_RESIDENT=1 enables the resident-weights variant (measured slower)
-#endif
 
 int gemm_act(const act_t* A, const act_t* W, const float* bias, act_t* C, int M, int N, int K, int act, int impl,
               cudaStream_t stream) {
@@ -808,52 +549,16 @@ int gemm_act(const act_t* A, const act_t* W, const float* bias, act_t* C, int M,
   VITED_CHECK((reinterpret_cast<uintptr_t>(A) & 15) == 0 && (reinterpret_cast<uintptr_t>(W) & 15) == 0 &&
                   (reinterpret_cast<uintptr_t>(C) & 15) == 0,
               "gemm_act: operands must be 16-byte aligned");
-  if (g_block_n == 0) {
-    const char* e = getenv("VITED_GEMM_BN");
-    g_block_n = e ? atoi(e) : -1;
-#ifdef VITED_EXPERIMENTAL
-    const char* r = getenv("VITED_GEMM_RESIDENT");
-    g_resident = r ? atoi(r) : 0;
-    const char* qd = getenv("VITED_GEMM_QUAD");
-    g_quad = qd ? atoi(qd) : 0;
-#endif
-    const char* o = getenv("VITED_GEMM_ORDER");
-    g_order = o ? atoi(o) : 0;
-    const char* pr = getenv("VITED_GEMM_PAIR");
-    g_pair = pr ? atoi(pr) : 1;
-  }
+  // Tile width: the widest of 256 / 192 / 128 that divides N. Large M (at least two 128-row blocks per SM) goes to the
+  // CTA-pair kernel when N takes a 256- or 192-wide tile.
   const int m_blks = (M + BM - 1) / BM;
-  // resident weights: K <= 384, 128-wide panels, and enough m-blocks per panel to amortise loading it
-#ifdef VITED_EXPERIMENTAL
-  const bool resident = g_resident && g_block_n < 0 && K <= 384 && N % 128 == 0 && N / 128 <= 16 &&
-                        m_blks >= 4 * (g_num_sms / (N / 128));
-#else
-  const bool resident = false;   // the resident-weights instantiation (KB_RES = 6) exists in -DVITED_EXPERIMENTAL builds only
-#endif
-  int bn = 128;
-  if (!resident) {
-    if (g_block_n == 128 || g_block_n == 192 || g_block_n == 256) bn = g_block_n;
-    else if (N % 256 == 0) bn = 256;
-    else if (N % 192 == 0) bn = 192;
-  }
+  const int bn = N % 256 == 0 ? 256 : N % 192 == 0 ? 192 : 128;
   CUtensorMap tA, tB, tC;
   if (make_tmap(&tA, A, (uint64_t)K, (uint64_t)M, (uint64_t)K * 2, BM)) return 1;
-  if (g_pair && g_block_n != 128 && m_blks >= 2 * g_num_sms && (N % 256 == 0 || N % 192 == 0)) {
-    const int pbn = (g_block_n == 192 || g_block_n == 256) ? g_block_n : (N % 256 == 0 ? 256 : 192);
-#ifdef VITED_EXPERIMENTAL
-    if (g_quad && m_blks >= 4 * g_num_sms) {
-      if (make_tmap(&tB, W, (uint64_t)K, (uint64_t)N, (uint64_t)K * 2, (uint32_t)pbn / 4)) return 1;
-      if (make_tmap(&tC, C, (uint64_t)N, (uint64_t)M, (uint64_t)N * 2, 32)) return 1;
-      if (pbn == 256)
-        return act == ACT_GELU ? launch_quad<256, ACT_GELU>(tA, tB, tC, bias, M, N, K, stream)
-                               : launch_quad<256, ACT_NONE>(tA, tB, tC, bias, M, N, K, stream);
-      return act == ACT_GELU ? launch_quad<192, ACT_GELU>(tA, tB, tC, bias, M, N, K, stream)
-                             : launch_quad<192, ACT_NONE>(tA, tB, tC, bias, M, N, K, stream);
-    }
-#endif
-    if (make_tmap(&tB, W, (uint64_t)K, (uint64_t)N, (uint64_t)K * 2, (uint32_t)pbn / 2)) return 1;
+  if (bn != 128 && m_blks >= 2 * g_num_sms) {
+    if (make_tmap(&tB, W, (uint64_t)K, (uint64_t)N, (uint64_t)K * 2, (uint32_t)bn / 2)) return 1;
     if (make_tmap(&tC, C, (uint64_t)N, (uint64_t)M, (uint64_t)N * 2, 32)) return 1;
-    if (pbn == 256)
+    if (bn == 256)
       return act == ACT_GELU ? launch_pair<256, ACT_GELU>(tA, tB, tC, bias, M, N, K, stream)
                              : launch_pair<256, ACT_NONE>(tA, tB, tC, bias, M, N, K, stream);
     return act == ACT_GELU ? launch_pair<192, ACT_GELU>(tA, tB, tC, bias, M, N, K, stream)
@@ -861,12 +566,9 @@ int gemm_act(const act_t* A, const act_t* W, const float* bias, act_t* C, int M,
   }
   if (make_tmap(&tB, W, (uint64_t)K, (uint64_t)N, (uint64_t)K * 2, (uint32_t)bn)) return 1;
   if (make_tmap(&tC, C, (uint64_t)N, (uint64_t)M, (uint64_t)N * 2, 32)) return 1;
-#ifdef VITED_EXPERIMENTAL
-  if (resident) return launch_act<128, 6>(tA, tB, tC, bias, M, N, K, act, stream);
-#endif
-  if (bn == 128) return launch_act<128, 0>(tA, tB, tC, bias, M, N, K, act, stream);
-  if (bn == 256) return launch_act<256, 0>(tA, tB, tC, bias, M, N, K, act, stream);
-  return launch_act<192, 0>(tA, tB, tC, bias, M, N, K, act, stream);
+  if (bn == 128) return launch_act<128>(tA, tB, tC, bias, M, N, K, act, stream);
+  if (bn == 256) return launch_act<256>(tA, tB, tC, bias, M, N, K, act, stream);
+  return launch_act<192>(tA, tB, tC, bias, M, N, K, act, stream);
 }
 
 }  // namespace vited

@@ -211,11 +211,6 @@ int attention(const AttnArgs& a, int impl, cudaStream_t stream);
 // tcgen05/TMEM kernels for the hot decoder shapes (attention_tc.cu); attention() dispatches to them by itself
 bool attention_tc_supported(const AttnArgs& a);
 int attention_tc(const AttnArgs& a, cudaStream_t stream);
-// puzzle shape with two (sequence, head) units per 128-row tile (attention_pair.cu; -DVITED_EXPERIMENTAL builds only)
-bool attention_pair_supported(const AttnArgs& a);
-int attention_pair(const AttnArgs& a, cudaStream_t stream);
-bool attention_tc_cls_supported(const AttnArgs& a);
-int attention_tc_cls(const AttnArgs& a, cudaStream_t stream);
 // class-token query only: q and o are the full split-layout buffers (q_has_cls = 1); only their class-token rows
 // (row n_seq*nq_patch + b) are read / written. The puzzle-shape warp kernel assumes nq_patch = 64.
 int attention_cls(const AttnArgs& a, cudaStream_t stream);

@@ -17,9 +17,10 @@
 //     residual boxes live in the h-tile region, which is dead once fc1 of the last chunk has completed.
 // TMEM: O = columns [0, 384), S buffers [384, 448) and [448, 512). Shared memory: 96 KB h tile / residual boxes,
 // 96 KB weight ring, 16 KB output staging, biases / LayerNorm parameters.
-// Template parameter CG = column groups of the GELU / epilogue warps: 2 (8 warps: 32 hidden columns of a chunk and a
-// 192-column half row each) or 4 (16 warps: 16 hidden columns and a 96-column quarter row each, residual boxes of half
-// the width, weight ring of 6 slots, 32 KB staging) -- same bytes, twice as many independent chains in flight.
+// Template parameter CG = column groups of the GELU / epilogue warps. The library instantiates CG = 2 (8 warps: 32 hidden
+// columns of a chunk and a 192-column half row each). CG = 4 (16 warps: 16 hidden columns and a 96-column quarter row
+// each, residual boxes of half the width, weight ring of 6 slots, 32 KB staging) was measured neutral
+// (profiles/README.md) and is not built.
 //
 // Template parameter PRO adds the cross-attention projection in front (cproj_mlp_resid_ln, the decoder's
 //     x_mid = x + o W_cproj^T + b_cproj;  h = norm2(x_mid);  then the MLP sub-block above on h and x_mid):
@@ -186,8 +187,6 @@ mlp_ln_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
   cluster_sync_all();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_holder;
-  pdl_launch_dependents();
-  pdl_wait();           // the prologue above overlapped the previous kernel's tail; global memory only from here on
 
   if (warp == 0) {
     // ===================== weight producer (both CTAs): slots in the order the issuer consumes them ================
@@ -705,11 +704,11 @@ bool cproj_mlp_resid_ln_supported(int M, int D, int K, int hidden) {
 }
 
 // PRO: a_in = o and Wp / bproj / ln2_* the cross projection and norm2; otherwise a_in = h and those are unused
-template <int CG, bool PRO>
+template <bool PRO>
 static int mlp_ln_launch(const act_t* a_in, const act_t* Wp, const float* bproj, const float* ln2_w, const float* ln2_b,
                          const act_t* W1, const float* b1, const act_t* W2, const float* b2, float* x, const float* ln_w,
                          const float* ln_b, act_t* h_out, int M, int D, int hidden, float eps, cudaStream_t stream) {
-  using Cfg = MlpCfg<CG>;
+  using Cfg = MlpCfg<2>;
   const char* name = PRO ? "cproj_mlp_resid_ln" : "mlp_resid_ln";
   const int sms = gemm_num_sms();
   VITED_CHECK(sms >= 2, "%s: no device", name);
@@ -717,7 +716,7 @@ static int mlp_ln_launch(const act_t* a_in, const act_t* Wp, const float* bproj,
   VITED_CHECK(smem <= 232448, "%s: hidden=%d needs %u bytes of shared memory", name, hidden, smem);
   static PerDeviceOnce once;
   if (once.first())
-    VITED_CUDA_OK(cudaFuncSetAttribute(mlp_ln_pair_kernel<CG, PRO>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
+    VITED_CUDA_OK(cudaFuncSetAttribute(mlp_ln_pair_kernel<2, PRO>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
   CUtensorMap tA, tWp, tW1, tW2, tX, tH;
   if (make_tmap_act_2d(&tA, a_in, (uint64_t)D, (uint64_t)M, (uint64_t)D * 2, 64, BM, 128)) return 1;
   if (make_tmap_act_2d(&tW1, W1, (uint64_t)D, (uint64_t)hidden, (uint64_t)D * 2, 64, HC / 2, 128)) return 1;
@@ -732,8 +731,9 @@ static int mlp_ln_launch(const act_t* a_in, const act_t* Wp, const float* bproj,
   const int tiles = (M + 2 * BM - 1) / (2 * BM);
   int pairs = sms / 2;
   if (pairs > tiles) pairs = tiles;
-  VITED_CUDA_OK(launch_pdl(mlp_ln_pair_kernel<CG, PRO>, dim3(2 * pairs), dim3(Cfg::kThreads), smem, stream, tA, tWp, tW1,
-                           tW2, tX, tH, bproj, ln2_w, ln2_b, b1, b2, ln_w, ln_b, M, hidden, eps));
+  mlp_ln_pair_kernel<2, PRO><<<2 * pairs, Cfg::kThreads, smem, stream>>>(tA, tWp, tW1, tW2, tX, tH, bproj, ln2_w, ln2_b,
+                                                                          b1, b2, ln_w, ln_b, M, hidden, eps);
+  VITED_CUDA_OK(cudaGetLastError());
   return 0;
 }
 
@@ -744,13 +744,8 @@ int mlp_resid_ln(const act_t* h_in, const act_t* W1, const float* b1, const act_
   VITED_CHECK(((reinterpret_cast<uintptr_t>(h_in) | reinterpret_cast<uintptr_t>(W1) | reinterpret_cast<uintptr_t>(W2) |
                 reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(h_out)) & 15) == 0,
               "mlp_resid_ln: operands must be 16-byte aligned");
-#ifdef VITED_EXPERIMENTAL   // measured neutral (profiles/README.md): not in the product library
-  if (epilogue_warps() == 16)
-    return mlp_ln_launch<4, false>(h_in, nullptr, nullptr, nullptr, nullptr, W1, b1, W2, b2, x, ln_w, ln_b, h_out, M, D,
-                                   hidden, eps, stream);
-#endif
-  return mlp_ln_launch<2, false>(h_in, nullptr, nullptr, nullptr, nullptr, W1, b1, W2, b2, x, ln_w, ln_b, h_out, M, D,
-                                 hidden, eps, stream);
+  return mlp_ln_launch<false>(h_in, nullptr, nullptr, nullptr, nullptr, W1, b1, W2, b2, x, ln_w, ln_b, h_out, M, D,
+                              hidden, eps, stream);
 }
 
 int cproj_mlp_resid_ln(const act_t* o, const act_t* Wp, const float* bp, float* x, const float* ln2_w,
@@ -763,7 +758,7 @@ int cproj_mlp_resid_ln(const act_t* o, const act_t* Wp, const float* bp, float* 
                 reinterpret_cast<uintptr_t>(W2) | reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(h_out)) &
                15) == 0,
               "cproj_mlp_resid_ln: operands must be 16-byte aligned");
-  return mlp_ln_launch<2, true>(o, Wp, bp, ln2_w, ln2_b, W1, b1, W2, b2, x, ln_w, ln_b, h_out, M, D, hidden, eps, stream);
+  return mlp_ln_launch<true>(o, Wp, bp, ln2_w, ln2_b, W1, b1, W2, b2, x, ln_w, ln_b, h_out, M, D, hidden, eps, stream);
 }
 
 }  // namespace vited
