@@ -59,18 +59,11 @@ enum {
   VITED_OPT_GEMM_IMPL = 0,      /* 0 = tcgen05/TMA kernel (default), 1 = SIMT debugging reference kernel        */
   VITED_OPT_ATTN_IMPL = 1,      /* 0 = default (tcgen05/TMEM kernel where the shape has one, else the mma.sync flash
                                    kernel), 1 = SIMT debugging reference kernel, 2 = mma.sync flash kernel always   */
-  VITED_OPT_CHUNK_ROWS = 2,     /* target token rows per decoder chunk (default 524288)                          */
-  VITED_OPT_CACHE_LAYER0 = 3,   /* 1 (default) = run decoder layer 0's self-attention once per item, not per pair */
+  VITED_OPT_CHUNK_ROWS = 2,     /* target token rows per decoder chunk (default 524288). Chunks of at least 8192 rows
+                                   (embed_dim 384) run the fused residual + LayerNorm kernels, smaller ones do not  */
   VITED_OPT_PROFILE = 4,        /* 1 = record a CUDA event before every launch (see vited_profile_json); default 0   */
-  VITED_OPT_PRUNE_TAIL = 5,     /* 1 (default) = in the last decoder layer run everything after the K/V projection of
-                                   its self-attention on the class-token rows only (only row 0 reaches the head)   */
-  VITED_OPT_FUSE_LN = 6,        /* 1 (default) = residual add + LayerNorm run in the epilogue of the producing GEMM
-                                   (embed_dim 384, large row counts); 0 = separate resid_ln kernel                  */
   VITED_OPT_KV_BUDGET_MB = 7,   /* vited_score_grid processes context rows in blocks whose K/V cache (all decoder
                                    layers) fits this many MB (default 8000; Hisfrag: 18.9 MB per fragment)          */
-  VITED_OPT_FUSE_MLP = 8,       /* 1 (default) = the MLP sub-block (fc1, GELU, fc2), its residual add and the next
-                                   layer's LayerNorm run in one kernel, hidden activations never written (needs
-                                   FUSE_LN; embed_dim 384, large row counts); 0 = fc1 GEMM + fused fc2 GEMM          */
   VITED_OPT_XSRC_BUDGET_MB = 9  /* vited_score_grid(_u8) holds the decoder input states of at most this many MB of grid
                                    columns at once (default 32000; (N_e + 1) * embed_dim * 4 bytes per column item,
                                    Hisfrag: 1.57 MB). When all columns of a call fit, they are built once up front;

@@ -15,11 +15,10 @@ for seed in (0, 5):
     model = model.cuda().eval()
     images = synthetic.synthetic_images(int(os.environ.get('N_ITEMS', '16')), 64, seed=33)
     want = orc.score_puzzle_grid(sd, 12, images, batch=80)
-    for name, opts in (('default', {}), ('unfused LN', {vited_b200.OPT_FUSE_LN: 0}), ('mma.sync attention', {vited_b200.OPT_ATTN_IMPL: 2}),
-                       ('unfused + mma.sync', {vited_b200.OPT_FUSE_LN: 0, vited_b200.OPT_ATTN_IMPL: 2}),
-                       ('no tail pruning / layer-0 cache', {vited_b200.OPT_PRUNE_TAIL: 0, vited_b200.OPT_CACHE_LAYER0: 0})):
-        for k in (vited_b200.OPT_FUSE_LN, vited_b200.OPT_PRUNE_TAIL, vited_b200.OPT_CACHE_LAYER0):
-            model.set_option(k, 1)
+    small = {vited_b200.OPT_CHUNK_ROWS: 65 * 100}   # chunks of 6,500 rows take the unfused residual + LayerNorm path
+    for name, opts in (('default', {}), ('unfused LN', small), ('mma.sync attention', {vited_b200.OPT_ATTN_IMPL: 2}),
+                       ('unfused + mma.sync', {**small, vited_b200.OPT_ATTN_IMPL: 2})):
+        model.set_option(vited_b200.OPT_CHUNK_ROWS, 524288)
         model.set_option(vited_b200.OPT_ATTN_IMPL, 0)
         for k, v in opts.items():
             model.set_option(k, v)

@@ -150,8 +150,7 @@ def test_resid_ln(D, has_cls):
 
 @pytest.mark.parametrize('shape', [(256, 384), (70000, 384), (33333, 1536), (1, 384), (300, 64), (40000, 192)],
                          ids=lambda s: 'x'.join(map(str, s)))
-@pytest.mark.parametrize('epi_warps', ['8'])
-def test_gemm_resid_ln_fused(shape, epi_warps):
+def test_gemm_resid_ln_fused(shape):
     """x += A W^T + b; h = LayerNorm(x): the fused tcgen05 epilogue (8 warps x 192-column half rows) against fp32 torch
     on the same 16-bit operands."""
     L = _lib()
@@ -180,8 +179,7 @@ def test_gemm_resid_ln_fused(shape, epi_warps):
 
 @pytest.mark.parametrize('shape', [(256, 1536), (70000, 1536), (33333, 1536), (1, 1536), (300, 64), (40000, 192),
                                    (262144 + 77, 1536)], ids=lambda s: 'x'.join(map(str, s)))
-@pytest.mark.parametrize('epi_warps', ['8'])
-def test_mlp_resid_ln_fused(shape, epi_warps):
+def test_mlp_resid_ln_fused(shape):
     """x += fc2(GELU(fc1(h))) + b2; h = LayerNorm(x): the fused MLP kernel (hidden activations kept in TMEM, GELU
     output fed to the second MMA as its A operand from TMEM) against fp32 torch on the same 16-bit operands, with the
     hidden activations rounded to 16 bits where the kernel rounds them. In place: h_out aliases h_in."""

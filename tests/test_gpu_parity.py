@@ -141,23 +141,18 @@ def hisfrag_case():
 
 def _restore(model):
     import vited_b200
-    for opt, val in ((vited_b200.OPT_FUSE_LN, 1), (vited_b200.OPT_PRUNE_TAIL, 1), (vited_b200.OPT_CACHE_LAYER0, 1),
-                     (vited_b200.OPT_KV_BUDGET_MB, 8000), (vited_b200.OPT_CHUNK_ROWS, 524288)):
-        model.set_option(opt, val)
+    model.set_option(vited_b200.OPT_KV_BUDGET_MB, 8000)
+    model.set_option(vited_b200.OPT_CHUNK_ROWS, 524288)
 
 
-@pytest.mark.parametrize('variant', ['default', 'unfused_ln', 'no_prune', 'no_layer0_cache', 'small_chunks'])
+@pytest.mark.parametrize('variant', ['default', 'unfused_ln', 'small_chunks'])
 def test_hisfrag_model_grid_matches_oracle_on_the_production_path(hisfrag_case, variant):
     import vited_b200
     from vited_b200 import grid
     model, kw, images, labels, want = hisfrag_case
     _restore(model)
     if variant == 'unfused_ln':
-        model.set_option(vited_b200.OPT_FUSE_LN, 0)
-    elif variant == 'no_prune':
-        model.set_option(vited_b200.OPT_PRUNE_TAIL, 0)
-    elif variant == 'no_layer0_cache':
-        model.set_option(vited_b200.OPT_CACHE_LAYER0, 0)
+        model.set_option(vited_b200.OPT_CHUNK_ROWS, 1025 * 7)         # 6 chunks of 6 pairs (6,150 rows: unfused)
     elif variant == 'small_chunks':
         model.set_option(vited_b200.OPT_CHUNK_ROWS, 1025 * 10)        # 4 chunks of 9 pairs (9,225 rows: still fused)
     n0 = model.launch_count()
@@ -263,7 +258,7 @@ def test_sharp_attention_matches_oracle_on_the_production_shape(gain):
 
 def test_grid_properties_puzzle_model():
     """Size-independent properties on the real puzzle model: grid == pair-wise API; row sharding is exact;
-    chunking and layer-0 caching do not change results; every off-diagonal entry is written."""
+    chunking does not change results; every off-diagonal entry is written."""
     import vited_b200
     from vited_b200 import grid
     model, sd, kw, images = _grid_case('puzzle_patch8_64', 40)
@@ -287,26 +282,6 @@ def test_grid_properties_puzzle_model():
     small = grid.score_puzzle(model, images)
     # (chunks this small take the unfused residual + LayerNorm path: one more 16-bit rounding per sub-block)
     np.testing.assert_allclose(small.cpu().numpy(), full.cpu().numpy(), rtol=0, atol=1e-2)
-    # (4) without the layer-0 cache (self-attention recomputed per pair): same values up to rounding noise
-    model.set_option(vited_b200.OPT_CACHE_LAYER0, 0)
-    nocache = grid.score_puzzle(model, images)
-    np.testing.assert_allclose(nocache.cpu().numpy(), full.cpu().numpy(), rtol=0, atol=1e-2)
-    # (5) without last-layer pruning (all 65 rows carried to the end): same values up to rounding noise
-    model.set_option(vited_b200.OPT_CACHE_LAYER0, 1)
-    model.set_option(vited_b200.OPT_PRUNE_TAIL, 0)
-    noprune = grid.score_puzzle(model, images)
-    np.testing.assert_allclose(noprune.cpu().numpy(), full.cpu().numpy(), rtol=0, atol=1e-2)
-    # (6) residual + LayerNorm as a separate kernel instead of the fused GEMM epilogue: same values up to rounding noise
-    #     (the fused path never rounds the projection output to 16 bits before the residual add)
-    model.set_option(vited_b200.OPT_PRUNE_TAIL, 1)
-    model.set_option(vited_b200.OPT_FUSE_LN, 0)
-    unfused = grid.score_puzzle(model, images)
-    np.testing.assert_allclose(unfused.cpu().numpy(), full.cpu().numpy(), rtol=0, atol=1e-2)
-    model.set_option(vited_b200.OPT_FUSE_LN, 1)
-    model.set_option(vited_b200.OPT_PRUNE_TAIL, 0)
-    both = grid.score_puzzle(model, images)
-    np.testing.assert_allclose(both.cpu().numpy(), full.cpu().numpy(), rtol=0, atol=1e-2)
-
 
 def test_argmax_agreement_puzzle_model():
     """>= 99.9 % identical argmax adjacency vs the fp32 oracle is the north-star bar; on a few hundred pairs the
@@ -338,6 +313,17 @@ def test_errors_are_loud():
         model.score_grid(torch.zeros(4, 3, kw['img_size'], kw['img_size'], device='cuda'), 0, 3, 2)
     out = model.score_grid(torch.zeros(0, 3, kw['img_size'], kw['img_size'], device='cuda'), 0)
     assert out.shape == (0, 0, kw['num_classes'])
+
+
+def test_removed_options_are_unknown():
+    """Options 3, 5, 6 and 8 once switched the layer-0 cache, the pruned last layer and the fused LayerNorm / MLP
+    kernels off. The decoder's launch sequence now follows from the input shape alone, and these numbers are errors."""
+    import vited_b200
+    z, kw = helpers.load_model_case('small_hd32')
+    model, _ = helpers.make_gpu_model(kw, 1)
+    for opt in (3, 5, 6, 8):
+        with pytest.raises(vited_b200.VitedError, match='unknown option'):
+            model.set_option(opt, 0)
 
 
 @pytest.mark.parametrize('name,mode,n', [('small_hd32', 'puzzle', 80), ('small_hd64', 'fragments', 90),

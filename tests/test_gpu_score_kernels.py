@@ -433,8 +433,7 @@ def _run_exact(kernel, x, lw, lb, g):
 @pytest.mark.parametrize('affine', ['unit', 'random'])
 @pytest.mark.parametrize('pattern', ['within', 'between'])
 @pytest.mark.parametrize('kernel', EXACT_KERNELS)
-@pytest.mark.parametrize('epi_warps', ['8'])
-def test_layernorm_of_exactly_representable_rows(kernel, pattern, affine, epi_warps):
+def test_layernorm_of_exactly_representable_rows(kernel, pattern, affine):
     """Rows whose LayerNorm is exactly +-1 (_exact_rows). With ln_w = 1, ln_b = 0 the output must be exactly +-1: a
     variance divided by D - 1 gives +-0.9987 (3 fp16 steps, 1 bf16 step below 1) and fails bit-exactly, and in the
     'between' pattern a lost between-group term of the Chan combination gives a zero variance. With random ln_w / ln_b

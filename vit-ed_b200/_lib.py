@@ -37,12 +37,8 @@ GRID_UPPER_TRI_DIAG = 1
 OPT_GEMM_IMPL = 0
 OPT_ATTN_IMPL = 1
 OPT_CHUNK_ROWS = 2
-OPT_CACHE_LAYER0 = 3
 OPT_PROFILE = 4
-OPT_PRUNE_TAIL = 5
-OPT_FUSE_LN = 6
 OPT_KV_BUDGET_MB = 7
-OPT_FUSE_MLP = 8
 OPT_XSRC_BUDGET_MB = 9
 
 _vp = ctypes.c_void_p

@@ -91,10 +91,6 @@ struct vited_engine {
   // options
   int gemm_impl = IMPL_FAST, attn_impl = IMPL_FAST;
   int64_t chunk_rows = 524288;   // measured: 262144 -> 524288 rows per chunk +4.7 % (fewer launch tails), no gain beyond
-  int cache_layer0 = 1;
-  int prune_tail = 1;   // last decoder layer: only the class-token row continues past self-attention
-  int fuse_ln = 1;      // residual + LayerNorm in the epilogue of the N = 384 GEMMs (gemm_ln.cu)
-  int fuse_mlp = 1;     // fc1 + GELU + fc2 + residual + LayerNorm in one kernel (mlp_ln.cu); needs fuse_ln
   int kv_budget_mb = 8000;  // K/V cache budget of one block of context rows in vited_score_grid
   int64_t xsrc_budget_mb = 32000;  // decoder input states of one window of grid columns in vited_score_grid
   int64_t launches = 0;
@@ -253,10 +249,14 @@ static int L_gemm(vited_engine* e, const act_t* A, const Linear& l, act_t* Cout,
   }
   return gemm_act(A, l.w, l.b, Cout, M, l.out, l.in, act, e->gemm_impl, s);
 }
-// fused x += A W^T + b; h = LN(x)  (gemm_ln.cu). Caller has checked use_fused_ln().
-static bool use_fused_ln(vited_engine* e, size_t rows, const Linear& l) {
-  return e->fuse_ln && e->gemm_impl == IMPL_FAST && rows >= 8192 && gemm_resid_ln_supported((int)rows, l.out, l.in);
+// Whether a decoder chunk of `rows` token rows runs fused: every residual add + LayerNorm in the epilogue of the kernel
+// that produces the sub-block output (gemm_ln.cu, mlp_ln.cu). Chunks below 8192 rows run the unfused sequence.
+static bool use_fused(vited_engine* e, size_t rows) {
+  const DecBlock& b = e->dec[0];
+  return e->gemm_impl == IMPL_FAST && rows >= 8192 && gemm_resid_ln_supported((int)rows, b.proj.out, b.proj.in) &&
+         cproj_mlp_resid_ln_supported((int)rows, e->D, b.cproj.in, e->hidden);
 }
+// fused x += A W^T + b; h = LN(x)  (gemm_ln.cu)
 static int L_gemm_ln(vited_engine* e, const act_t* A, const Linear& l, float* x, const LNorm& ln, act_t* h, int M,
                      cudaStream_t s) {
   if (e->profile) {
@@ -270,10 +270,6 @@ static int L_gemm_ln(vited_engine* e, const act_t* A, const Linear& l, float* x,
   return gemm_resid_ln(A, l.w, l.b, x, ln.w, ln.b, h, M, l.out, l.in, 1e-6f, s);
 }
 // fused x += cproj(o); x += fc2(GELU(fc1(norm2(x)))) ; h = LN(x)  (mlp_ln.cu)
-static bool use_fused_mlp(vited_engine* e, size_t rows, const Linear& cproj, const Linear& fc1, const Linear& fc2) {
-  return e->fuse_mlp && use_fused_ln(e, rows, fc2) && use_fused_ln(e, rows, cproj) && cproj.out == e->D &&
-         fc1.in == e->D && fc2.in == fc1.out && cproj_mlp_resid_ln_supported((int)rows, e->D, cproj.in, fc1.out);
-}
 static int L_cproj_mlp_ln(vited_engine* e, const act_t* o, const Linear& cproj, const LNorm& norm2, const Linear& fc1,
                           const Linear& fc2, float* x, const LNorm& ln, act_t* h_out, int M, cudaStream_t s) {
   if (e->profile) {
@@ -444,22 +440,21 @@ static int encoder_stack(vited_engine* e, int B, float* out_tokens, cudaStream_t
   return 0;
 }
 
-// prepare_x2 (vision_transformer.py:390-395) [+ decoder layer 0's self-attention sub-block when cached] for a
-// sub-batch whose patch tokens are in e->tok. Result (split layout, B sequences) is left in e->x.
+// prepare_x2 (vision_transformer.py:390-395) + decoder layer 0's self-attention sub-block for a sub-batch whose patch
+// tokens are in e->tok: that sub-block depends on the item alone, so it runs once per item, not once per pair. Result
+// (split layout, B sequences) is left in e->x.
 static int decoder_item_state(vited_engine* e, int B, cudaStream_t s) {
   const size_t rows = (size_t)B * e->Nd;
   TRY(ensure_rows(e, rows));
   float* x = e->x.as<float>();
   prof_mark(e, "assemble", 0.0, (double)rows * e->D * 6.0, s);
   TRY(assemble_tokens(e->tok.as<act_t>(), e->pos, e->cls, x, B, e->Ne, e->D, 1, s));
-  if (e->cache_layer0) {
-    DecBlock& b = e->dec[0];
-    TRY(L_resid_ln(e, x, nullptr, nullptr, nullptr, 0, &b.norm1, e->h.as<act_t>(), B, 1, 0, s));
-    TRY(L_gemm(e, e->h.as<act_t>(), b.qkv, e->qkv.as<act_t>(), (int)rows, ACT_NONE, s));
-    TRY(L_attn_self(e, e->qkv.as<act_t>(), e->o.as<act_t>(), B, 1, s));
-    TRY(L_gemm(e, e->o.as<act_t>(), b.proj, e->delta.as<act_t>(), (int)rows, ACT_NONE, s));
-    TRY(L_resid_ln(e, x, e->delta.as<act_t>(), nullptr, nullptr, 0, nullptr, nullptr, B, 1, 1, s));
-  }
+  DecBlock& b = e->dec[0];
+  TRY(L_resid_ln(e, x, nullptr, nullptr, nullptr, 0, &b.norm1, e->h.as<act_t>(), B, 1, 0, s));
+  TRY(L_gemm(e, e->h.as<act_t>(), b.qkv, e->qkv.as<act_t>(), (int)rows, ACT_NONE, s));
+  TRY(L_attn_self(e, e->qkv.as<act_t>(), e->o.as<act_t>(), B, 1, s));
+  TRY(L_gemm(e, e->o.as<act_t>(), b.proj, e->delta.as<act_t>(), (int)rows, ACT_NONE, s));
+  TRY(L_resid_ln(e, x, e->delta.as<act_t>(), nullptr, nullptr, 0, nullptr, nullptr, B, 1, 1, s));
   return 0;
 }
 
@@ -508,69 +503,36 @@ static int decode_chunk(vited_engine* e, int P, const int* ci, const int* xj, co
   act_t* hid = e->hid.as<act_t>();
   const size_t kv_per_layer = (size_t)n_kv_seq * e->Ne * 2 * D;
   const size_t L = e->dec.size();
-  // With FUSE_LN the residual add + LayerNorm of a sub-block boundary runs in the epilogue of the GEMM that produces
-  // the sub-block output (proj -> norm_cross, cross proj -> norm2, fc2 -> the NEXT layer's norm1), so `delta` is never
-  // written and the separate resid_ln pass disappears.
-  const bool fuse = use_fused_ln(e, rows, e->dec[0].proj);
-  bool h_is_norm1 = false;   // h already holds norm1(x) of the current layer (fc2 of the previous layer was fused)
+  // Fused, the residual add + LayerNorm of every sub-block boundary runs in the epilogue of the kernel that produces the
+  // sub-block output (proj -> norm_cross, cross proj + MLP -> the next layer's norm1), so `delta` is never written and
+  // h enters every layer after the first as norm1(x). Unfused, every sub-block writes `delta` and resid_ln folds it in.
+  const bool fused = use_fused(e, rows);
+  float* x_c = x + cls_off * D;      // the class-token rows, which alone continue past the last layer's K/V
+  act_t* h_c = h + cls_off * D;
+  act_t* d_c = delta + cls_off * D;
+  act_t* q_c = q + cls_off * D;
+  act_t* o_c = o + cls_off * D;
   for (size_t l = 0; l < L; ++l) {
     DecBlock& b = e->dec[l];
-    const bool first = (l == 0);
-    // In the last layer only row 0 (the class token) of every sequence reaches the head, so after the keys/values of
-    // its self-attention are formed every kernel runs on the P class-token rows alone.
-    const bool tail = e->prune_tail && (l + 1 == L);
+    const bool last = l + 1 == L;
     const act_t* kvl = e->kv.as<act_t>() + l * kv_per_layer;
-    if (!tail) {
-      if (first && e->cache_layer0) {
-        TRY(L_resid_ln(e, x, nullptr, xsrc, xj, n_src, &b.norm_cross, h, P, 1, 1, s, x_off));
-      } else {
-        if (first) TRY(L_resid_ln(e, x, nullptr, xsrc, xj, n_src, &b.norm1, h, P, 1, 1, s, x_off));
-        else if (!h_is_norm1) TRY(L_resid_ln(e, x, delta, nullptr, nullptr, 0, &b.norm1, h, P, 1, 1, s));
+    // ---- self-attention sub-block ----
+    if (l == 0) {
+      // layer 0's self-attention ran once per item (decoder_item_state): gather the pair's item state
+      if (!last) TRY(L_resid_ln(e, x, nullptr, xsrc, xj, n_src, &b.norm_cross, h, P, 1, 1, s, x_off));
+      else TRY(L_resid_ln_rows(e, x_c, nullptr, xsrc + (size_t)n_src * e->Ne * D, xj, &b.norm_cross, h_c, P, s, x_off));
+    } else {
+      if (!fused) TRY(L_resid_ln(e, x, delta, nullptr, nullptr, 0, &b.norm1, h, P, 1, 1, s));
+      if (!last) {
         TRY(L_gemm(e, h, b.qkv, qkv, (int)rows, ACT_NONE, s));
         TRY(L_attn_self(e, qkv, o, P, 1, s));
-        if (fuse) {
+        if (fused) {
           TRY(L_gemm_ln(e, o, b.proj, x, b.norm_cross, h, (int)rows, s));
         } else {
           TRY(L_gemm(e, o, b.proj, delta, (int)rows, ACT_NONE, s));
           TRY(L_resid_ln(e, x, delta, nullptr, nullptr, 0, &b.norm_cross, h, P, 1, 1, s));
         }
-      }
-      TRY(L_gemm(e, h, b.q, q, (int)rows, ACT_NONE, s));
-      TRY(L_attn_cross(e, q, kvl, o, P, n_kv_seq, ci, s));
-      h_is_norm1 = false;
-      if (fuse && l + 1 < L && use_fused_mlp(e, rows, b.cproj, b.fc1, b.fc2)) {
-        // the cross projection, its residual add and norm2, the whole MLP sub-block, its residual add and the next
-        // layer's norm1 in one kernel: neither the intermediate residual rows nor norm2's output nor `hid` is written
-        TRY(L_cproj_mlp_ln(e, o, b.cproj, b.norm2, b.fc1, b.fc2, x, e->dec[l + 1].norm1, h, (int)rows, s));
-        h_is_norm1 = true;
       } else {
-        if (fuse) {
-          TRY(L_gemm_ln(e, o, b.cproj, x, b.norm2, h, (int)rows, s));
-        } else {
-          TRY(L_gemm(e, o, b.cproj, delta, (int)rows, ACT_NONE, s));
-          TRY(L_resid_ln(e, x, delta, nullptr, nullptr, 0, &b.norm2, h, P, 1, 1, s));
-        }
-        if (fuse && l + 1 < L) {
-          TRY(L_gemm(e, h, b.fc1, hid, (int)rows, ACT_GELU, s));
-          TRY(L_gemm_ln(e, hid, b.fc2, x, e->dec[l + 1].norm1, h, (int)rows, s));
-          h_is_norm1 = true;
-        } else {
-          TRY(L_gemm(e, h, b.fc1, hid, (int)rows, ACT_GELU, s));
-          TRY(L_gemm(e, hid, b.fc2, delta, (int)rows, ACT_NONE, s));
-        }
-      }
-    } else {
-      float* x_c = x + cls_off * D;
-      act_t* h_c = h + cls_off * D;
-      act_t* d_c = delta + cls_off * D;
-      act_t* q_c = q + cls_off * D;
-      act_t* o_c = o + cls_off * D;
-      if (first && e->cache_layer0) {
-        // single-layer decoder with the layer-0 cache: gather the class-token rows only
-        TRY(L_resid_ln_rows(e, x_c, nullptr, xsrc + (size_t)n_src * e->Ne * D, xj, &b.norm_cross, h_c, P, s, x_off));
-      } else {
-        if (first) TRY(L_resid_ln(e, x, nullptr, xsrc, xj, n_src, &b.norm1, h, P, 1, 1, s, x_off));
-        else if (!h_is_norm1) TRY(L_resid_ln(e, x, delta, nullptr, nullptr, 0, &b.norm1, h, P, 1, 1, s));
         // keys/values for every token, the query for the class token only (qkv rows: [0,D) q, [D,3D) k|v)
         Linear w_kv = b.qkv; w_kv.w = b.qkv.w + D * D; w_kv.b = b.qkv.b + D; w_kv.out = 2 * (int)D;
         Linear w_q = b.qkv; w_q.out = (int)D;
@@ -580,17 +542,32 @@ static int decode_chunk(vited_engine* e, int P, const int* ci, const int* xj, co
         TRY(L_gemm(e, o_c, b.proj, d_c, P, ACT_NONE, s));
         TRY(L_resid_ln_rows(e, x_c, d_c, nullptr, nullptr, &b.norm_cross, h_c, P, s));
       }
+    }
+    // ---- cross-attention + MLP sub-block ----
+    if (!last) {
+      TRY(L_gemm(e, h, b.q, q, (int)rows, ACT_NONE, s));
+      TRY(L_attn_cross(e, q, kvl, o, P, n_kv_seq, ci, s));
+      if (fused) {
+        // the cross projection, its residual add and norm2, the whole MLP sub-block, its residual add and the next
+        // layer's norm1 in one kernel: neither the intermediate residual rows nor norm2's output nor `hid` is written
+        TRY(L_cproj_mlp_ln(e, o, b.cproj, b.norm2, b.fc1, b.fc2, x, e->dec[l + 1].norm1, h, (int)rows, s));
+      } else {
+        TRY(L_gemm(e, o, b.cproj, delta, (int)rows, ACT_NONE, s));
+        TRY(L_resid_ln(e, x, delta, nullptr, nullptr, 0, &b.norm2, h, P, 1, 1, s));
+        TRY(L_gemm(e, h, b.fc1, hid, (int)rows, ACT_GELU, s));
+        TRY(L_gemm(e, hid, b.fc2, delta, (int)rows, ACT_NONE, s));
+      }
+    } else {
       TRY(L_gemm(e, h_c, b.q, q_c, P, ACT_NONE, s));
       TRY(L_attn_cls(e, q, (int)D, kvl, kvl + D, 2 * (int)D, o, P, 0, n_kv_seq, ci, s));
       TRY(L_gemm(e, o_c, b.cproj, d_c, P, ACT_NONE, s));
       TRY(L_resid_ln_rows(e, x_c, d_c, nullptr, nullptr, &b.norm2, h_c, P, s));
       TRY(L_gemm(e, h_c, b.fc1, hid, P, ACT_GELU, s));
       TRY(L_gemm(e, hid, b.fc2, d_c, P, ACT_NONE, s));
-      h_is_norm1 = false;
     }
   }
-  head.x = x + cls_off * D;
-  head.delta = delta + cls_off * D;
+  head.x = x_c;
+  head.delta = d_c;
   head.ln_w = e->norm.w; head.ln_b = e->norm.b; head.head_w = e->head_w; head.head_b = e->head_b;
   head.P = P; head.D = e->D; head.C = e->C; head.eps = 1e-6f;
   prof_mark(e, "head", 0.0, (double)P * e->D * 6.0, s);
@@ -661,10 +638,6 @@ int vited_set_option(vited_engine* e, int option, int64_t value) {
       VITED_CHECK(value >= 1, "chunk_rows must be positive");
       e->chunk_rows = value;
       return 0;
-    case VITED_OPT_CACHE_LAYER0: e->cache_layer0 = value ? 1 : 0; return 0;
-    case VITED_OPT_PRUNE_TAIL: e->prune_tail = value ? 1 : 0; return 0;
-    case VITED_OPT_FUSE_LN: e->fuse_ln = value ? 1 : 0; return 0;
-    case VITED_OPT_FUSE_MLP: e->fuse_mlp = value ? 1 : 0; return 0;
     case VITED_OPT_KV_BUDGET_MB:
       VITED_CHECK(value >= 1, "kv budget must be positive");
       e->kv_budget_mb = value;

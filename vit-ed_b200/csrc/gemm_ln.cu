@@ -7,11 +7,10 @@
 // (tcgen05.st) while the row statistics are combined, and the normalised fp16 row leaves through TMA stores.
 //
 // Structure = gemm_tc_pair_kernel (cta_group::2, TMA ring, one MMA thread) with N = 384 issued as two N = 192 MMAs per
-// k-step and a full-row epilogue: 4 * CG epilogue warps per CTA, warp (q, c) owns TMEM lane quarter q (32 rows) and
-// column group c of CG; one thread = one row part. Row statistics use the shifted one-pass form (pivot = first element
-// of the row part) and Chan's combination across the CG parts. The library instantiates CG = 2 (192-column halves,
-// 8 warps); CG = 4 (96-column quarters, 16 warps) was measured neutral (profiles/README.md) and is not built.
+// k-step and a full-row epilogue: 8 epilogue warps per CTA, warp (q, c) owns TMEM lane quarter q (32 rows) and the
+// 192-column half c of the row; one thread = one row half. The LayerNorm arithmetic is ln_epilogue.cuh's.
 #include "kernels.h"
+#include "ln_epilogue.cuh"
 
 namespace vited {
 
@@ -22,26 +21,24 @@ constexpr int BK = 64;
 constexpr int LN_N = 384;
 constexpr int NH = 192;        // columns per MMA
 
-template <int CG>
 struct LnCfg {
-  static_assert(CG == 2 || CG == 4, "two or four column groups");
-  static constexpr int kEpiWarps = 4 * CG;
+  static constexpr int kEpiWarps = 8;
   static constexpr int kThreads = 128 + 32 * kEpiWarps;
-  static constexpr int NW = LN_N / CG;                             // columns per epilogue warp: 192 / 96
-  static constexpr int XW = 64 / CG;                               // columns per residual box: 32 / 16
+  static constexpr int NW = LN_N / 2;                              // columns per epilogue warp: 192
+  static constexpr int XW = 32;                                    // columns per residual box
   static constexpr int CHUNKS = NW / XW;                           // residual boxes per warp and tile: 6
-  static constexpr int HW = 128 / CG;                              // columns per pass-2 slab: 64 / 32
+  static constexpr int HW = 64;                                    // columns per pass-2 slab
   static constexpr int SLABS = NW / HW;                            // 3
-  static constexpr int ROWB = XW * 4;                              // bytes per box row (= HW * 2) = swizzle span: 128 / 64
+  static constexpr int ROWB = XW * 4;                              // bytes per box row (= HW * 2) = swizzle span: 128
   static constexpr uint32_t A_BYTES = BM * BK * 2;
   static constexpr uint32_t BH_BYTES = (NH / 2) * BK * 2;          // this CTA's 96 rows of one 192-row weight half
   static constexpr uint32_t STAGE_BYTES = A_BYTES + 2 * BH_BYTES;
   static constexpr int kStages = 3;
-  static constexpr uint32_t XBOX = 32 * ROWB;                      // 32 rows x XW fp32, hardware-swizzled: 4 KB / 2 KB
+  static constexpr uint32_t XBOX = 32 * ROWB;                      // 32 rows x XW fp32, hardware-swizzled: 4 KB
   static constexpr uint32_t X_BYTES = kEpiWarps * 2 * XBOX;        // 64 KB
   static constexpr uint32_t H_BYTES = kEpiWarps * XBOX;            // 32 rows x HW fp16 per warp: 32 KB
   static constexpr uint32_t PARAM_BYTES = 3 * LN_N * 4;
-  static constexpr uint32_t PART_BYTES = CG * BM * 8;               // (mean, M2) of every row part
+  static constexpr uint32_t PART_BYTES = 2 * BM * 8;                // (mean, M2) of every row half
   static constexpr uint32_t BAR_BYTES = 512;
   static constexpr uint32_t SMEM_BYTES = 1024 + kStages * STAGE_BYTES + X_BYTES + H_BYTES + PARAM_BYTES + PART_BYTES + BAR_BYTES;
   static_assert(SMEM_BYTES <= 232448, "shared memory budget");
@@ -55,13 +52,12 @@ __device__ unsigned long long g_ln_trace[3 * 32 * 8];   // [0 = epilogue warp (q
 #define TRL(who, t, ev) do { } while (0)
 #endif
 
-template <int CG>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(LnCfg<CG>::kThreads, 1)
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(LnCfg::kThreads, 1)
 gemm_ln_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                     const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmH,
                     const float* __restrict__ bias, const float* __restrict__ ln_w, const float* __restrict__ ln_b,
                     int M, int K, float eps) {
-  using Cfg = LnCfg<CG>;
+  using Cfg = LnCfg;
   constexpr int kStages = Cfg::kStages;
   constexpr int NW = Cfg::NW, XW = Cfg::XW, CHUNKS = Cfg::CHUNKS, HW = Cfg::HW, ROWB = Cfg::ROWB;
   extern __shared__ uint8_t smem_raw[];
@@ -175,7 +171,7 @@ gemm_ln_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     // ===================== full-row epilogue (both CTAs, own 128 rows) =====================
     const int ew = warp - 4;
     const int q = warp & 3;       // TMEM lane quarter: rows q*32 .. q*32+31 of this CTA's 128
-    const int c = ew >> 2;        // column group: columns [c * NW, (c + 1) * NW)
+    const int c = ew >> 2;        // row half: columns [c * NW, (c + 1) * NW)
     uint8_t* xbox = sX + ew * 2 * Cfg::XBOX;
     uint8_t* hbox = sH + ew * Cfg::XBOX;
     uint64_t* my_xfull = xfull + ew * 2;
@@ -226,31 +222,13 @@ gemm_ln_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
           const uint32_t off = swz_chunk<ROWB>(i, lane) << 4;
           const float4 xv = lds_f4(in_row + off);
           const float4 b4 = lds_f4(bias_a + 16 * i);
-          // packed fp32 pairs: the epilogue passes are issue bound (16 epilogue warps changed nothing), FADD2 / FFMA2
-          // halve their arithmetic instructions
-          float4 v;
-          f2_unpack(f2_add(f2_from_bits(acc[4 * i + 0], acc[4 * i + 1]), f2_add(f2_pack(b4.x, b4.y), f2_pack(xv.x, xv.y))), v.x, v.y);
-          f2_unpack(f2_add(f2_from_bits(acc[4 * i + 2], acc[4 * i + 3]), f2_add(f2_pack(b4.z, b4.w), f2_pack(xv.z, xv.w))), v.z, v.w);
+          const float4 v = ln_resid4(acc + 4 * i, b4, xv);
           sts_f4(out_row + off, v);
           acc[4 * i + 0] = __float_as_uint(v.x); acc[4 * i + 1] = __float_as_uint(v.y);
           acc[4 * i + 2] = __float_as_uint(v.z); acc[4 * i + 3] = __float_as_uint(v.w);
         }
         if (j == 0) c0 = __uint_as_float(acc[0]);
-        {
-          uint64_t s2[2] = {0ull, 0ull}, q2[2] = {0ull, 0ull};                 // four independent chains each
-          const uint64_t nc0 = f2_dup(-c0);
-#pragma unroll
-          for (int i = 0; i < XW / 2; ++i) {
-            const uint64_t d = f2_add(f2_from_bits(acc[2 * i], acc[2 * i + 1]), nc0);
-            s2[i & 1] = f2_add(s2[i & 1], d);
-            q2[i & 1] = f2_fma(d, d, q2[i & 1]);
-          }
-          float s4[4], q4[4];
-          f2_unpack(s2[0], s4[0], s4[1]); f2_unpack(s2[1], s4[2], s4[3]);
-          f2_unpack(q2[0], q4[0], q4[1]); f2_unpack(q2[1], q4[2], q4[3]);
-          s += (s4[0] + s4[1]) + (s4[2] + s4[3]);
-          ss += (q4[0] + q4[1]) + (q4[2] + q4[3]);
-        }
+        ln_accum_stats(acc, c0, s, ss);
         tmem_st_cols(tlane + j * XW, acc);
         fence_proxy_async_smem();
         __syncwarp();                             // every lane has read the in-box and written the out-box
@@ -262,34 +240,10 @@ gemm_ln_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       }
       tmem_st_wait();
       if (who >= 0) TRL(who, t, 2);
-      // ---- combine the CG column groups of every row (Chan): n = NW each ----
-      const float inv_n = 1.f / NW;
-      const float mean_a = c0 + s * inv_n, m2_a = ss - s * s * inv_n;
-      sPart[c * BM + q * 32 + lane] = make_float2(mean_a, m2_a);
-      asm volatile("bar.sync %0, %1;" ::"r"(q + 1), "n"(32 * CG) : "memory");
-      float mean, var;
-      if constexpr (CG == 2) {
-        const float2 o = sPart[(c ^ 1) * BM + q * 32 + lane];
-        const float dm = o.x - mean_a;
-        mean = 0.5f * (mean_a + o.x);
-        var = (m2_a + o.y + dm * dm * (0.5f * NW)) * (1.f / LN_N);
-      } else {
-        float mg[CG], m2 = 0.f, msum = 0.f;
-#pragma unroll
-        for (int k = 0; k < CG; ++k) {
-          const float2 o = sPart[k * BM + q * 32 + lane];
-          mg[k] = o.x;
-          m2 += o.y;
-          msum += o.x;
-        }
-        mean = msum * (1.f / CG);
-        float between = 0.f;
-#pragma unroll
-        for (int k = 0; k < CG; ++k) between = fmaf(mg[k] - mean, mg[k] - mean, between);
-        var = (m2 + between * (float)NW) * (1.f / LN_N);
-      }
-      const float rstd = rsqrtf(fmaxf(var, 0.f) + eps);
-      const uint64_t nmean2 = f2_dup(-mean), rstd2 = f2_dup(rstd);
+      // ---- combine the two row halves (the q-th pair of warps meets at named barrier q + 1) ----
+      uint64_t nmean2, rstd2;
+      ln_row_stats<NW, 64>(&sPart[c * BM + q * 32 + lane], &sPart[(c ^ 1) * BM + q * 32 + lane], q + 1, s, ss, c0, eps,
+                           nmean2, rstd2);
       if (who >= 0) TRL(who, t, 3);
       // ---- pass 2: normalise out of TMEM, fp16, HW-column slabs through the warp's staging box ----
       const uint32_t hbox_a = smem_u32(hbox) + lane * ROWB, g_a = smem_u32(sG), bt_a = smem_u32(sBt);
@@ -311,23 +265,9 @@ gemm_ln_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
             if (lane == 0) mbar_arrive_leader(tempty);
           }
 #pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            const float4 g0 = lds_f4(g_a + col0 * 4 + 32 * i);
-            const float4 g1v = lds_f4(g_a + col0 * 4 + 32 * i + 16);
-            const float4 t0 = lds_f4(bt_a + col0 * 4 + 32 * i);
-            const float4 t1 = lds_f4(bt_a + col0 * 4 + 32 * i + 16);
-            float y[8];
-            f2_unpack(f2_fma(f2_mul(f2_add(f2_from_bits(v[8 * i + 0], v[8 * i + 1]), nmean2), rstd2), f2_pack(g0.x, g0.y), f2_pack(t0.x, t0.y)), y[0], y[1]);
-            f2_unpack(f2_fma(f2_mul(f2_add(f2_from_bits(v[8 * i + 2], v[8 * i + 3]), nmean2), rstd2), f2_pack(g0.z, g0.w), f2_pack(t0.z, t0.w)), y[2], y[3]);
-            f2_unpack(f2_fma(f2_mul(f2_add(f2_from_bits(v[8 * i + 4], v[8 * i + 5]), nmean2), rstd2), f2_pack(g1v.x, g1v.y), f2_pack(t1.x, t1.y)), y[4], y[5]);
-            f2_unpack(f2_fma(f2_mul(f2_add(f2_from_bits(v[8 * i + 6], v[8 * i + 7]), nmean2), rstd2), f2_pack(g1v.z, g1v.w), f2_pack(t1.z, t1.w)), y[6], y[7]);
-            uint4 pk;
-            pk.x = pack_act(y[0], y[1]);
-            pk.y = pack_act(y[2], y[3]);
-            pk.z = pack_act(y[4], y[5]);
-            pk.w = pack_act(y[6], y[7]);
-            sts_u4(hbox_a + (swz_chunk<ROWB>(hh * 4 + i, lane) << 4), pk);
-          }
+          for (int i = 0; i < 4; ++i)
+            sts_u4(hbox_a + (swz_chunk<ROWB>(hh * 4 + i, lane) << 4),
+                   ln_normalise8(v + 8 * i, g_a + col0 * 4 + 32 * i, bt_a + col0 * 4 + 32 * i, nmean2, rstd2));
         }
         fence_proxy_async_smem();
         __syncwarp();
@@ -362,12 +302,12 @@ int gemm_resid_ln(const act_t* A, const act_t* W, const float* bias, float* x, c
   VITED_CHECK(gemm_resid_ln_supported(M, N, K), "gemm_resid_ln: unsupported shape M=%d N=%d K=%d (N must be 384)", M, N, K);
   VITED_CHECK(((reinterpret_cast<uintptr_t>(A) | reinterpret_cast<uintptr_t>(W) | reinterpret_cast<uintptr_t>(x) |
                 reinterpret_cast<uintptr_t>(h)) & 15) == 0, "gemm_resid_ln: operands must be 16-byte aligned");
-  using Cfg = LnCfg<2>;
+  using Cfg = LnCfg;
   const int sms = gemm_num_sms();
   VITED_CHECK(sms >= 2, "gemm_resid_ln: no device");
   static PerDeviceOnce once;
   if (once.first())
-    VITED_CUDA_OK(cudaFuncSetAttribute(gemm_ln_pair_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    VITED_CUDA_OK(cudaFuncSetAttribute(gemm_ln_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)Cfg::SMEM_BYTES));
   CUtensorMap tA, tB, tX, tH;
   if (make_tmap_act_2d(&tA, A, (uint64_t)K, (uint64_t)M, (uint64_t)K * 2, 64, BM, 128)) return 1;
@@ -377,8 +317,7 @@ int gemm_resid_ln(const act_t* A, const act_t* W, const float* bias, float* x, c
   const int tiles = (M + 2 * BM - 1) / (2 * BM);
   int pairs = sms / 2;
   if (pairs > tiles) pairs = tiles;
-  gemm_ln_pair_kernel<2><<<2 * pairs, Cfg::kThreads, Cfg::SMEM_BYTES, stream>>>(tA, tB, tX, tH, bias, ln_w, ln_b, M, K,
-                                                                                  eps);
+  gemm_ln_pair_kernel<<<2 * pairs, Cfg::kThreads, Cfg::SMEM_BYTES, stream>>>(tA, tB, tX, tH, bias, ln_w, ln_b, M, K, eps);
   VITED_CUDA_OK(cudaGetLastError());
   return 0;
 }

@@ -12,15 +12,12 @@
 //     O += P_c W2_c^T (M 256, N 2 x 192, K 64) into the 384-column output accumulator;
 //   * issue order G1(0) G1(1) | G2(c) G1(c+2) ...: the tensor pipe runs fc1 of chunk c+1 while the GELU warps work on
 //     chunk c; the weight chunks (W1_c: 64 x 384, W2_c: 384 x 64) stream from L2 through a ring of 12-KB slots;
-//   * the full-row epilogue of gemm_ln.cu (residual tile through TMA boxes, updated row parked in TMEM, shifted one-pass
-//     statistics, Chan combination of the two column halves, normalise, TMA stores) runs on the same eight warps. Its
-//     residual boxes live in the h-tile region, which is dead once fc1 of the last chunk has completed.
+//   * the full-row epilogue of gemm_ln.cu (residual tile through TMA boxes, updated row parked in TMEM, the LayerNorm
+//     arithmetic of ln_epilogue.cuh, TMA stores) runs on the same eight warps. Its residual boxes live in the h-tile
+//     region, which is dead once fc1 of the last chunk has completed.
 // TMEM: O = columns [0, 384), S buffers [384, 448) and [448, 512). Shared memory: 96 KB h tile / residual boxes,
-// 96 KB weight ring, 16 KB output staging, biases / LayerNorm parameters.
-// Template parameter CG = column groups of the GELU / epilogue warps. The library instantiates CG = 2 (8 warps: 32 hidden
-// columns of a chunk and a 192-column half row each). CG = 4 (16 warps: 16 hidden columns and a 96-column quarter row
-// each, residual boxes of half the width, weight ring of 6 slots, 32 KB staging) was measured neutral
-// (profiles/README.md) and is not built.
+// 96 KB weight ring, 16 KB output staging, biases / LayerNorm parameters. GELU / epilogue warp (q, c) owns TMEM lane
+// quarter q, 32 hidden columns of a chunk and the 192-column half c of the output row.
 //
 // Template parameter PRO adds the cross-attention projection in front (cproj_mlp_resid_ln, the decoder's
 //     x_mid = x + o W_cproj^T + b_cproj;  h = norm2(x_mid);  then the MLP sub-block above on h and x_mid):
@@ -34,6 +31,7 @@
 //   * fc2 accumulates onto the parked 2 x_mid (the hidden operands are 2 GELU), so the epilogue's v = 0.5 O + b2 needs
 //     no residual read: x_mid and h never reach global memory.
 #include "kernels.h"
+#include "ln_epilogue.cuh"
 
 namespace vited {
 
@@ -46,26 +44,24 @@ constexpr int NH = 192;          // columns per fc2 MMA
 constexpr int HC = 64;           // hidden units per chunk
 constexpr int KB1 = LN_N / BK;   // k-blocks of fc1 (K = 384)
 
-template <int CG>
 struct MlpCfg {
-  static_assert(CG == 2 || CG == 4, "two or four column groups");
-  static constexpr int kEpiWarps = 4 * CG;
+  static constexpr int kEpiWarps = 8;
   static constexpr int kThreads = 128 + 32 * kEpiWarps;
-  static constexpr int NW = LN_N / CG;                                // output columns per epilogue warp: 192 / 96
-  static constexpr int XW = 64 / CG;                                  // columns per residual box: 32 / 16
+  static constexpr int NW = LN_N / 2;                                 // output columns per epilogue warp: 192
+  static constexpr int XW = 32;                                       // columns per residual box
   static constexpr int CHUNKS = NW / XW;                              // residual boxes per warp and tile: 6
-  static constexpr int ROWB = XW * 4;                                 // bytes per residual-box row = swizzle span: 128 / 64
-  static constexpr int GW = HC / CG;                                  // hidden columns of a chunk per GELU warp: 32 / 16
+  static constexpr int ROWB = XW * 4;                                 // bytes per residual-box row = swizzle span: 128
+  static constexpr int GW = HC / 2;                                   // hidden columns of a chunk per GELU warp: 32
   static constexpr uint32_t A_KB_BYTES = BM * BK * 2;                 // one k-block of the h tile: 128 rows x 128 B
   static constexpr uint32_t A_BYTES = KB1 * A_KB_BYTES;               // 96 KB
   static constexpr uint32_t SLOT_BYTES = 12288;                       // 3 k-blocks of W1 (32 rows each) or 96 rows of W2
   // 6 slots left the issuer waiting for weights 11.6 k of 63 k cycles per tile (trace), 8 changed nothing in the step:
-  // the issuer runs ahead of the tensor pipe by the ring depth. The 16-warp form needs the 24 KB for its staging boxes.
-  static constexpr int kSlots = CG == 2 ? 8 : 6;
+  // the issuer runs ahead of the tensor pipe by the ring depth.
+  static constexpr int kSlots = 8;
   static constexpr uint32_t W1_KB_BYTES = (HC / 2) * BK * 2;          // this CTA's 32 rows of one k-block: 4 KB
-  static constexpr uint32_t XBOX = 32 * ROWB;                         // 32 rows x XW fp32, hardware-swizzled: 4 KB / 2 KB
+  static constexpr uint32_t XBOX = 32 * ROWB;                         // 32 rows x XW fp32, hardware-swizzled: 4 KB
   static constexpr uint32_t OUT_BYTES = kEpiWarps * 2048;             // pass-2 staging: 32 rows x 32 fp16 per warp (64B swizzle)
-  static constexpr uint32_t PART_BYTES = CG * BM * 8;                 // (mean, M2) of every row part
+  static constexpr uint32_t PART_BYTES = 2 * BM * 8;                  // (mean, M2) of every row half
   static constexpr uint32_t BAR_BYTES = 512;
   static_assert(kEpiWarps * 3 * XBOX == A_BYTES, "the residual boxes (2 in + 1 out per warp) reuse the h-tile region");
   static_assert((2 * kSlots + 9 + 2 * kEpiWarps + 3) * 8 <= BAR_BYTES, "barrier block");
@@ -91,15 +87,15 @@ __device__ long long g_mlp_trace2[32 * 8];      // pass-1 breakdown of epilogue 
 #define TRM_CLK() 0ll
 #endif
 
-template <int CG, bool PRO>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MlpCfg<CG>::kThreads, 1)
+template <bool PRO>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MlpCfg::kThreads, 1)
 mlp_ln_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmWp,
                    const __grid_constant__ CUtensorMap tmW1, const __grid_constant__ CUtensorMap tmW2,
                    const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmH,
                    const float* __restrict__ bproj, const float* __restrict__ ln2_w, const float* __restrict__ ln2_b,
                    const float* __restrict__ b1, const float* __restrict__ b2, const float* __restrict__ ln_w,
                    const float* __restrict__ ln_b, int M, int hidden, float eps) {
-  using Cfg = MlpCfg<CG>;
+  using Cfg = MlpCfg;
   constexpr int kSlots = Cfg::kSlots;
   constexpr int NW = Cfg::NW, XW = Cfg::XW, CHUNKS = Cfg::CHUNKS, ROWB = Cfg::ROWB, GW = Cfg::GW;
   extern __shared__ uint8_t smem_raw[];
@@ -373,7 +369,7 @@ mlp_ln_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
     // (both CTAs, own 128 rows)
     const int ew = warp - 4;
     const int q = warp & 3;       // TMEM lane quarter: rows q*32 .. q*32+31 of this CTA's 128
-    const int c = ew >> 2;        // column group (of a hidden chunk: GW of 64; of the output row: NW of 384)
+    const int c = ew >> 2;        // column half (of a hidden chunk: GW of 64; of the output row: NW of 384)
     uint8_t* xbox = sA + ew * 3 * Cfg::XBOX;             // two in-boxes, then the out-box
     uint8_t* obox = xbox + 2 * Cfg::XBOX;
     uint8_t* hbox = sOut + ew * 2048;
@@ -383,73 +379,8 @@ mlp_ln_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
     const uint32_t tS = tmem_base + lane_off + kColS + c * GW;
     uint32_t sfull_ph = 0;        // bit b: parity of the next s_full[b] phase
     int g = 0;                    // residual boxes issued / consumed so far (2-deep per warp)
-    // shifted one-pass statistics of one chunk of this lane's row part (pivot c0 = the part's first element)
-    auto accum_stats = [&](const uint32_t (&acc)[XW], float c0, float& s, float& ss) {
-      uint64_t s2[2] = {0ull, 0ull}, q2[2] = {0ull, 0ull};                 // four independent chains each
-      const uint64_t nc0 = f2_dup(-c0);
-#pragma unroll
-      for (int i = 0; i < XW / 2; ++i) {
-        const uint64_t d = f2_add(f2_from_bits(acc[2 * i], acc[2 * i + 1]), nc0);
-        s2[i & 1] = f2_add(s2[i & 1], d);
-        q2[i & 1] = f2_fma(d, d, q2[i & 1]);
-      }
-      float s4[4], q4[4];
-      f2_unpack(s2[0], s4[0], s4[1]); f2_unpack(s2[1], s4[2], s4[3]);
-      f2_unpack(q2[0], q4[0], q4[1]); f2_unpack(q2[1], q4[2], q4[3]);
-      s += (s4[0] + s4[1]) + (s4[2] + s4[3]);
-      ss += (q4[0] + q4[1]) + (q4[2] + q4[3]);
-    };
-    // combine the CG column groups of every row (Chan): n = NW each. all_warps: exchange over every epilogue warp of
-    // the CTA (the prologue: afterwards no warp reads its residual boxes any more) instead of the CG warps of quarter q
-    auto row_stats = [&](float s, float ss, float c0, bool all_warps, uint64_t& nmean2, uint64_t& rstd2) {
-      const float inv_n = 1.f / NW;
-      const float mean_a = c0 + s * inv_n, m2_a = ss - s * s * inv_n;
-      sPart[c * BM + q * 32 + lane] = make_float2(mean_a, m2_a);
-      if (all_warps) asm volatile("bar.sync 5, %0;" ::"n"(32 * Cfg::kEpiWarps) : "memory");
-      else asm volatile("bar.sync %0, %1;" ::"r"(q + 1), "n"(32 * CG) : "memory");
-      float mean, var;
-      if constexpr (CG == 2) {
-        const float2 o = sPart[(c ^ 1) * BM + q * 32 + lane];
-        const float dm = o.x - mean_a;
-        mean = 0.5f * (mean_a + o.x);
-        var = (m2_a + o.y + dm * dm * (0.5f * NW)) * (1.f / LN_N);
-      } else {
-        float mg[CG], m2 = 0.f, msum = 0.f;
-#pragma unroll
-        for (int k = 0; k < CG; ++k) {
-          const float2 o = sPart[k * BM + q * 32 + lane];
-          mg[k] = o.x;
-          m2 += o.y;
-          msum += o.x;
-        }
-        mean = msum * (1.f / CG);
-        float between = 0.f;
-#pragma unroll
-        for (int k = 0; k < CG; ++k) between = fmaf(mg[k] - mean, mg[k] - mean, between);
-        var = (m2 + between * (float)NW) * (1.f / LN_N);
-      }
-      const float rstd = rsqrtf(fmaxf(var, 0.f) + eps);
-      nmean2 = f2_dup(-mean);
-      rstd2 = f2_dup(rstd);
-    };
-    // 8 normalised 16-bit values of columns [col, col + 8) (g_a / bt_a: shared-window address of column col's parameters)
-    auto normalise8 = [&](const uint32_t* v, uint32_t g_a, uint32_t bt_a, uint64_t nmean2, uint64_t rstd2) {
-      const float4 g0 = lds_f4(g_a);
-      const float4 g1v = lds_f4(g_a + 16);
-      const float4 t0 = lds_f4(bt_a);
-      const float4 t1 = lds_f4(bt_a + 16);
-      float y[8];
-      f2_unpack(f2_fma(f2_mul(f2_add(f2_from_bits(v[0], v[1]), nmean2), rstd2), f2_pack(g0.x, g0.y), f2_pack(t0.x, t0.y)), y[0], y[1]);
-      f2_unpack(f2_fma(f2_mul(f2_add(f2_from_bits(v[2], v[3]), nmean2), rstd2), f2_pack(g0.z, g0.w), f2_pack(t0.z, t0.w)), y[2], y[3]);
-      f2_unpack(f2_fma(f2_mul(f2_add(f2_from_bits(v[4], v[5]), nmean2), rstd2), f2_pack(g1v.x, g1v.y), f2_pack(t1.x, t1.y)), y[4], y[5]);
-      f2_unpack(f2_fma(f2_mul(f2_add(f2_from_bits(v[6], v[7]), nmean2), rstd2), f2_pack(g1v.z, g1v.w), f2_pack(t1.z, t1.w)), y[6], y[7]);
-      uint4 pk;
-      pk.x = pack_act(y[0], y[1]);
-      pk.y = pack_act(y[2], y[3]);
-      pk.z = pack_act(y[4], y[5]);
-      pk.w = pack_act(y[6], y[7]);
-      return pk;
-    };
+    float2* part_mine = &sPart[c * BM + q * 32 + lane];
+    const float2* part_other = &sPart[(c ^ 1) * BM + q * 32 + lane];
     for (int t = 0; t < my_tiles; ++t) {
       const int tile = pair + t * num_pairs;
       const int row0 = tile * 2 * BM + (int)rank * BM + q * 32;
@@ -479,16 +410,14 @@ mlp_ln_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
           for (int i = 0; i < XW / 4; ++i) {
             const float4 xv = lds_f4(in_row + (swz_chunk<ROWB>(i, lane) << 4));
             const float4 b4 = lds_f4(bias_a + 16 * i);
-            float4 v;
-            f2_unpack(f2_add(f2_from_bits(acc[4 * i + 0], acc[4 * i + 1]), f2_add(f2_pack(b4.x, b4.y), f2_pack(xv.x, xv.y))), v.x, v.y);
-            f2_unpack(f2_add(f2_from_bits(acc[4 * i + 2], acc[4 * i + 3]), f2_add(f2_pack(b4.z, b4.w), f2_pack(xv.z, xv.w))), v.z, v.w);
+            const float4 v = ln_resid4(acc + 4 * i, b4, xv);
             acc[4 * i + 0] = __float_as_uint(v.x); acc[4 * i + 1] = __float_as_uint(v.y);
             acc[4 * i + 2] = __float_as_uint(v.z); acc[4 * i + 3] = __float_as_uint(v.w);
           }
           __syncwarp();                           // every lane has read the in-box: refill it
           if (lane == 0 && j + 2 < CHUNKS) issue_x(j + 2, g + 2);
           if (j == 0) c0 = __uint_as_float(acc[0]);
-          accum_stats(acc, c0, s, ss);
+          ln_accum_stats(acc, c0, s, ss);
 #pragma unroll
           for (int i = 0; i < XW / 2; ++i) {      // park 2 x_mid (exact): fc2 accumulates onto it
             float lo, hi;
@@ -499,8 +428,9 @@ mlp_ln_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
           tmem_st_cols(tlane + j * XW, acc);
         }
         tmem_st_wait();
+        // (exchanged over every epilogue warp of the CTA: afterwards no warp reads its residual boxes any more)
         uint64_t nmean2, rstd2;
-        row_stats(s, ss, c0, true, nmean2, rstd2);
+        ln_row_stats<NW, 32 * Cfg::kEpiWarps>(part_mine, part_other, 5, s, ss, c0, eps, nmean2, rstd2);
         // ---- prologue pass 2: h = norm2(0.5 park) as 16-bit values straight into the h tile: row r of k-block kb at
         //      kb * 16 KB + r * 128 B, 16-byte chunk i at i ^ (r & 7) (the 128B swizzle fc1's descriptor reads) ----
         const uint32_t h_row = smem_u32(sA) + (uint32_t)(q * 32 + lane) * 128;
@@ -521,8 +451,8 @@ mlp_ln_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
 #pragma unroll
           for (int i = 0; i < 4; ++i)
             sts_u4(dst + (swz_chunk<128>((col0 % BK) / 8 + i, lane) << 4),
-                   normalise8(v + 8 * i, smem_u32(sG2) + (col0 + 8 * i) * 4, smem_u32(sBt2) + (col0 + 8 * i) * 4, nmean2,
-                              rstd2));
+                   ln_normalise8(v + 8 * i, smem_u32(sG2) + (col0 + 8 * i) * 4, smem_u32(sBt2) + (col0 + 8 * i) * 4, nmean2,
+                                 rstd2));
         }
         fence_proxy_async_smem();                 // the h tile is read by the tensor core (async proxy)
         tc_fence_before();
@@ -602,8 +532,6 @@ mlp_ln_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
         for (int i = 0; i < XW / 4; ++i) {
           const uint32_t off = swz_chunk<ROWB>(i, lane) << 4;
           const float4 b4 = lds_f4(bias_a + 16 * i);
-          // packed fp32 pairs: the epilogue passes are issue bound (16 epilogue warps changed nothing), FADD2 / FFMA2
-          // halve their arithmetic instructions
           float4 v;
           if constexpr (PRO) {
             f2_unpack(f2_fma(f2_from_bits(acc[4 * i + 0], acc[4 * i + 1]), f2_dup(0.5f), f2_pack(b4.x, b4.y)), v.x, v.y);
@@ -619,7 +547,7 @@ mlp_ln_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
         }
         if (j == 0) c0 = __uint_as_float(acc[0]);
         const long long k3 = TRM_CLK(); (void)k3;
-        accum_stats(acc, c0, s, ss);
+        ln_accum_stats(acc, c0, s, ss);
         const long long k4 = TRM_CLK(); (void)k4;
         tmem_st_cols(tlane + j * XW, acc);
         fence_proxy_async_smem();
@@ -644,7 +572,7 @@ mlp_ln_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
         mbar_arrive(a_free);
       }
       uint64_t nmean2, rstd2;
-      row_stats(s, ss, c0, false, nmean2, rstd2);
+      ln_row_stats<NW, 64>(part_mine, part_other, q + 1, s, ss, c0, eps, nmean2, rstd2);
       // ---- pass 2: normalise out of TMEM, fp16, 32-column chunks through the warp's staging box (64B-swizzled rows) ----
       const uint32_t hbox_a = smem_u32(hbox) + lane * 64, g_a = smem_u32(sG), bt_a = smem_u32(sBt);
       auto normalise_chunk = [&](const uint32_t (&v)[32], int j) {
@@ -654,7 +582,7 @@ mlp_ln_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
 #pragma unroll
         for (int i = 0; i < 4; ++i)
           sts_u4(hbox_a + (swz_chunk<64>(i, lane) << 4),
-                 normalise8(v + 8 * i, g_a + col0 * 4 + 32 * i, bt_a + col0 * 4 + 32 * i, nmean2, rstd2));
+                 ln_normalise8(v + 8 * i, g_a + col0 * 4 + 32 * i, bt_a + col0 * 4 + 32 * i, nmean2, rstd2));
         fence_proxy_async_smem();
         __syncwarp();
         if (lane == 0) {
@@ -679,7 +607,7 @@ mlp_ln_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
       }
       if (ew == 0) TRM(0, t, 4, TRM_CLK());
       // the sPart exchange of the next tile must not overtake a slow partner still reading this tile's entry
-      asm volatile("bar.sync %0, %1;" ::"r"(q + 1), "n"(32 * CG) : "memory");
+      asm volatile("bar.sync %0, %1;" ::"r"(q + 1), "n"(64) : "memory");
     }
     if (lane == 0) tma_store_wait_all();
   }
@@ -700,7 +628,7 @@ bool mlp_resid_ln_supported(int M, int D, int hidden) {
 }
 
 bool cproj_mlp_resid_ln_supported(int M, int D, int K, int hidden) {
-  return mlp_resid_ln_supported(M, D, hidden) && K == D && MlpCfg<2>::smem_bytes(hidden, true) <= 232448;
+  return mlp_resid_ln_supported(M, D, hidden) && K == D && MlpCfg::smem_bytes(hidden, true) <= 232448;
 }
 
 // PRO: a_in = o and Wp / bproj / ln2_* the cross projection and norm2; otherwise a_in = h and those are unused
@@ -708,7 +636,7 @@ template <bool PRO>
 static int mlp_ln_launch(const act_t* a_in, const act_t* Wp, const float* bproj, const float* ln2_w, const float* ln2_b,
                          const act_t* W1, const float* b1, const act_t* W2, const float* b2, float* x, const float* ln_w,
                          const float* ln_b, act_t* h_out, int M, int D, int hidden, float eps, cudaStream_t stream) {
-  using Cfg = MlpCfg<2>;
+  using Cfg = MlpCfg;
   const char* name = PRO ? "cproj_mlp_resid_ln" : "mlp_resid_ln";
   const int sms = gemm_num_sms();
   VITED_CHECK(sms >= 2, "%s: no device", name);
@@ -716,7 +644,7 @@ static int mlp_ln_launch(const act_t* a_in, const act_t* Wp, const float* bproj,
   VITED_CHECK(smem <= 232448, "%s: hidden=%d needs %u bytes of shared memory", name, hidden, smem);
   static PerDeviceOnce once;
   if (once.first())
-    VITED_CUDA_OK(cudaFuncSetAttribute(mlp_ln_pair_kernel<2, PRO>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
+    VITED_CUDA_OK(cudaFuncSetAttribute(mlp_ln_pair_kernel<PRO>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
   CUtensorMap tA, tWp, tW1, tW2, tX, tH;
   if (make_tmap_act_2d(&tA, a_in, (uint64_t)D, (uint64_t)M, (uint64_t)D * 2, 64, BM, 128)) return 1;
   if (make_tmap_act_2d(&tW1, W1, (uint64_t)D, (uint64_t)hidden, (uint64_t)D * 2, 64, HC / 2, 128)) return 1;
@@ -731,7 +659,7 @@ static int mlp_ln_launch(const act_t* a_in, const act_t* Wp, const float* bproj,
   const int tiles = (M + 2 * BM - 1) / (2 * BM);
   int pairs = sms / 2;
   if (pairs > tiles) pairs = tiles;
-  mlp_ln_pair_kernel<2, PRO><<<2 * pairs, Cfg::kThreads, smem, stream>>>(tA, tWp, tW1, tW2, tX, tH, bproj, ln2_w, ln2_b,
+  mlp_ln_pair_kernel<PRO><<<2 * pairs, Cfg::kThreads, smem, stream>>>(tA, tWp, tW1, tW2, tX, tH, bproj, ln2_w, ln2_b,
                                                                           b1, b2, ln_w, ln_b, M, hidden, eps);
   VITED_CUDA_OK(cudaGetLastError());
   return 0;

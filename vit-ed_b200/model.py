@@ -254,7 +254,7 @@ class VisionTransformerCustom(nn.Module):
             pass
 
     def set_option(self, option, value):
-        """Engine knobs (debug kernels, chunk rows, layer-0 caching); see include/vited_b200.h."""
+        """Engine knobs (debug kernels, chunk rows, memory budgets, profiling); see include/vited_b200.h."""
         if self._engine is None:
             self._ensure_engine(next(self.parameters()).device)
         _lib.check(_lib.lib.vited_set_option(self._engine, int(option), int(value)), 'vited_set_option')
