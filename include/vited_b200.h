@@ -247,6 +247,17 @@ VITED_API int vited_train_attention_chk(int backward, const void* q, int q_ld, c
  * int32 after it is a sticky flag set to 1 when that value is non-finite. */
 VITED_API int vited_train_grad_norm(const int64_t* table, int n_tensors, double* partials, int n_partials,
                                     float* out_sumsq_and_flag, void* stream);
+/* replaces: the inf that an overflowing fp16 autocast gradient carries into p.grad, where torch.amp.GradScaler finds it.
+ * table: the layout of vited_train_grad_norm ((pointer to f32, numel) per tensor, on the device). If *flag (device
+ * int32, e.g. the one the range checks set) is non-zero, element 0 of every tensor with numel > 0 is set to +inf;
+ * otherwise nothing is written. No host read of the flag. */
+VITED_API int vited_train_mark_overflow(const int64_t* table, int n_tensors, const int32_t* flag, void* stream);
+/* replaces: the images gradient of Conv2d(kernel = stride = p) in timm PatchEmbed (vision_transformer.py:383, :391).
+ * dcol [B * (S/p)^2, C*p*p] f32 (the dgrad of the patch-embedding GEMM, rows and columns as vited_op_im2col writes
+ * them) -> dimages [B, C, S, S] f32: the inverse permutation of vited_op_im2col. The patches do not overlap, so every
+ * element of dimages is written exactly once (overwritten, not accumulated). p % 4 == 0, S % p == 0, both pointers
+ * 16-byte aligned. */
+VITED_API int vited_train_col2im(const float* dcol, float* dimages, int B, int C, int S, int p, void* stream);
 /* replaces: optimizer.step() of torch.optim.AdamW (misc/optimizer.py:12-46) after clip_grad_norm_.
  * table [n_tensors, 6] int64 on the device: (param, grad, exp_avg, exp_avg_sq pointers (f32, numel elements each),
  * numel, weight decay as the bit pattern of a double) per tensor; max_numel = the largest numel. One step of the

@@ -91,6 +91,8 @@ SIGNATURES = {
     "vited_train_attention_chk": (_i, [_i, _vp, _i, _vp, _i, _vp, _i, _vp, _i, _vp, _vp, _i, _vp, _vp, _i, _vp, _i, _vp, _i, _i,
                                        _i, _i, _i, _i, _f, _vp, _vp]),
     "vited_train_grad_norm": (_i, [_vp, _i, _vp, _i, _vp, _vp]),
+    "vited_train_mark_overflow": (_i, [_vp, _i, _vp, _vp]),
+    "vited_train_col2im": (_i, [_vp, _vp, _i, _i, _i, _i, _vp]),
     "vited_train_adamw": (_i, [_vp, _i, _i64, _d, _d, _d, _d, _f, _d, _d, _vp]),
     "vited_op_gemm": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
     "vited_op_gemm_resid_ln": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _f, _vp]),

@@ -1172,6 +1172,12 @@ int vited_train_grad_norm(const int64_t* table, int n_tensors, double* partials,
                           void* stream) {
   return train_grad_norm(table, n_tensors, partials, n_partials, out_sumsq_and_flag, (cudaStream_t)stream);
 }
+int vited_train_mark_overflow(const int64_t* table, int n_tensors, const int32_t* flag, void* stream) {
+  return train_mark_overflow(table, n_tensors, flag, (cudaStream_t)stream);
+}
+int vited_train_col2im(const float* dcol, float* dimages, int B, int C, int S, int p, void* stream) {
+  return train_col2im(dcol, dimages, B, C, S, p, (cudaStream_t)stream);
+}
 int vited_train_adamw(const int64_t* table, int n_tensors, int64_t max_numel, double lr, double beta1, double beta2,
                       double eps, float clip_coef, double bias_correction1, double bias_correction2, void* stream) {
   return train_adamw(table, n_tensors, max_numel, lr, beta1, beta2, eps, clip_coef, bias_correction1, bias_correction2,

@@ -162,6 +162,7 @@ int train_gather_rows(const float* in, const int* idx, float* out, int n_blocks,
                       int in_row_off, int out_block_stride, int out_row_off, int D, int accumulate, cudaStream_t s);
 int train_scatter_add_rows(const float* src, const int* idx, float* dst, int n_blocks, int rows_per, int src_block_stride,
                            int src_row_off, int dst_block_stride, int dst_row_off, int D, float alpha, cudaStream_t s);
+int train_col2im(const float* dcol, float* dimages, int B, int C, int S, int p, cudaStream_t s);
 // flag non-null (backward only): *flag = 1 when a dS value of the tensor-core kernels does not survive its conversion to
 // the 16-bit type (kActRangeLimit); the fp32 SIMT kernels convert nothing and never touch it
 int train_attention(int backward, const act_t* q, int q_ld, const act_t* k, int k_ld, const act_t* v, int v_ld, act_t* o,
@@ -187,6 +188,7 @@ constexpr float kActRangeLimit = 65504.f;
 float train_range_limit();
 int train_range_check(const void* x, int is_f32, int64_t n, float limit, int* flag, cudaStream_t s);
 int train_grad_norm(const int64_t* table, int n_tensors, double* partials, int n_partials, float* out, cudaStream_t s);
+int train_mark_overflow(const int64_t* table, int n_tensors, const int* flag, cudaStream_t s);
 int train_adamw(const int64_t* table, int n_tensors, int64_t max_numel, double lr, double beta1, double beta2, double eps,
                 float clip_coef, double bc1, double bc2, cudaStream_t s);
 int train_bce_logits(const float* logits, const float* labels, int n, float* loss, float* dlogits, float grad_scale,

@@ -203,6 +203,31 @@ __global__ void scatter_add_rows_kernel(const float* __restrict__ src, const int
 }
 
 // ---------------------------------------------------------------------------------------------------------------
+// col2im: the inverse permutation of im2col_kernel (rowops.cu) for Conv2d(kernel = stride = p). Patches do not
+// overlap, so every image element is one column of one patch row and is written once (no atomics). Four consecutive
+// px per thread (p % 4 == 0): a 16-byte load from dcol and a 16-byte store into the image row.
+// ---------------------------------------------------------------------------------------------------------------
+__global__ void col2im_kernel(const float* __restrict__ dcol, float* __restrict__ dimg, int B, int C, int S, int p) {
+  const int G = S / p;
+  const int K = C * p * p;
+  const int segs_per_row = K / 4;
+  const size_t total = (size_t)B * G * G * segs_per_row;
+  for (size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
+    const int seg = (int)(idx % segs_per_row);
+    const size_t row = idx / segs_per_row;
+    const int col = seg * 4;
+    const int c = col / (p * p);
+    const int py = (col / p) % p;
+    const int px = col % p;
+    const int t = (int)(row % (G * G));
+    const size_t b = row / (G * G);
+    const int gy = t / G, gx = t % G;
+    const float4 v = *reinterpret_cast<const float4*>(dcol + row * K + col);
+    *reinterpret_cast<float4*>(dimg + ((b * C + c) * S + (gy * p + py)) * S + gx * p + px) = v;
+  }
+}
+
+// ---------------------------------------------------------------------------------------------------------------
 // softmax attention, plain layout: q row (s, i) at q[(s * Tq + i) * q_ld + h * hd ...], k / v row (s, j) likewise.
 // Three kernels, one warp per row, no atomics and nothing quadratic stored:
 //   forward      (per query row i): p = softmax(q_i K^T * scale), o_i = p V, lse_i = log sum exp
@@ -456,6 +481,17 @@ int train_scatter_add_rows(const float* src, const int* idx, float* dst, int n_b
   if (total == 0) return 0;
   scatter_add_rows_kernel<<<blocks_for(total), kThreads, 0, s>>>(src, idx, dst, n_blocks, rows_per, src_block_stride,
                                                                 src_row_off, dst_block_stride, dst_row_off, D, alpha);
+  VITED_CUDA_OK(cudaGetLastError());
+  return 0;
+}
+int train_col2im(const float* dcol, float* dimages, int B, int C, int S, int p, cudaStream_t s) {
+  VITED_CHECK(B >= 0 && C > 0 && p > 0 && p % 4 == 0 && S % p == 0,
+              "train col2im: patch size %d must be a multiple of 4 and divide img size %d (B %d, C %d)", p, S, B, C);
+  VITED_CHECK((reinterpret_cast<uintptr_t>(dcol) | reinterpret_cast<uintptr_t>(dimages)) % 16 == 0,
+              "train col2im: dcol and dimages must be 16-byte aligned");
+  const size_t total = (size_t)B * (S / p) * (S / p) * (C * p * p / 4);
+  if (total == 0) return 0;
+  col2im_kernel<<<blocks_for(total), kThreads, 0, s>>>(dcol, dimages, B, C, S, p);
   VITED_CUDA_OK(cudaGetLastError());
   return 0;
 }

@@ -90,6 +90,14 @@ __global__ void grad_norm_final_kernel(const double* __restrict__ partials, int 
   }
 }
 
+// element 0 of every (non-empty) tensor of a grad_norm table = +inf when the sticky flag is set: a saturated 16-bit
+// conversion then shows as a non-finite gradient, the only overflow signal torch.amp.GradScaler reads
+__global__ void mark_overflow_kernel(const int64_t* __restrict__ table, int n_tensors, const int* __restrict__ flag) {
+  if (*flag == 0) return;
+  for (int t = blockIdx.x * blockDim.x + threadIdx.x; t < n_tensors; t += gridDim.x * blockDim.x)
+    if (table[t * kNormCols + 1] > 0) *reinterpret_cast<float*>(table[t * kNormCols]) = __int_as_float(0x7f800000);
+}
+
 // torch.optim.AdamW (foreach=False, fused=False, amsgrad=False, maximize=False), per element of every tensor:
 //   p *= 1 - lr * wd                 (Python double, applied as a float scalar; skipped for wd == 0 as torch does)
 //   m.lerp_(g, 1 - beta1)            (torch's lerp: m + w (g - m) for |w| < 0.5, else g - (g - m)(1 - w))
@@ -162,6 +170,14 @@ int train_grad_norm(const int64_t* table, int n_tensors, double* partials, int n
   grad_norm_partial_kernel<<<n_partials, kThreads, 0, s>>>(table, n_tensors, partials);
   VITED_CUDA_OK(cudaGetLastError());
   grad_norm_final_kernel<<<1, 1024, 0, s>>>(partials, n_partials, out);
+  VITED_CUDA_OK(cudaGetLastError());
+  return 0;
+}
+
+int train_mark_overflow(const int64_t* table, int n_tensors, const int* flag, cudaStream_t s) {
+  VITED_CHECK(table && flag && n_tensors >= 0, "train mark overflow: bad arguments (n_tensors %d)", n_tensors);
+  if (n_tensors == 0) return 0;
+  mark_overflow_kernel<<<(n_tensors + kThreads - 1) / kThreads, kThreads, 0, s>>>(table, n_tensors, flag);
   VITED_CUDA_OK(cudaGetLastError());
   return 0;
 }

@@ -5,7 +5,9 @@ Same constructor arguments, same three-mode ``forward`` and same ``state_dict`` 
 models/build.py:15-32), so ``load_pretrained`` (misc/utils.py:48-127) and the callers at evaluation.py:107,
 hisfrag.py:214,229 work unchanged. The parameters are ordinary fp32 ``nn.Parameter``s (that is what a checkpoint
 restores); the arithmetic runs in the sm_100a kernels behind ``include/vited_b200.h``. There is no PyTorch compute
-path: a forward on a non-CUDA tensor, or without the built library, raises.
+path: a forward on a non-CUDA tensor, or without the built library, raises. In training mode with gradients wanted the
+forward modes are torch.autograd Functions on the training kernels (``train.encode`` / ``train.decode``), so the
+reference's training loop works unchanged; see ``forward``.
 """
 import ctypes
 import math
@@ -14,7 +16,7 @@ from functools import partial
 import torch
 import torch.nn as nn
 
-from . import _lib
+from . import _lib, train
 
 
 class _PatchEmbed(nn.Module):
@@ -205,12 +207,15 @@ class VisionTransformerCustom(nn.Module):
     def _param_versions(self):
         return tuple((p.data_ptr(), p._version) for p in self.parameters())
 
-    def _ensure_engine(self, device):
+    def _check_device(self, device):
         if device.type != 'cuda':
             raise _lib.VitedError('vit-ed_b200 runs on CUDA (sm_100a) tensors only; there is no CPU fallback')
         first = next(self.parameters())
         if first.device != device:
             raise _lib.VitedError(f'model parameters are on {first.device}, input is on {device}; call model.cuda()')
+
+    def _ensure_engine(self, device):
+        self._check_device(device)
         index = device.index if device.index is not None else torch.cuda.current_device()
         if self._engine is None or self._engine_device != index:
             self._release_engine()
@@ -284,11 +289,36 @@ class VisionTransformerCustom(nn.Module):
         return t.contiguous()
 
     # ------------------------------------------------------------------ reference API
-    @torch.no_grad()
+    _ENCODE_PARAMS = ('patch_embed.proj.', 'pos_embed', 'blocks.')
+    _DECODE_PARAMS = ('patch_embed.proj.', 'cls_token', 'pos_embed', 'cross_blocks.', 'norm.', 'head.')
+
+    def _mode_params(self, prefixes):
+        """(names, parameters) of one forward mode: what the reference's graph of that mode uses."""
+        named = [(n, p) for n, p in self.named_parameters() if n.startswith(prefixes)]
+        return [n for n, _ in named], [p for _, p in named]
+
+    def _differentiable(self, params, *inputs):
+        """A forward runs through torch.autograd (train.encode / train.decode, the training kernels) only when the
+        caller is training: grad mode on, the module in training mode, and a parameter of the mode or a floating-point
+        input requiring grad. Everything else -- eval(), no_grad, inference_mode, frozen parameters -- runs the scoring
+        engine. Train and eval compute the same function here (no dropout, no BatchNorm)."""
+        if not (torch.is_grad_enabled() and self.training):
+            return False
+        return any(p.requires_grad for p in params) or any(t.is_floating_point() and t.requires_grad for t in inputs)
+
     def forward_first_part(self, x1):
         """[B, C, S, S] -> encoder tokens [B, N_e, D] (reference vision_transformer.py:382-388)."""
+        images = x1
         x1 = self._prep(x1)
         self._check_images(x1)
+        names, params = self._mode_params(self._ENCODE_PARAMS)
+        if self._differentiable(params, images):
+            self._check_device(x1.device)
+            return train.encode(self, images, names, params)
+        return self._encode(x1)
+
+    @torch.no_grad()
+    def _encode(self, x1):
         eng = self._ensure_engine(x1.device)
         out = torch.empty((x1.shape[0], self.patch_embed.num_patches, self.embed_dim), dtype=torch.float32,
                           device=x1.device)
@@ -296,29 +326,54 @@ class VisionTransformerCustom(nn.Module):
                    'vited_encode')
         return out
 
-    @torch.no_grad()
     def forward(self, x, x2=None, forward_first_part=False):
-        """Three modes, as reference vision_transformer.py:412-420."""
+        """Three modes, as reference vision_transformer.py:412-420. In training mode with gradients wanted (see
+        ``_differentiable``) each mode is a torch.autograd Function: ``loss.backward()`` reaches the parameters, the
+        context tokens and images that require grad. The backward runs at loss scale 1: the 16-bit gradient operands
+        carry whatever scale the caller applied (torch.amp.GradScaler), and so does ``p.grad``, as under fp16
+        autocast. A 16-bit overflow in the backward shows as +inf in the gradients, where GradScaler looks for it.
+        Like fp16 autocast without a scaler, an fp16 build can underflow small gradients; a bf16 build cannot."""
         if forward_first_part:
             return self.forward_first_part(x)
         if x2 is not None:
+            tokens, images = x, x2
             x = self._prep(x)
             x2 = self._prep(x2)
             self._check_images(x2)
             n_e = self.patch_embed.num_patches
             if x.dim() != 3 or x.shape[1] != n_e or x.shape[2] != self.embed_dim or x.shape[0] != x2.shape[0]:
                 raise ValueError(f'expected context tokens [{x2.shape[0]}, {n_e}, {self.embed_dim}], got {tuple(x.shape)}')
-            eng = self._ensure_engine(x2.device)
-            out = torch.empty((x2.shape[0], self.num_classes), dtype=torch.float32, device=x2.device)
+            self._check_device(x2.device)
             if x.device != x2.device:
                 raise _lib.VitedError(f'context tokens are on {x.device}, images on {x2.device}')
-            _lib.check(_lib.lib.vited_decode(eng, x.data_ptr(), x2.data_ptr(), x2.shape[0], out.data_ptr(),
-                                             self._stream(x2.device)), 'vited_decode')
-            return out
+            names, params = self._mode_params(self._DECODE_PARAMS)
+            if self._differentiable(params, tokens, images):
+                return train.decode(self, tokens, images, names, params)
+            return self._decode(x, x2)
+        pairs = x
         x = self._prep(x)
         if x.dim() != 5 or x.shape[1] != 2:
             raise ValueError(f'expected stacked pairs [B, 2, C, S, S], got {tuple(x.shape)}')
         self._check_images(x[:, 0])
+        if self._differentiable(list(self.parameters()), pairs):
+            self._check_device(x.device)
+            first, second = torch.unbind(pairs, 1)                 # as the reference's forward composes the two parts
+            enc_names, enc_params = self._mode_params(self._ENCODE_PARAMS)
+            dec_names, dec_params = self._mode_params(self._DECODE_PARAMS)
+            tokens = train.encode(self, first, enc_names, enc_params)
+            return train.decode(self, tokens, second, dec_names, dec_params)
+        return self._forward_pairs(x)
+
+    @torch.no_grad()
+    def _decode(self, x, x2):
+        eng = self._ensure_engine(x2.device)
+        out = torch.empty((x2.shape[0], self.num_classes), dtype=torch.float32, device=x2.device)
+        _lib.check(_lib.lib.vited_decode(eng, x.data_ptr(), x2.data_ptr(), x2.shape[0], out.data_ptr(),
+                                         self._stream(x2.device)), 'vited_decode')
+        return out
+
+    @torch.no_grad()
+    def _forward_pairs(self, x):
         eng = self._ensure_engine(x.device)
         out = torch.empty((x.shape[0], self.num_classes), dtype=torch.float32, device=x.device)
         _lib.check(_lib.lib.vited_forward_pairs(eng, x.data_ptr(), x.shape[0], out.data_ptr(), self._stream(x.device)),

@@ -7,7 +7,13 @@ streams only: every arithmetic step is a C-ABI call (include/vited_b200.h, "Hisf
 -- forward, dgrad, wgrad -- run on the tcgen05 GEMM (``vited_op_gemm``) with 16-bit operands; LayerNorm, GELU, softmax
 attention (forward and backward), residual adds, gathers / scatter-adds and the loss run in fp32 kernels of
 csrc/train_ops.cu. Gradients carry a loss scale (default 1024) while they are 16-bit GEMM operands and are unscaled when
-accumulated into the fp32 parameter gradients. There is no PyTorch autograd and no CPU path.
+accumulated into the fp32 parameter gradients. There is no CPU path.
+
+``encode`` / ``decode`` are the same forward and backward sequences as torch.autograd Functions: what
+``VisionTransformerCustom`` runs in training mode, so that ``loss.backward()`` of the caller's own loop reaches the
+parameters (and the context tokens and images that require grad). They run at loss scale 1 -- the incoming gradient
+carries the caller's GradScaler scale -- with every 16-bit conversion range-checked; an overflow is written into the
+returned gradients as +inf (``vited_train_mark_overflow``), where GradScaler finds it.
 
 ``train_iteration`` completes the reference's iteration (misc/engine.py:189-257, misc/utils.py:206-226) on the device:
 the same step with overflow detection for the loss-scaled 16-bit gradients (``LossScaler``, GradScaler's rule),
@@ -406,28 +412,79 @@ def _train_step(model, samples, groups, labels, loss_scale, profile=False, flag=
     if next(iter(sd.values())).device != dev:
         raise _lib.VitedError('model parameters and samples are on different devices; call model.cuda()')
     B = samples.shape[0]
-    D, heads = model.embed_dim, model.num_heads
-    ne = model.patch_embed.num_patches
-    nd = ne + 1
+    D, ne = model.embed_dim, model.patch_embed.num_patches
     P = groups.shape[0]
     g0 = groups[:, 0].to(device=dev, dtype=torch.int32).contiguous()    # image whose decoder state seeds the pair
     g1 = groups[:, 1].to(device=dev, dtype=torch.int32).contiguous()    # image whose encoder tokens are the context
-    zeros_b = torch.zeros(max(B, P), dtype=torch.int32, device=dev)
     y = labels.to(dev).float().contiguous().view(-1)
 
     # ---------------- forward ----------------
-    # patch embedding as an im2col GEMM (timm PatchEmbed; vision_transformer.py:383, :391), shared by both stacks
+    patch, tok32 = _patch_embed_forward(ops, sd, model, samples)          # shared by both stacks
+    enc, enc_out = _encoder_forward(ops, sd, model, tok32, B)
+    dec, logits_pad = _decoder_forward(ops, sd, model, tok32, g0, enc_out, g1)
+    C = model.num_classes
+    logits = logits_pad[:, :C].contiguous()
+    loss = ops.empty(1)
+    dlogits = ops.empty(P * C)
+    yy = y if y.numel() == P * C else y.view(P, 1).expand(P, C).contiguous().view(-1)
+    ops._chk(_lib.lib.vited_train_bce_logits(_p(logits), _p(yy), P * C, _p(loss), _p(dlogits), ops.S, ops.stream),
+             'train_bce_logits')
+
+    # ---------------- backward ----------------
+    dtok = ops.zeros(B * ne, D)
+    dctx = _decoder_backward(ops, sd, model, dec, dlogits.view(P, C), dtok)
+    denc = ops.zeros(B * ne, D)
+    _scatter_add(ops, dctx, g1, P, ne, ne, 0, denc, ne, 0)
+    ops.add_(dtok, _encoder_backward(ops, sd, model, enc, denc))
+    patch.backward(dtok, need_dx=False)
+
+    for name, p in model.named_parameters():
+        g = ops.grads.get(name)
+        p.grad = torch.zeros_like(p) if g is None else g.view_as(p).to(p.dtype)
+    model.train_launches = ops.launches
+    model.train_profile = ops.profile_read() if profile else None   # time between consecutive calls, by entry point
+    return loss[0], logits, groups, labels
+
+
+# ----------------------------------------------------------------------------------------------------------------
+# the forward / backward sequences of the two stacks, shared by train_step and the autograd Functions below
+# ----------------------------------------------------------------------------------------------------------------
+def _zeros_index(n, dev):
+    return torch.zeros(n, dtype=torch.int32, device=dev)
+
+
+def _patch_embed_forward(ops, sd, model, images):
+    """timm PatchEmbed as an im2col GEMM (vision_transformer.py:383, :391): images [B, C, S, S] fp32 contiguous ->
+    (the layer, tokens [B * Ne, D] fp32)."""
+    B = images.shape[0]
     kpe = model.in_chans * model.patch_size ** 2
-    col16 = ops.empty(B * ne, kpe, dtype=ops.act)
-    ops._chk(_lib.lib.vited_op_im2col(_p(samples), _p(col16), B, model.in_chans, model.img_size, model.patch_size, ops.stream),
-             'op_im2col')
+    col16 = ops.empty(B * model.patch_embed.num_patches, kpe, dtype=ops.act)
+    ops._chk(_lib.lib.vited_op_im2col(_p(images), _p(col16), B, model.in_chans, model.img_size, model.patch_size,
+                                      ops.stream), 'op_im2col')
     patch = _Linear(ops, sd, 'patch_embed.proj')
-    tok32 = ops.to_f32(patch.forward(col16))                              # [B * Ne, D]
-    pos32 = sd['pos_embed'].view(nd, D)
-    cls32 = sd['cls_token'].view(1, D)
-    # encoder input: tokens + pos_embed[:, 1:]  (:378-380)
+    return patch, ops.to_f32(patch.forward(col16))
+
+
+def _patch_embed_backward(ops, model, patch, dtok, images_grad):
+    """Accumulates the patch-embedding weight / bias gradients; returns d images [B, C, S, S] fp32 when
+    ``images_grad`` (dgrad on the tcgen05 GEMM, then col2im), else None."""
+    dcol = patch.backward(dtok, need_dx=images_grad)
+    if not images_grad:
+        return None
+    B = dtok.shape[0] // model.patch_embed.num_patches
+    dimg = ops.empty(B, model.in_chans, model.img_size, model.img_size)
+    ops._chk(_lib.lib.vited_train_col2im(_p(dcol), _p(dimg), B, model.in_chans, model.img_size, model.patch_size,
+                                         ops.stream), 'train_col2im')
+    return dimg
+
+
+def _encoder_forward(ops, sd, model, tok32, B):
+    """encoder input tokens + pos_embed[:, 1:] (:378-380), then the blocks -> (the layers, output [B * Ne, D])."""
+    D, heads = model.embed_dim, model.num_heads
+    ne = model.patch_embed.num_patches
+    nd = ne + 1
     x = ops.empty(B * ne, D)
-    _gather(ops, pos32, zeros_b, B, ne, nd, 1, x, ne, 0, False)
+    _gather(ops, sd['pos_embed'].view(nd, D), _zeros_index(B, ops.dev), B, ne, nd, 1, x, ne, 0, False)
     ops.add_(x, tok32)
     enc = []
     for l in range(model.depth):
@@ -435,14 +492,40 @@ def _train_step(model, samples, groups, labels, loss_scale, profile=False, flag=
         mlp = _Mlp(ops, sd, f'blocks.{l}.mlp', f'blocks.{l}.norm2')
         x = mlp.forward(att.forward(x))
         enc.append((att, mlp))
-    enc_out = x
+    return enc, x
+
+
+def _encoder_backward(ops, sd, model, enc, dx):
+    """d output [B * Ne, D] (loss-scaled) -> d input tokens [B * Ne, D]; accumulates the blocks' and pos_embed's
+    gradients."""
+    D, ne = model.embed_dim, model.patch_embed.num_patches
+    B = dx.shape[0] // ne
+    for att, mlp in reversed(enc):
+        dx = att.backward(mlp.backward(dx))
+    g_pos = ops.grad('pos_embed', sd['pos_embed']).view(ne + 1, D)
+    _scatter_add(ops, dx, _zeros_index(B, ops.dev), B, ne, ne, 0, g_pos, ne + 1, 1, alpha=1.0 / ops.S)
+    return dx
+
+
+def _decoder_forward(ops, sd, model, tok32, g0, ctx_src, g1):
+    """The decoder of P = len(g0) pairs: pair p starts from the patch tokens ``tok32`` [items * Ne, D] of item g0[p]
+    and attends to the encoder tokens of item g1[p] of ``ctx_src`` (g1 None: ``ctx_src`` already is [P * Ne, D] in pair
+    order). Returns (the saved state, padded logits [P, ceil8(C)] fp32)."""
+    D, heads = model.embed_dim, model.num_heads
+    ne = model.patch_embed.num_patches
+    nd = ne + 1
+    P = g0.shape[0]
+    zeros_p = _zeros_index(P, ops.dev)
     # decoder input (prepare_x2, :390-395) of pair p: cls + pos[0] | tokens of image g0[p] + pos[1:]
     x = ops.empty(P * nd, D)
-    _gather(ops, pos32, zeros_b, P, nd, nd, 0, x, nd, 0, False)
-    _gather(ops, cls32, zeros_b, P, 1, 1, 0, x, nd, 0, True)
+    _gather(ops, sd['pos_embed'].view(nd, D), zeros_p, P, nd, nd, 0, x, nd, 0, False)
+    _gather(ops, sd['cls_token'].view(1, D), zeros_p, P, 1, 1, 0, x, nd, 0, True)
     _gather(ops, tok32, g0, P, ne, ne, 0, x, nd, 1, True)
-    ctx = ops.empty(P * ne, D)
-    _gather(ops, enc_out, g1, P, ne, ne, 0, ctx, ne, 0, False)
+    if g1 is None:
+        ctx = ctx_src
+    else:
+        ctx = ops.empty(P * ne, D)
+        _gather(ops, ctx_src, g1, P, ne, ne, 0, ctx, ne, 0, False)
     dec = []
     for l in range(model.c_depth):
         pre = f'cross_blocks.{l}'
@@ -453,22 +536,23 @@ def _train_step(model, samples, groups, labels, loss_scale, profile=False, flag=
         dec.append((att, cross, mlp))
     # final norm on the class-token rows, head (:400, :417 -> timm forward_head)
     xc = ops.empty(P, D)
-    arange_p = torch.arange(P, dtype=torch.int32, device=dev)
+    arange_p = torch.arange(P, dtype=torch.int32, device=ops.dev)
     _gather(ops, x, arange_p, P, 1, nd, 0, xc, 1, 0, False)
     norm = _LayerNorm(ops, sd, 'norm')
     head = _Linear(ops, sd, 'head')
-    C = model.num_classes
     logits_pad = ops.to_f32(head.forward(norm.forward(xc)))               # [P, ceil8(C)]
-    logits = logits_pad[:, :C].contiguous()
-    loss = ops.empty(1)
-    dlogits = ops.empty(P * C)
-    yy = y if y.numel() == P * C else y.view(P, 1).expand(P, C).contiguous().view(-1)
-    ops._chk(_lib.lib.vited_train_bce_logits(_p(logits), _p(yy), P * C, _p(loss), _p(dlogits), ops.S, ops.stream),
-             'train_bce_logits')
+    return (dec, norm, head, g0, arange_p), logits_pad
 
-    # ---------------- backward ----------------
-    dl_pad = ops.zeros(P, logits_pad.shape[1])
-    dl_pad[:, :C] = dlogits.view(P, C)                                    # (strided device copy: plumbing)
+
+def _decoder_backward(ops, sd, model, state, dlogits, dtok):
+    """d logits [P, C] (loss-scaled) -> d context [P * Ne, D] in pair order; scatter-adds the d patch tokens of every
+    pair into ``dtok`` [items * Ne, D] at its item g0[p]; accumulates every decoder parameter's gradient."""
+    dec, norm, head, g0, arange_p = state
+    D, ne = model.embed_dim, model.patch_embed.num_patches
+    nd = ne + 1
+    P, C = dlogits.shape
+    dl_pad = ops.zeros(P, head.n_pad)
+    dl_pad[:, :C] = dlogits                                               # (strided device copy: plumbing)
     dxc = ops.zeros(P, D)
     norm.backward(head.backward(dl_pad), dxc)
     dx = ops.zeros(P * nd, D)
@@ -477,27 +561,134 @@ def _train_step(model, samples, groups, labels, loss_scale, profile=False, flag=
     for att, cross, mlp in reversed(dec):
         dx = att.backward(cross.backward(mlp.backward(dx), dctx))
     inv = 1.0 / ops.S
+    zeros_p = _zeros_index(P, ops.dev)
     g_pos = ops.grad('pos_embed', sd['pos_embed']).view(nd, D)
     g_cls = ops.grad('cls_token', sd['cls_token']).view(1, D)
-    dtok = ops.zeros(B * ne, D)
-    _scatter_add(ops, dx, zeros_b, P, nd, nd, 0, g_pos, nd, 0, alpha=inv)
-    _scatter_add(ops, dx, zeros_b, P, 1, nd, 0, g_cls, 1, 0, alpha=inv)
+    _scatter_add(ops, dx, zeros_p, P, nd, nd, 0, g_pos, nd, 0, alpha=inv)
+    _scatter_add(ops, dx, zeros_p, P, 1, nd, 0, g_cls, 1, 0, alpha=inv)
     _scatter_add(ops, dx, g0, P, ne, nd, 1, dtok, ne, 0)
-    denc = ops.zeros(B * ne, D)
-    _scatter_add(ops, dctx, g1, P, ne, ne, 0, denc, ne, 0)
-    dx = denc
-    for att, mlp in reversed(enc):
-        dx = att.backward(mlp.backward(dx))
-    _scatter_add(ops, dx, zeros_b, B, ne, ne, 0, g_pos, nd, 1, alpha=inv)
-    ops.add_(dtok, dx)
-    patch.backward(dtok, need_dx=False)
+    return dctx
 
-    for name, p in model.named_parameters():
-        g = ops.grads.get(name)
-        p.grad = torch.zeros_like(p) if g is None else g.view_as(p).to(p.dtype)
-    model.train_launches = ops.launches
-    model.train_profile = ops.profile_read() if profile else None   # time between consecutive calls, by entry point
-    return loss[0], logits, groups, labels
+
+# ----------------------------------------------------------------------------------------------------------------
+# torch.autograd: the model's forward modes as differentiable Functions (VisionTransformerCustom in training mode)
+# ----------------------------------------------------------------------------------------------------------------
+def _mark_overflow(ops, tensors):
+    """+inf into element 0 of every fp32 tensor of ``tensors`` when a range check of this backward set the flag (on the
+    device: no host read), so that GradScaler sees the overflow that the saturating 16-bit conversions would hide."""
+    table = torch.tensor([[t.data_ptr(), t.numel()] for t in tensors], dtype=torch.int64).to(ops.dev)
+    ops._chk(_lib.lib.vited_train_mark_overflow(_p(table), len(tensors), _p(ops.flag), ops.stream), 'train_mark_overflow')
+
+
+def _forward_ops(dev, names, params):
+    """The ops of one differentiable forward: loss scale 1 (the incoming gradient carries the caller's scale) and an
+    overflow flag for its backward, and the state_dict of the mode's parameters."""
+    ops = _Ops(dev, 1.0, flag=torch.zeros(1, dtype=torch.int32, device=dev))
+    return ops, {n: p.detach().float().contiguous() for n, p in zip(names, params)}
+
+
+def _begin_backward(ctx):
+    """The ops of ctx's forward, on the calling thread's current stream; a second backward through the same graph
+    (``retain_graph=True``) and double backward raise."""
+    ctx.saved_tensors                                  # torch's own errors: graph already freed, inputs modified in place
+    if torch.is_grad_enabled():
+        raise RuntimeError('vit-ed_b200: double backward (create_graph=True) through the model is not supported')
+    if ctx.state is None:
+        raise RuntimeError('vit-ed_b200: the saved activations of this forward were freed by its first backward; '
+                           'run the forward again instead of backward(retain_graph=True) twice')
+    state, ctx.state = ctx.state, None                 # freed when this backward returns
+    ops = state[0]
+    ops.stream = ctypes.c_void_p(torch.cuda.current_stream(ops.dev).cuda_stream)
+    return state
+
+
+def _param_grads(ops, ctx, names, first):
+    """The gradients of the Function's parameter inputs (positions ``first``...), None where none is needed."""
+    return [ops.grads[n] if ctx.needs_input_grad[first + i] else None for i, n in enumerate(names)]
+
+
+def _finish(ops, grads, inputs):
+    """Marks an overflow into every gradient, then hands them out in the shapes / dtypes of their inputs."""
+    _mark_overflow(ops, [g for g in grads if g is not None])
+    return [None if g is None else g.view(shape).to(dtype) for g, (shape, dtype) in zip(grads, inputs)]
+
+
+class _Encode(torch.autograd.Function):
+    """model(images, forward_first_part=True): images [B, C, S, S] -> encoder tokens [B, Ne, D]. Inputs: the model,
+    the parameter names, the images and the parameters (patch_embed.proj.*, pos_embed, blocks.*)."""
+
+    @staticmethod
+    def forward(ctx, model, names, images, *params):
+        dev = images.device
+        with torch.cuda.device(dev):
+            ops, sd = _forward_ops(dev, names, params)
+            x = images.detach().float().contiguous()
+            B = x.shape[0]
+            patch, tok32 = _patch_embed_forward(ops, sd, model, x)
+            enc, out = _encoder_forward(ops, sd, model, tok32, B)
+        ctx.state = (ops, sd, patch, enc)
+        ctx.model, ctx.names = model, names
+        ctx.inputs = [(t.shape, t.dtype) for t in (images, *params)]
+        ctx.save_for_backward(*params)          # their storage is read by the backward (LayerNorm weights)
+        return out.view(B, model.patch_embed.num_patches, model.embed_dim)
+
+    @staticmethod
+    def backward(ctx, dtokens):
+        ops, sd, patch, enc = _begin_backward(ctx)
+        model = ctx.model
+        with torch.cuda.device(ops.dev):
+            dx = dtokens.detach().float().contiguous().view(-1, model.embed_dim)
+            dtok = _encoder_backward(ops, sd, model, enc, dx)
+            dimg = _patch_embed_backward(ops, model, patch, dtok, ctx.needs_input_grad[2])
+            grads = _finish(ops, [dimg] + _param_grads(ops, ctx, ctx.names, 3), ctx.inputs)
+        return (None, None, *grads)
+
+
+class _Decode(torch.autograd.Function):
+    """model(tokens, images): context tokens [B, Ne, D] x images [B, C, S, S] -> logits [B, num_classes]. Inputs: the
+    model, the parameter names, the tokens, the images and the parameters (patch_embed.proj.*, cls_token, pos_embed,
+    cross_blocks.*, norm.*, head.*)."""
+
+    @staticmethod
+    def forward(ctx, model, names, tokens, images, *params):
+        dev = images.device
+        with torch.cuda.device(dev):
+            ops, sd = _forward_ops(dev, names, params)
+            x = images.detach().float().contiguous()
+            P = x.shape[0]
+            ctx_tokens = tokens.detach().float().contiguous().view(-1, model.embed_dim)
+            patch, tok32 = _patch_embed_forward(ops, sd, model, x)
+            items = torch.arange(P, dtype=torch.int32, device=dev)        # pair p decodes its own image p
+            state, logits_pad = _decoder_forward(ops, sd, model, tok32, items, ctx_tokens, None)
+            logits = logits_pad[:, :model.num_classes].contiguous()
+        ctx.state = (ops, sd, patch, state)
+        ctx.model, ctx.names = model, names
+        ctx.inputs = [(t.shape, t.dtype) for t in (tokens, images, *params)]
+        ctx.save_for_backward(tokens, *params)  # their storage is read by the backward (context LayerNorm input)
+        return logits
+
+    @staticmethod
+    def backward(ctx, dlogits):
+        ops, sd, patch, state = _begin_backward(ctx)
+        model = ctx.model
+        with torch.cuda.device(ops.dev):
+            dl = dlogits.detach().float().contiguous()
+            dtok = ops.zeros(dl.shape[0] * model.patch_embed.num_patches, model.embed_dim)
+            dctx = _decoder_backward(ops, sd, model, state, dl, dtok)
+            dimg = _patch_embed_backward(ops, model, patch, dtok, ctx.needs_input_grad[3])
+            dctx = dctx if ctx.needs_input_grad[2] else None
+            grads = _finish(ops, [dctx, dimg] + _param_grads(ops, ctx, ctx.names, 4), ctx.inputs)
+        return (None, None, *grads)
+
+
+def encode(model, images, names, params):
+    """Differentiable ``model(images, forward_first_part=True)`` over the parameters ``params`` (named ``names``)."""
+    return _Encode.apply(model, tuple(names), images, *params)
+
+
+def decode(model, tokens, images, names, params):
+    """Differentiable ``model(tokens, images)`` over the parameters ``params`` (named ``names``)."""
+    return _Decode.apply(model, tuple(names), tokens, images, *params)
 
 
 # ----------------------------------------------------------------------------------------------------------------
